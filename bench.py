@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — 10 s-clip waveform -> scores throughput (clips/s) of the B200 path, beside the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--clips C] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--clips C] [--impl b200|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (fused log-mel -> VGGish -> multi-level-attention head) over one batch of
 C synthetic 10 s / 16 kHz clips per GPU (default 256 = BASELINE.json configs[1]).  For N > 1 the driver launches
@@ -21,6 +21,9 @@ One JSON line is printed by rank 0:
              with the NCCL all-reduce of the gradient bucket at N > 1)
   e2e_dropin the reference-named API: per-clip waveform_to_examples + Ensemble.forward, and Ensemble.forward_waveform
 --impl reference times the CPU path alone (rank 0 only) on a bounded sample of the same workload.
+--dump-outputs DIR writes the scores of the last timed step (the global batch at N > 1; for --impl reference the first
+clips of the batch that its sample timed) to DIR/scores.npy.  Inputs and weights are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -84,6 +87,22 @@ def emit(line):
     (_OUT or sys.stdout).write(json.dumps(line) + "\n")
     (_OUT or sys.stdout).flush()
 
+
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, scores):
+    """--dump-outputs: writes the scores (clips x classes) the timed path returned in its last step as
+    out_dir/scores.npy, float32, so that two builds run with the same arguments can be compared output for output.
+    Scores larger than DUMP_MAX_BYTES are cut to a fixed sample of clips (seed 0, in clip order)."""
+    scores = scores.detach().float().cpu().numpy()
+    max_rows = (DUMP_MAX_BYTES - 4096) // (4 * scores.shape[1])                   # 4096: room for the .npy header
+    if scores.shape[0] > max_rows:
+        scores = scores[np.sort(np.random.default_rng(0).choice(scores.shape[0], max_rows, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "scores.npy"), np.ascontiguousarray(scores, dtype=np.float32))
+
+
 def igemm_traffic():
     """(DRAM bytes per launch of the dominant kernel, where the figure comes from): read from the committed ncu
     capture — a profiler figure, not a measurement of this run."""
@@ -136,7 +155,8 @@ def oracle_pass(waves, vsd, msd):
 
 
 def time_cpu(vsd, msd, steps, warmup, budget_s):
-    """Times `steps` oracle passes (after `warmup`) on a sample sized so that the whole run takes ~budget_s."""
+    """Times `steps` oracle passes (after `warmup`) on a sample sized so that the whole run takes ~budget_s; returns the
+    scores of the last pass with the timings."""
     synth, _, _ = _oracle_modules()
     probe = synth.fast_clips(0, 2).numpy()
     oracle_pass(probe[:1], vsd, msd)                         # page-in / thread pools
@@ -149,10 +169,10 @@ def time_cpu(vsd, msd, steps, warmup, budget_s):
         oracle_pass(waves, vsd, msd)
     t0 = time.perf_counter()
     for _ in range(steps):
-        oracle_pass(waves, vsd, msd)
+        scores = oracle_pass(waves, vsd, msd)
     dt = time.perf_counter() - t0
     return {"clips_per_s": n * steps / dt, "ms_per_step": 1e3 * dt / steps, "sample_clips": n, "steps": steps,
-            "threads": torch.get_num_threads()}
+            "threads": torch.get_num_threads(), "scores": scores}
 
 
 def run_reference(args, rank):
@@ -164,6 +184,8 @@ def run_reference(args, rank):
     msd = synth.mla_state_dict(MODEL_CONF, 128, 600, N_CLASSES, 10, seed=2)
     # ~90 s of CPU work for the whole run by default (VMB_BENCH_CPU_BUDGET_S overrides, e.g. for the CPU test suite)
     r = time_cpu(vsd, msd, args.steps, args.warmup, budget_s=float(os.environ.get("VMB_BENCH_CPU_BUDGET_S", "90")))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["scores"])
     sample = (f"{r['sample_clips']} of the {args.clips} clips of a step per timed pass, {args.steps} passes after "
               f"{args.warmup} warm-ups; numpy float64 front end + torch {torch.__version__} CPU fp32")
     line = {
@@ -604,6 +626,14 @@ def run_b200(args, rank, local_rank, world):
     sampler.join(timeout=1.0)
     vgg.check_saturation()
     finite = bool(torch.isfinite(scores).all().item())
+    if args.dump_outputs:
+        dumped = scores
+        if world > 1:                                               # the global batch: every rank's shard in rank order
+            parts = [torch.empty_like(scores) for _ in range(world)]
+            dist.all_gather(parts, scores)
+            dumped = torch.cat(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, dumped)
     peaks = measured_peaks()
 
     # ---- the same step back to back for >= 3 s: the sustained regime
@@ -843,7 +873,11 @@ def main():
                     help="seconds the configs[2..4] / drop-in legs may take before the line is printed without them")
     ap.add_argument("--no-config-legs", action="store_true",
                     help="skip the batch8192 / stream_1h / train / e2e_dropin legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the scores of the last timed step to DIR/scores.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -288,3 +288,36 @@ def test_bench_reference_arm_prints_exactly_one_json_line():
     assert d["impl"] == "reference" and d["unit"] == "clips/s" and d["value"] > 0
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+
+
+def test_bench_reference_arm_dumps_the_scores_of_its_last_step(tmp_path):
+    """--dump-outputs DIR: the reference arm writes the scores of its last timed pass, which are the oracle's scores of
+    the first clips of the benchmark batch."""
+    import json
+    import subprocess
+    import sys
+    import bench
+    from b200 import synth
+    env = dict(os.environ, VMB_BENCH_CPU_BUDGET_S="2")
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup",
+                        "0", "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, env=env, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    n = json.loads(r.stdout)["reference_sample_clips_per_step"]
+    got = np.load(tmp_path / "out" / "scores.npy")
+    assert got.dtype == np.float32 and got.shape == (n, 527)
+    want = bench.oracle_pass(synth.fast_clips(0, n).numpy(), synth.vggish_state_dict(0),
+                             synth.mla_state_dict((2, 1), 128, 600, 527, 10, seed=2)).numpy()
+    np.testing.assert_allclose(got, want, rtol=0, atol=1e-5)
+
+
+def test_bench_dump_is_capped_to_a_fixed_sample(tmp_path):
+    """Scores above bench.DUMP_MAX_BYTES are cut to the same sample of clips on every run, kept in clip order."""
+    import bench
+    scores = torch.rand(40000, 527, generator=torch.Generator().manual_seed(0))
+    scores[:, 0] = torch.arange(40000)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), scores)
+    a, b = np.load(tmp_path / "a" / "scores.npy"), np.load(tmp_path / "b" / "scores.npy")
+    assert os.path.getsize(tmp_path / "a" / "scores.npy") <= bench.DUMP_MAX_BYTES and np.array_equal(a, b)
+    rows = a[:, 0].astype(np.int64)
+    assert a.shape[0] > 30000 and np.all(np.diff(rows) > 0) and np.array_equal(a, scores.numpy()[rows])

@@ -16,6 +16,8 @@ import torch.multiprocessing as mp
 
 from conftest import PKG, ROOT
 
+THREADS = 2             # torch splits fp32 reductions by thread count: the ranks and the check below use the same one
+
 
 def _free_port():
     with socket.socket() as s:
@@ -30,7 +32,7 @@ def _worker(rank, world, port, out_dir):
             sys.path.insert(0, p)
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
                       LOCAL_RANK=str(rank))
-    torch.set_num_threads(2)
+    torch.set_num_threads(THREADS)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     from b200 import sharding, synth, training
     from oracle import model_torch, train_torch
@@ -89,7 +91,15 @@ def _worker(rank, world, port, out_dir):
     dist.destroy_process_group()
 
 
-def test_two_rank_gloo(tmp_path):
+@pytest.fixture
+def rank_thread_count():
+    threads = torch.get_num_threads()
+    torch.set_num_threads(THREADS)
+    yield
+    torch.set_num_threads(threads)
+
+
+def test_two_rank_gloo(tmp_path, rank_thread_count):
     world = 2
     mp.spawn(_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
     got = torch.load(os.path.join(tmp_path, "rank0.pt"))
@@ -111,7 +121,7 @@ def test_two_rank_gloo(tmp_path):
         _, _, grads = train_torch.head_step(sd, x[lo:hi], labels[lo:hi], conf)
         for key, shape, off in p_layout:
             want[off:off + grads[key].numel()] += grads[key].reshape(-1) / world
-    assert torch.allclose(got["bucket"], want, rtol=1e-4, atol=1e-6)      # thread counts differ between processes
+    assert torch.allclose(got["bucket"], want, rtol=1e-4, atol=1e-6)      # the all-reduce sums in another order
     # sharded optimiser step == all-reduce + Adam on every rank; the slices tile the padded bucket in rank order
     assert got["slices"][0][0] == 0 and got["slices"][-1][1] == got["npad"]
     assert all(a[1] == b[0] for a, b in zip(got["slices"], got["slices"][1:]))

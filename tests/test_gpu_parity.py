@@ -986,3 +986,19 @@ def test_pcm16_host_pipeline(vgg_handle, head_handle):
     pipe.wait_host(pipe.submit_host(pcm, out, clips_per_batch=2))
     want = pipe.forward((pcm.float() / 32768.0).to(DEV)).cpu()
     assert torch.equal(out, want)
+
+
+def test_bench_dumps_the_scores_of_its_last_timed_step(tmp_path, vgg_sd, head_handle):
+    """bench.py --dump-outputs DIR: DIR/scores.npy holds what the timed device-resident step returned, bit for bit."""
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "1", "--clips", "64",
+                        "--sustained-seconds", "0", "--no-config-legs", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = np.load(tmp_path / "scores.npy")
+    vgg = engine.VggishHandle(vgg_sd, DEV, precision="fp16")
+    want = engine.Pipeline(vgg, head_handle).forward(synth.fast_clips(0, 64).to(DEV)).cpu().numpy()
+    vgg.close()
+    assert got.dtype == np.float32 and np.array_equal(got, want)

@@ -7,6 +7,18 @@ import torch
 from b200 import synth
 from oracle import frontend_np, model_torch
 
+GOLDEN_THREADS = 8      # the CPU thread count make_golden.py ran the reference with
+
+
+@pytest.fixture(autouse=True)
+def _golden_thread_count():
+    """torch splits fp32 reductions by thread count, so the last bits of the oracle's outputs depend on it: the oracle
+    runs with the thread count the golden vectors were made with, whatever the host has."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(threads)
+
 
 def test_tables_bit_exact(golden_front):
     assert np.array_equal(frontend_np.periodic_hann(400), golden_front["hann400"])
