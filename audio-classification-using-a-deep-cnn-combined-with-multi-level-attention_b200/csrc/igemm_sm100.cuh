@@ -174,8 +174,9 @@ int planes_gemm_gradstats(const void* a_planes, const void* b_planes, float* out
                           int planes, const PlanesGradStats& gs, cudaStream_t stream);
 int planes_gemm_stats(const void* a_planes, const void* b_planes, const float* bias, float* out, long long ldo, int M,
                       int N, int K, int planes, const PlanesStats& stats, cudaStream_t stream);
-// Split-K GEMM over ROW-major operands read as MN-major UMMA operands (head training, weight gradients dW = G^T A):
-// out fp32 [M][ldo] += sum_r a[r][m] b[r][n]; a_planes bf16 [K][planes * a_cols], b_planes bf16 [K][planes * b_cols].
+// GEMM over ROW-major operands read as MN-major UMMA operands (head training, weight gradients dW = G^T A):
+// out fp32 [M][ldo] (+)= sum_r a[r][m] b[r][n]; a_planes bf16 [K][planes * a_cols], b_planes bf16 [K][planes * b_cols].
+// ksplit > 1 or -1: K slices added into out with vector reductions (out zeroed by the caller); ksplit 0: plain stores.
 int planes_gemm_mn(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M,
                    int N, int K, int planes, int ksplit, cudaStream_t stream);
 bool planes_gemm_enabled();

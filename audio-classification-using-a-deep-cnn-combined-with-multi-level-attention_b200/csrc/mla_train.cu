@@ -417,6 +417,144 @@ struct FBnBackward {
   }
 };
 
+// ------------------------------------------------------------------ wide first layer (emb_in wider than the hidden width)
+// The level-0 norm0 output y = gamma_t xhat + beta_t never exists: the first Linear reads the planes of xhat, and a tile
+// pass applies the affine to its output (FAffine: U = gamma_t P + beta_t s + b with P = xhat W^T and
+// s[o] = sum_f W[o][f]).  In the backward pass, with G = dL/dU of block (0, 0):
+//   dbeta_t  = sum_{r in t} G[r,:] . s          dgamma_t = sum_{r in t} G[r,:] . P[r,:]
+//   dW[o][f] = sum_r (gamma_t G[r][o]) xhat[r][f] + c[o],   c[o] = sum_t beta_t sum_{r in t} G[r][o]
+// so no GEMM over the input width runs but the forward one and dW, and nothing divides by gamma.  Both contract in
+// slices of at most kWideSlice (forward: input columns) / kDwSlice (dW: rows) per tcgen05 accumulator.
+constexpr int kWideSlice = 768, kDwSlice = 1024;
+
+// xhat = (x - mean_t) rstd_t (the same expression GradIn::xhat evaluates)
+struct FNormalize {
+  const float* u; long long ld; int T;
+  const float* stat;
+  __device__ void prologue(bool) {}
+  __device__ int time_steps() const { return T; }
+  __device__ float operator()(int r, int t, int c) const {
+    return (__ldg(u + static_cast<long long>(r) * ld + c) - __ldg(stat + 2 * t)) * __ldg(stat + 2 * t + 1);
+  }
+};
+
+// U = gamma_t P + (beta_t s[c] + b[c]) from P = xhat W^T
+struct FAffine {
+  const float* p; long long ld; int T;
+  const float *gamma, *beta, *s, *bias;
+  __device__ void prologue(bool) {}
+  __device__ int time_steps() const { return T; }
+  __device__ float operator()(int r, int t, int c) const {
+    return fmaf(__ldg(gamma + t), __ldg(p + static_cast<long long>(r) * ld + c), fmaf(__ldg(beta + t), __ldg(s + c), __ldg(bias + c)));
+  }
+};
+
+// s[o] = sum_f W[o][f] in double, one CTA per row
+__global__ void __launch_bounds__(256) row_sum_kernel(const float* __restrict__ w, int n_in, float* __restrict__ s) {
+  const float* row = w + static_cast<long long>(blockIdx.x) * n_in;
+  double acc = 0;
+  for (int f = threadIdx.x; f < n_in; f += blockDim.x) acc += __ldg(row + f);
+#pragma unroll
+  for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  __shared__ double red[8];
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double a = 0;
+    for (int i = 0; i < 8; ++i) a += red[i];
+    s[blockIdx.x] = static_cast<float>(a);
+  }
+}
+
+struct WideGradOut {
+  __nv_bfloat16* planes;      // [rows_pad][3 * cols_pad]: gamma_t G (the dW GEMM's A operand)
+  long long rows, rows_pad;
+  int cols, cols_pad;
+  const float* gamma0;        // norm0 weight [T]
+  const float* P; long long ldp;   // xhat W^T [rows][ldp] from the forward GEMM
+  const float* wsum;          // s [cols_pad]
+  float* col_sum;             // d(bias) [cols] += sum over rows of G
+  float* col_sum_t;           // [T][cols_pad] += sum over the rows of time step t of G (zeroed by the caller)
+  double* acc0;               // norm0's backward slot [T][2] += {G . s, G . P}
+};
+
+// Block (0, 0)'s BatchNorm backward (FBnBackward, G = dL/dU) on 64 x 64 tiles, as tile_body runs it, writing what the
+// wide first layer needs instead of G's planes: see the identities above.
+__global__ void __launch_bounds__(256) wide_grad_tile_kernel(FBnBackward f, WideGradOut o) {
+  vmb::pdl_launch_dependents();   // programmatic dependent launch: see sm100_ptx.cuh
+  vmb::pdl_wait();
+  __shared__ float tile[kTile][kTile + 1];
+  __shared__ double dots[16][2];
+  f.prologue(blockIdx.x == 0 && blockIdx.y == 0);
+  if (threadIdx.x < 32) dots[threadIdx.x >> 1][threadIdx.x & 1] = 0.0;
+  __syncthreads();
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+  const int r0 = blockIdx.y * kTile, c0 = blockIdx.x * kTile;
+  const int T = f.time_steps();
+  const int c = c0 + 2 * tx;
+  const float s0 = c < o.cols_pad ? __ldg(o.wsum + c) : 0.f, s1 = c + 1 < o.cols_pad ? __ldg(o.wsum + c + 1) : 0.f;
+#pragma unroll
+  for (int i = 0; i < kTile / 8; ++i) {
+    const int r = r0 + ty + 8 * i;   // one row per warp: the row's dot products are warp sums
+    float v0 = 0.f, v1 = 0.f, gs = 0.f, gp = 0.f, gam = 0.f;
+    int t = 0;
+    if (r < o.rows) {
+      t = T > 1 ? r % T : 0;
+      gam = __ldg(o.gamma0 + t);
+      const float* prow = o.P + static_cast<long long>(r) * o.ldp;
+      if (c < o.cols) { v0 = f(r, t, c); gs = v0 * s0; gp = v0 * __ldg(prow + c); }
+      if (c + 1 < o.cols) { v1 = f(r, t, c + 1); gs = fmaf(v1, s1, gs); gp = fmaf(v1, __ldg(prow + c + 1), gp); }
+    }
+    tile[ty + 8 * i][2 * tx] = v0;
+    tile[ty + 8 * i][2 * tx + 1] = v1;
+    if (r < o.rows_pad && c < o.cols_pad)
+      store_split_pair(gam * v0, gam * v1, o.planes + static_cast<long long>(r) * (static_cast<long long>(kPl) * o.cols_pad) + c,
+                       o.cols_pad);
+#pragma unroll
+    for (int off = 16; off; off >>= 1) {
+      gs += __shfl_xor_sync(0xffffffffu, gs, off);
+      gp += __shfl_xor_sync(0xffffffffu, gp, off);
+    }
+    if (tx == 0 && r < o.rows) {
+      atomicAdd(&dots[t][0], static_cast<double>(gs));
+      atomicAdd(&dots[t][1], static_cast<double>(gp));
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x < kTile && c0 + static_cast<int>(threadIdx.x) < o.cols) {
+    const int cc = c0 + threadIdx.x;
+    float s = 0.f;
+#pragma unroll 8
+    for (int j = 0; j < kTile; ++j) s += tile[j][threadIdx.x];
+    atomicAdd(o.col_sum + cc, s);
+    for (int t = 0; t < T; ++t) {   // rows past `rows` hold zeros
+      float st = 0.f;
+      for (int j = (t - r0 % T + T) % T; j < kTile; j += T) st += tile[j][threadIdx.x];
+      atomicAdd(o.col_sum_t + static_cast<long long>(t) * o.cols_pad + cc, st);
+    }
+  }
+  if (threadIdx.x < 2 * T) atomicAdd(o.acc0 + threadIdx.x, dots[threadIdx.x >> 1][threadIdx.x & 1]);
+}
+
+// grads dW [n_out][n_in] = the GEMM's sum_r (gamma_t G) xhat [n_out][ldw] + c[o]; grid = (column chunks, n_out)
+__global__ void __launch_bounds__(256)
+wide_dw_finish_kernel(const float* __restrict__ dw, long long ldw, float* __restrict__ dst, int n_in,
+                      const float* __restrict__ col_sum_t, int ldc, const float* __restrict__ beta0, int T) {
+  vmb::pdl_launch_dependents();
+  vmb::pdl_wait();
+  const int o = blockIdx.y;
+  __shared__ float c_o;
+  if (threadIdx.x == 0) {
+    double c = 0;
+    for (int t = 0; t < T; ++t) c += double(__ldg(beta0 + t)) * __ldg(col_sum_t + static_cast<long long>(t) * ldc + o);
+    c_o = static_cast<float>(c);
+  }
+  __syncthreads();
+  const float* src = dw + static_cast<long long>(o) * ldw;
+  float* out = dst + static_cast<long long>(o) * n_in;
+  for (int f = blockIdx.x * blockDim.x + threadIdx.x; f < n_in; f += gridDim.x * blockDim.x) out[f] = src[f] + c_o;
+}
+
 // ------------------------------------------------------------------ attention (one CTA per clip)
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
@@ -834,6 +972,11 @@ struct vmb_mla_trainer {
   float *dA = nullptr, *dB = nullptr, *dEnext = nullptr;  // fp32 gradient buffers [R][Hp]
   float* dWtmp = nullptr;                          // padded dW GEMM output
   int Hp, Kp, inpad, ycols, ycols_pad;
+  // wide first layer (inpad > Hp): xin_p holds the planes of xhat, not of the norm0 output (see FNormalize)
+  bool wide = false;
+  float* P0 = nullptr;                             // xhat W^T of the first Linear [R][Hp]
+  float* wsum = nullptr;                           // s[o] = sum_f W[o][f] [Hp]
+  float* gsum_t = nullptr;                         // per-time-step column sums of block (0, 0)'s G [T][Hp]
   // The dropout seed of the step lives in device memory, so that a captured step can be replayed with a new seed.
   unsigned long long* seed_dev = nullptr;
   // CUDA graph of the whole step (vmb_mla_train_step): ~110 kernel launches, memsets and stream fork / join events cost
@@ -878,7 +1021,13 @@ void carve(vmb_mla_trainer* h, char* base) {
   h->acc_bytes = c.off;
   h->stat = c.take<float>(size_t(h->n_slots) * kSlot * 2);
   h->xin_p = c.take<__nv_bfloat16>(size_t(Rp) * kPl * inpad);
-  h->xin_pt = c.take<__nv_bfloat16>(size_t(inpad) * kPl * Rp);
+  if (h->wide) {   // only the MN-major weight-gradient path runs at this width: no transposed planes
+    h->P0 = c.take<float>(size_t(R) * Hp);
+    h->wsum = c.take<float>(size_t(Hp));
+    h->gsum_t = c.take<float>(size_t(h->T) * Hp);
+  } else {
+    h->xin_pt = c.take<__nv_bfloat16>(size_t(inpad) * kPl * Rp);
+  }
   for (int l = 0; l < h->n_levels; ++l) {
     for (int j = 0; j < h->lvl[l].n_fc; ++j) {
       h->U[l][j] = c.take<float>(size_t(R) * Hp);
@@ -923,7 +1072,9 @@ void carve(vmb_mla_trainer* h, char* base) {
   auto planes_for = [&](FcRef& f) {
     f.bias_pad = c.take<float>(size_t(f.n_out_pad));
     f.wp = c.take<__nv_bfloat16>(size_t(f.n_out_pad) * kPl * f.n_in_pad);
-    f.wtp = c.take<__nv_bfloat16>(size_t(f.n_in_pad) * kPl * f.n_out_pad);
+    // the transposed weights feed only the dX GEMM, which the wide first layer does not run
+    f.wtp = (h->wide && &f == &h->lvl[0].fc[0]) ? nullptr
+                                                 : c.take<__nv_bfloat16>(size_t(f.n_in_pad) * kPl * f.n_out_pad);
   };
   for (int l = 0; l < h->n_levels; ++l) {
     for (int j = 0; j < h->lvl[l].n_fc; ++j) planes_for(h->lvl[l].fc[j]);
@@ -1004,16 +1155,21 @@ bool mn_dw_enabled() {
 // dW [M][ldo] = sum over rows r of a[r][m] b[r][n]: a_planes [K][kPl * a_cols], b_planes [K][kPl * b_cols]
 int gemm_dw_mn(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M, int N,
                long long K, cudaStream_t st) {
-  if (cudaMemsetAsync(out, 0, size_t(M) * ldo * sizeof(float), st) != cudaSuccess) {
+  // one wave of (K slice, tile) work items, each slice at least four 32-row K-blocks long.  An output of more tiles
+  // than SMs (the wide first layer's dW) is split only into slices of at most kDwSlice rows, the length the 640-wide
+  // layers' slices have at 512 clips (precision of the tcgen05 accumulator, see gemm_bn); one slice: plain stores.
+  const int mn = (M / 128) * (N / 128);
+  int ks = vmb::num_sms() / mn;
+  if (ks == 0) ks = int((K + kDwSlice - 1) / kDwSlice);
+  const bool plain = ks == 1 && mn > vmb::num_sms();
+  if (ks > K / 32 / 4) ks = int(K / 32 / 4);
+  if (ks < 1) ks = 1;
+  if (!plain && cudaMemsetAsync(out, 0, size_t(M) * ldo * sizeof(float), st) != cudaSuccess) {
     vmb::set_kernel_error("dW buffer clear failed");
     return 1;
   }
-  // one wave of (K slice, tile) work items, each slice at least four 32-row K-blocks long
-  const int mn = (M / 128) * (N / 128);
-  int ks = vmb::num_sms() / mn;
-  if (ks > K / 32 / 4) ks = int(K / 32 / 4);
-  if (ks < 1) ks = 1;
-  if (vmb::planes_gemm_mn(a_planes, a_cols, b_planes, b_cols, out, ldo, M, N, int(K), kPl, ks > 1 ? ks : -1, st)) {
+  if (vmb::planes_gemm_mn(a_planes, a_cols, b_planes, b_cols, out, ldo, M, N, int(K), kPl, plain ? 0 : ks > 1 ? ks : -1,
+                          st)) {
     vmb::set_kernel_error("%s", vmb::planes_gemm_last_error());
     return 1;
   }
@@ -1109,12 +1265,24 @@ int vmb_mla_trainer_create(vmb_mla_trainer_t** handle, int n_levels, const int* 
   if (t_steps < 1 || t_steps > 16) return fail("vmb_mla_trainer_create: 1 <= T <= 16");
   if (emb_in < 1 || emb_in > 16384 || hidden < 1 || hidden > 1024 || n_classes < 1 || n_classes > 1024)
     return fail("vmb_mla_trainer_create: hidden and n_classes must be in 1..1024, emb_in in 1..16384");
-  if (pad128(emb_in) > std::max(pad128(hidden), pad128(n_classes)))
-    return fail("vmb_mla_trainer_create: emb_in wider than the hidden width is not supported by the trainer yet");
   if (max_batch < 2 || max_batch * t_steps > 0x7fffffffLL / 2048) return fail("vmb_mla_trainer_create: bad max_batch");
+  const bool wide = pad128(emb_in) > std::max(pad128(hidden), pad128(n_classes));
+  if (wide) {
+    // The wide first layer's largest per-step buffer is the operand planes of xhat, [pad64(batch * T)][3 * inpad]
+    // bf16: its element count stays within a signed 32-bit index (at emb_in 12288, T = 10: 5824 clips)
+    const long long per_row = static_cast<long long>(kPl) * pad128(emb_in);
+    const long long max_rows = 0x7fffffffLL / per_row / 64 * 64;
+    if (pad64(max_batch * t_steps) > max_rows) {
+      char msg[256];
+      snprintf(msg, sizeof msg, "vmb_mla_trainer_create: max_batch %lld too large for emb_in %d, T %d: at most %lld clips",
+               max_batch, emb_in, t_steps, max_rows / t_steps);
+      return fail("%s", msg);
+    }
+  }
   vmb_mla_trainer* h = new vmb_mla_trainer();
   h->n_levels = n_levels; h->emb_in = emb_in; h->H = hidden; h->K = n_classes; h->T = t_steps;
   h->max_batch = max_batch;
+  h->wide = wide;
   h->Hp = std::max(pad128(hidden), pad128(n_classes));
   h->Kp = h->Hp;
   h->inpad = pad128(emb_in);
@@ -1261,8 +1429,31 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
   const bool estats_fused = estats_env && T <= 16;   // norm0 statistics of levels >= 1 from the pass that writes the embedding
   const bool mn_dw = mn_dw_enabled();   // weight-gradient GEMMs read the row-major planes: no transposed planes are written
   auto tplanes = [&](__nv_bfloat16* pt) { return mn_dw ? static_cast<__nv_bfloat16*>(nullptr) : pt; };
+  if (h->wide && !mn_dw)
+    return fail("vmb_mla_train: emb_in wider than the hidden width needs the planes GEMM and its MN-major weight-gradient "
+                "kernel (VMB_PLANES_GEMM=0 or VMB_TRAIN_MN_DW=0 is set)");
+  const LevelRef& L0 = h->lvl[0];
   // Linear (+ bias) into `out` and the BatchNorm statistics of its first `cols` columns
   auto gemm_bn = [&](const void* a, const FcRef& fc, float* out, int k_pad, int cols, const BnRef& bn, cudaStream_t ss) {
+    if (h->wide && &fc == &L0.fc[0]) {
+      // P = xhat W^T with the K loop cut into slices of kWideSlice columns (fp32 reductions into a zeroed P): one
+      // tcgen05 accumulator summed over all 12288 columns loses ~1e-4 relative to its per-step truncation, which moved
+      // gradients past the fp32 reference's tolerance.  Then U = gamma_t P + beta_t s + b and U's statistics.
+      if (cudaMemsetAsync(h->P0, 0, size_t(R) * Hp * sizeof(float), ss) != cudaSuccess) {
+        vmb::set_kernel_error("wide-layer output clear failed");
+        return 1;
+      }
+      if (vmb::planes_gemm(a, fc.wp, nullptr, h->P0, Hp, 0, int(R), Hp, k_pad, kPl, (k_pad + kWideSlice - 1) / kWideSlice,
+                           ss)) {
+        vmb::set_kernel_error("%s", vmb::planes_gemm_last_error());
+        return 1;
+      }
+      FAffine f{h->P0, Hp, T, params + L0.norm0.g, params + L0.norm0.b, h->wsum, fc.bias_pad};
+      TileOut o{nullptr, nullptr, out, Hp, nullptr, R, R, cols, Hp};
+      o.stats = statjob(bn, double(B) * cols);
+      o.stats_T = T;
+      return run_tile(f, o, ss, "wide-layer affine + statistics");
+    }
     if (fuse_stats) return gemm_stats(a, fc.wp, fc.bias_pad, out, Hp, R, Hp, k_pad, statjob(bn, double(B) * cols), cols, ss);
     int r = gemm(a, fc.wp, fc.bias_pad, out, Hp, R, Hp, k_pad, ss);
     return r ? r : time_stats(out, Hp, cols, bn, true, ss);
@@ -1284,6 +1475,12 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     vmb::count_launch();
     TRY(vmb::check_launch("weights_split_kernel"));
   }
+  if (!rc && h->wide) {   // s[o] = sum_f W[o][f] of the wide first Linear (its GEMM epilogue and the backward pass)
+    row_sum_kernel<<<static_cast<unsigned>(L0.fc[0].n_out), 256, 0, ws_stream>>>(params + L0.fc[0].w, L0.fc[0].n_in,
+                                                                                h->wsum);
+    vmb::count_launch();
+    TRY(vmb::check_launch("row_sum_kernel"));
+  }
   if (forked) cudaEventRecord(h->ev_w, h->side);
   bool weights_pending = forked;
 
@@ -1298,7 +1495,10 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     __nv_bfloat16* np = l == 0 ? h->xin_p : h->N_p[l];
     __nv_bfloat16* npt = tplanes(l == 0 ? h->xin_pt : h->N_pt[l]);
     if (!(l > 0 && estats_fused)) TRY(time_stats(in, ld_in, F_in, L.norm0, true, st));
-    {
+    if (l == 0 && h->wide) {
+      TileOut o{np, nullptr, nullptr, 0, nullptr, R, Rp, F_in, in_pad};
+      TRY(run_tile(FNormalize{in, ld_in, T, slotstat(L.norm0.slot)}, o, st, "norm0 forward (xhat)"));
+    } else {
       FBnAct f{in, ld_in, T, F_in, slotstat(L.norm0.slot), params + L.norm0.g, params + L.norm0.b, 0, 0.f, h->seed_dev, 0};
       TileOut o{np, npt, nullptr, 0, nullptr, R, Rp, F_in, in_pad};
       TRY(run_tile(f, o, st, "norm0 forward"));
@@ -1394,8 +1594,16 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       cudaStreamWaitEvent(h->side, h->ev_fork, 0);
     }
     int r = dw_gemm(ops, h->dWtmp, ldo, M, N, Kc, s);
-    if (!r && cudaMemcpy2DAsync(dst, dst_pitch, h->dWtmp, size_t(ldo) * 4, width, height, cudaMemcpyDeviceToDevice, s) !=
-                  cudaSuccess) {
+    if (!r && dst == grads + L0.fc[0].w && h->wide) {
+      // the wide first Linear: dW = the GEMM's sum_r (gamma_t G) xhat + c[o] (see wide_grad_tile_kernel)
+      const int n_in = L0.fc[0].n_in;
+      vmb::launch_pdl(wide_dw_finish_kernel, dim3(unsigned((n_in + 1023) / 1024), unsigned(height)), dim3(256), 0, s,
+                      static_cast<const float*>(h->dWtmp), ldo, dst, n_in, static_cast<const float*>(h->gsum_t), Hp,
+                      params + L0.norm0.b, T);
+      vmb::count_launch();
+      r = vmb::check_launch("wide_dw_finish_kernel");
+    } else if (!r && cudaMemcpy2DAsync(dst, dst_pitch, h->dWtmp, size_t(ldo) * 4, width, height, cudaMemcpyDeviceToDevice,
+                                       s) != cudaSuccess) {
       vmb::set_kernel_error("dW copy failed");
       r = 1;
     }
@@ -1546,16 +1754,35 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
         TRY(vmb::check_launch("bn_time_backward_reduce_kernel"));
       }
       FBnBackward f{gi, acc, double(B) * H, grads + L.norms[j].g, grads + L.norms[j].b};
-      TileOut o{h->G_p, tplanes(h->G_pt), nullptr, Hp, grads + fc.b, R, Rp, H, Hp};
+      const bool wide0 = h->wide && l == 0 && j == 0;
       before_g_overwrite();
-      TRY(run_tile(f, o, st, "fc BN backward"));
+      if (wide0) {
+        // G of the wide first Linear: gamma_t-scaled planes for dW, the sums for c[o] and for norm0's two gradients
+        if (cudaMemsetAsync(h->gsum_t, 0, size_t(T) * Hp * sizeof(float), st) != cudaSuccess) {
+          vmb::set_kernel_error("wide-layer column sums clear failed");
+          rc = 1;
+        }
+        WideGradOut o{h->G_p, R, Rp, H, Hp, params + L.norm0.g, h->P0, Hp, h->wsum, grads + fc.b, h->gsum_t,
+                      block_acc(0, -1)};
+        if (!rc) {
+          vmb::launch_pdl(wide_grad_tile_kernel, tile_grid(Rp, Hp), dim3(256), 0, st, f, o);
+          vmb::count_launch();
+          TRY(vmb::check_launch("wide_grad_tile_kernel"));
+        }
+      } else {
+        TileOut o{h->G_p, tplanes(h->G_pt), nullptr, Hp, grads + fc.b, R, Rp, H, Hp};
+        TRY(run_tile(f, o, st, "fc BN backward"));
+      }
       // dW [H][n_in] = dU^T * A_prev^T ; dA_prev [R][n_in] = dU * W
       const __nv_bfloat16* prev_pt = j > 0 ? h->A_pt[l][j - 1] : (l == 0 ? h->xin_pt : h->N_pt[l]);
       const __nv_bfloat16* prev_p = j > 0 ? h->A_p[l][j - 1] : (l == 0 ? h->xin_p : h->N_p[l]);
       TRY(dw_job(DwOps{h->G_pt, prev_pt, h->G_p, Hp, prev_p, fc.n_in_pad}, fc.n_in_pad, Hp, fc.n_in_pad, Rp, grads + fc.w, size_t(fc.n_in) * 4,
                  size_t(fc.n_in) * 4, H));
       float* dprev = (da1 == h->dA) ? h->dB : h->dA;
-      TRY(gemm_into_block(h->G_p, fc.wtp, dprev, fc.n_in_pad, l, j - 1, nullptr, st));   // j - 1 == -1: the level's norm0
+      if (wide0)
+        pre_reduced = true;   // no dX GEMM: norm0's two reductions came from wide_grad_tile_kernel
+      else
+        TRY(gemm_into_block(h->G_p, fc.wtp, dprev, fc.n_in_pad, l, j - 1, nullptr, st));   // j - 1 == -1: the level's norm0
       da1 = dprev;
       da2 = nullptr;
     }
@@ -1573,9 +1800,10 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       pre_reduced = false;
       FBnBackward f{gi, acc, double(B) * F_in, grads + L.norm0.g, grads + L.norm0.b};
       // level 0: only the parameter gradients are needed (written by the prologue); still run one tile row so
-      // the prologue executes.  level > 0: fp32 gradient wrt E_{l-1}
-      TileOut o{nullptr, nullptr, l > 0 ? h->dEnext : nullptr, Hp, nullptr, l > 0 ? R : 1, l > 0 ? R : 1, F_in,
-                l > 0 ? Hp : 32};
+      // the prologue executes (with the wide first layer no element is evaluated: there is no dY).  level > 0: fp32
+      // gradient wrt E_{l-1}
+      TileOut o{nullptr, nullptr, l > 0 ? h->dEnext : nullptr, Hp, nullptr, l > 0 ? R : 1, l > 0 ? R : 1,
+                (l == 0 && h->wide) ? 0 : F_in, l > 0 ? Hp : 32};
       TRY(run_tile(f, o, st, "norm0 backward"));
     }
   }

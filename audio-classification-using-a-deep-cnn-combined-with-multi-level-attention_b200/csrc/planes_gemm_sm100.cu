@@ -578,12 +578,15 @@ static int planes_gemm_any(const void* a_planes, const void* b_planes, const flo
 // out [M][ldo] += sum_r A[r][m] B[r][n] over plane products: both operands stored ROW-major over the contraction index,
 // a_planes bf16 [K][planes * a_cols], b_planes bf16 [K][planes * b_cols] (the layout the forward / dX GEMMs consume), read
 // as MN-major UMMA operands — the weight-gradient GEMMs need no transposed copies of the activations and gradients.
-// M <= a_cols, N <= b_cols, both multiples of 128; K % 32 == 0; ksplit as in planes_gemm (> 1 or -1: out is added to).
+// M <= a_cols, N <= b_cols, both multiples of 128; K % 32 == 0; ksplit > 1 or -1: out is added to; ksplit 0: out is
+// overwritten with plain stores (outputs of many tiles and a short contraction, e.g. the 600 x 12288 weight gradient of
+// a wide first Linear at up to 1024 rows: 480 tiles of 128 x 128 fill the SMs without a K split).
 int planes_gemm_mn(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M,
                    int N, int K, int planes, int ksplit, cudaStream_t stream) {
   if (M <= 0) return 0;
   if (K % kBK != 0 || M % 128 != 0 || N % 128 != 0 || M > a_cols || N > b_cols || (planes != 2 && planes != 3) ||
-      (ksplit <= 1 && ksplit != -1)) {
+      (ksplit < 0 && ksplit != -1) || ksplit == 1 || ldo < N || !out ||
+      (ksplit == 0 && (ldo % 8 || (reinterpret_cast<uintptr_t>(out) & 31)))) {
     snprintf(g_perr, sizeof g_perr, "planes_gemm_mn: bad shape (M=%d N=%d K=%d planes=%d ksplit=%d)", M, N, K, planes, ksplit);
     return 1;
   }
@@ -609,6 +612,9 @@ int planes_gemm_mn(const void* a_planes, int a_cols, const void* b_planes, int b
   p.ksplit = ksplit;
   p.ldo = ldo;
   p.out = out;
+  if (ksplit == 0)
+    return planes == 3 ? launch_planes<3, false, 0, 128, true>(ta, tb, p, stream)
+                       : launch_planes<2, false, 0, 128, true>(ta, tb, p, stream);
   return planes == 3 ? launch_planes<3, true, 0, 128, true>(ta, tb, p, stream)
                      : launch_planes<2, true, 0, 128, true>(ta, tb, p, stream);
 }

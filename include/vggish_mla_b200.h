@@ -232,7 +232,14 @@ int vmb_mla_forward_fp32(vmb_mla_t* handle, const float* emb_dev, long long batc
  * owned by the handle, ordered after / before `stream` by events.  x / labels are copied into staging buffers owned by
  * the handle first and the seed is written to device memory, so any input addresses and any seed may follow; a distinct
  * (params, running, grads, loss, scores, batch, dropout_p) captures its own graph (four are kept).  Environment
- * VMB_TRAIN_GRAPH=0 keeps the eager launches; the results are the same either way. */
+ * VMB_TRAIN_GRAPH=0 keeps the eager launches; the results are the same either way.
+ * vmb_mla_trainer_create: 1..4 levels of 1..4 Linears, hidden and n_classes in 1..1024, T in 1..16, emb_in in
+ * 1..16384.  An emb_in wider than the hidden width (padded to 128: the just_bottlenecks head, emb_in = 12288) takes a
+ * wide-first-layer path: no gradient with respect to the input is formed (the CNN is frozen), only the forward and the
+ * weight-gradient GEMM run over the input width, and it needs the planes GEMM (VMB_PLANES_GEMM, VMB_TRAIN_MN_DW not 0).
+ * max_batch: 2 <= max_batch and max_batch * T <= 2^31 / 2048; with the wide path also
+ * pad64(max_batch * T) * 3 * pad128(emb_in) < 2^31 (the element count of the input's operand planes; 5824 clips at
+ * emb_in = 12288, T = 10).  A larger max_batch is rejected before anything is allocated. */
 long long vmb_mla_train_param_count(int n_levels, const int* n_fc, int emb_in, int hidden, int n_classes, int t_steps,
                                     long long* n_running_out);
 int vmb_mla_trainer_create(vmb_mla_trainer_t** handle, int n_levels, const int* n_fc, int emb_in, int hidden,
