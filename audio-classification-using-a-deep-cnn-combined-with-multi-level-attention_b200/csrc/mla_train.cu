@@ -1669,9 +1669,12 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     pre_reduced = false;
     return gemm(a, wt, nullptr, out, Hp, R, n_pad, Hp, s);
   };
+  // att / cla of one clip, [T][K] fp32 each: 128 KB at the largest accepted shape (T = 16, K = 1024)
+  const size_t att_smem = size_t(2) * T * K * sizeof(float);
   static std::atomic<unsigned long long> att_attr{0};   // one bit per device: the attribute is per device
   if (vmb::device_needs_setup(att_attr))
-    cudaFuncSetAttribute(att_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+    cudaFuncSetAttribute(att_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         int(2 * 16 * 1024 * sizeof(float)));
   auto att_branch = [&](int l, cudaStream_t s, bool own_side, float* out_dA) {
     const LevelRef& L = h->lvl[l];
     const __nv_bfloat16* e_pt = h->A_pt[l][L.n_fc - 1];
@@ -1683,7 +1686,6 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
                  params + L.normf.g, params + L.normf.b};
     double* acc_v = slotacc(L.normv.bslot);
     double* acc_f = slotacc(L.normf.bslot);
-    const size_t att_smem = (size_t(2) * T * K + K) * sizeof(float);
     att_backward_kernel<<<static_cast<unsigned>(B), 256, att_smem, s>>>(ap, h->Y, h->dY, h->ycols_pad, l * K,
                                                                         h->row_stats[l], gv, gf, Hp, acc_v, acc_f);
     vmb::count_launch();

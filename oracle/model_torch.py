@@ -71,9 +71,12 @@ def _bn_time(sd: dict, prefix: str, x: torch.Tensor, training: bool) -> torch.Te
                         sd[prefix + ".weight"], sd[prefix + ".bias"], training, 0.1, BN_EPS)
 
 
-def mla_forward(sd: dict, x: torch.Tensor, model_conf, training: bool = False, dropout_p: float = 0.0):
+def mla_forward(sd: dict, x: torch.Tensor, model_conf, training: bool = False, dropout_p: float = 0.0,
+                masks: dict | None = None, relu_pre: list | None = None):
     """x (B, T, M) -> (B, K) sigmoid scores.  training=True uses batch statistics (running stats are not
-    updated here) and dropout_p (the reference's DR = 0.4) if non-zero."""
+    updated here) and dropout_p (the reference's DR = 0.4) if non-zero.  `masks` {(level, j): (B, T, H) scale}
+    replaces F.dropout with given inverted-dropout scales (oracle.dropout_np.step_masks); `relu_pre` collects the
+    input of every ReLU."""
     embs = []
     h = x
     for lvl, n_fc in enumerate(model_conf):
@@ -81,8 +84,13 @@ def mla_forward(sd: dict, x: torch.Tensor, model_conf, training: bool = False, d
         h = _bn_time(sd, p + ".norm0", h, training)
         for j in range(n_fc):
             h = F.linear(h, sd[f"{p}.fc.{j}.weight"], sd[f"{p}.fc.{j}.bias"])
-            h = F.relu(_bn_time(sd, f"{p}.norms.{j}", h, training))
-            if training and dropout_p > 0:
+            h = _bn_time(sd, f"{p}.norms.{j}", h, training)
+            if relu_pre is not None:
+                relu_pre.append(h.detach())
+            h = F.relu(h)
+            if masks is not None:
+                h = h * torch.as_tensor(masks[(lvl, j)], dtype=h.dtype, device=h.device)
+            elif training and dropout_p > 0:
                 h = F.dropout(h, dropout_p, True)
         embs.append(h)
     ys = []
