@@ -53,6 +53,11 @@ SIGNATURES = {
     "vmb_vggish_destroy": (None, [_c_p]),
     "vmb_vggish_workspace_bytes": (_sz, [_ll]),
     "vmb_vggish_forward": (_int, [_c_p, _c_p, _ll, _c_p, _c_p, _c_p, _sz, _c_p]),
+    "vmb_vggish_fc_train_workspace_bytes": (_sz, [_ll]),
+    "vmb_vggish_fc_grad_count": (_ll, []),
+    "vmb_vggish_refresh_fc": (_int, [_c_p, C.POINTER(_c_p), C.POINTER(_c_p), _c_p]),
+    "vmb_vggish_forward_train": (_int, [_c_p, _c_p, _ll, _c_p, _c_p, _sz, _c_p]),
+    "vmb_vggish_fc_backward": (_int, [_c_p, _c_p, _sz, _c_p, _ll, _c_p, _c_p]),
     "vmb_mla_create": (_int, [C.POINTER(_c_p), _int, C.POINTER(_int), _int, _int, _int, _int, _c_p, _ll, _c_p]),
     "vmb_mla_destroy": (None, [_c_p]),
     "vmb_mla_num_classes": (_int, [_c_p]),
@@ -69,6 +74,7 @@ SIGNATURES = {
     "vmb_mla_train_wait_tail": (_int, [_c_p, _c_p]),
     "vmb_mla_train_forward": (_int, [_c_p, _c_p, _c_p, _c_p, _ll, C.c_float, C.c_ulonglong, _c_p, _c_p]),
     "vmb_mla_train_backward": (_int, [_c_p, _c_p, _c_p, _c_p, _ll, C.c_float, C.c_ulonglong, _c_p, _c_p]),
+    "vmb_mla_train_backward_dx": (_int, [_c_p, _c_p, _c_p, _c_p, _ll, C.c_float, C.c_ulonglong, _c_p, _c_p, _c_p]),
     "vmb_adam_step": (_int, [_c_p, _c_p, _c_p, _c_p, _ll, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _ll,
                              C.c_float, _c_p]),
     "vmb_dp_slice": (None, [_ll, _int, _int, C.POINTER(_ll), C.POINTER(_ll)]),

@@ -258,6 +258,91 @@ class VggishHandle:
                   "vmb_vggish_forward")
         return (emb, bott) if want_bottleneck else emb
 
+    # -- train-mode FC stack (fc1-fc3 trainable, convs frozen): csrc/fc_train.cu
+    @property
+    def fc_trainable(self) -> bool:
+        """True once refresh_fc() has derived the training copy of the FC weights."""
+        return bool(getattr(self, "_fc_refreshed", False))
+
+    def refresh_fc(self, weights, biases) -> None:
+        """Re-derive every device copy of the FC weights (inference copy and training planes) from fp32 masters
+        [embeddings.0/2/4.weight], [embeddings.0/2/4.bias] — stream-ordered, the conv weights are not touched."""
+        if not self.has_fc:
+            raise B200Error("this handle was built without the FC stack")
+        with torch.cuda.device(self.device):
+            keep = [t.detach().to(device=self.device, dtype=torch.float32).contiguous() for t in (*weights, *biases)]
+            fw = (C.c_void_p * 3)(*[t.data_ptr() for t in keep[:3]])
+            fb = (C.c_void_p * 3)(*[t.data_ptr() for t in keep[3:]])
+            check(_lib.lib().vmb_vggish_refresh_fc(self._h, fw, fb, stream_ptr()), "vmb_vggish_refresh_fc")
+            self._fc_keep = keep        # the masters' copies must outlive the enqueued kernels that read them
+        self._fc_refreshed = True
+
+    def _train_workspace(self, n: int):
+        need = int(_lib.lib().vmb_vggish_fc_train_workspace_bytes(n))
+        ws = getattr(self, "_train_ws", None)
+        if ws is None or ws.numel() < need + 1024:
+            self._train_ws = None
+            ws = self._train_ws = torch.empty(need + 1024, device=self.device, dtype=torch.uint8)
+        return (ws.data_ptr() + 1023) // 1024 * 1024, need
+
+    def forward_train(self, examples: torch.Tensor) -> torch.Tensor:
+        """(n, 96, 64) / (n, 1, 96, 64) fp32 CUDA -> (n, 128) fp32 embeddings, keeping what fc_backward() needs."""
+        self.check_saturation(synchronize=False)
+        examples = _need_cuda(examples, "examples")
+        if examples.dim() == 4 and examples.shape[1] == 1:
+            examples = examples[:, 0]
+        if examples.dim() != 3 or tuple(examples.shape[1:]) != (96, 64):
+            raise ValueError(f"examples must be (n, 1, 96, 64) or (n, 96, 64), got {tuple(examples.shape)}")
+        examples = examples.contiguous()
+        n = examples.shape[0]
+        emb = torch.empty((n, 128), device=self.device, dtype=torch.float32)
+        with torch.cuda.device(self.device):
+            base, need = self._train_workspace(n)
+            check(_lib.lib().vmb_vggish_forward_train(self._h, ptr(examples), n, ptr(emb), base, need, stream_ptr()),
+                  "vmb_vggish_forward_train")
+        self._train_n = n
+        return emb
+
+    def fc_backward(self, d_emb: torch.Tensor) -> torch.Tensor:
+        """d(loss)/d(emb) (n, 128) of the last forward_train -> flat fp32 FC gradients in state_dict order."""
+        n = getattr(self, "_train_n", None)
+        if n is None:
+            raise B200Error("fc_backward without a forward_train")
+        d = d_emb.to(device=self.device, dtype=torch.float32).contiguous()
+        if tuple(d.shape) != (n, 128):
+            raise ValueError(f"d_emb must be ({n}, 128), got {tuple(d.shape)}")
+        grads = torch.empty(int(_lib.lib().vmb_vggish_fc_grad_count()), device=self.device, dtype=torch.float32)
+        with torch.cuda.device(self.device):
+            base, need = self._train_workspace(n)
+            check(_lib.lib().vmb_vggish_fc_backward(self._h, base, need, ptr(d), n, ptr(grads), stream_ptr()),
+                  "vmb_vggish_fc_backward")
+        return grads
+
+    def train_features(self) -> torch.Tensor:
+        """(n, 12288) float64 conv features of the last forward_train, as its FC stack saw them (sum of the three
+        operand planes at the start of the workspace)."""
+        n = self._train_n
+        base, _ = self._train_workspace(n)
+        off = base - self._train_ws.data_ptr()
+        planes = self._train_ws[off:off + n * 3 * 12288 * 2].view(torch.bfloat16).view(n, 3, 12288)
+        return planes.double().sum(dim=1)
+
+
+FC_GRAD_LAYOUT = (("0.weight", (4096, 12288)), ("0.bias", (4096,)), ("2.weight", (4096, 4096)), ("2.bias", (4096,)),
+                  ("4.weight", (128, 4096)), ("4.bias", (128,)))
+
+
+def fc_grad_views(flat: torch.Tensor) -> dict:
+    """The flat FC gradient buffer as {embeddings key suffix: tensor view} in state_dict order."""
+    out, off = {}, 0
+    for key, shape in FC_GRAD_LAYOUT:
+        n = 1
+        for s in shape:
+            n *= s
+        out[key] = flat[off:off + n].view(shape)
+        off += n
+    return out
+
 
 def pack_mla_params(sd: dict, model_conf: Sequence[int], device: torch.device) -> torch.Tensor:
     """Flatten a MultiLevelAttention state_dict into the layout documented in vggish_mla_b200.h."""

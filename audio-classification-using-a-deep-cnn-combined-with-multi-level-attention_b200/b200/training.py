@@ -322,6 +322,7 @@ class _HeadTrainFn(torch.autograd.Function):
     def forward(ctx, module, x, *params):
         st = module._b200_train_state()
         tr: HeadTrainer = st["trainer"]
+        ctx.x_dtype = x.dtype
         x = x.detach().to(tr.device, torch.float32).contiguous()
         if x.shape[0] > tr.max_batch:
             raise B200Error(f"batch {x.shape[0]} > trainer capacity {tr.max_batch}")
@@ -349,22 +350,44 @@ class _HeadTrainFn(torch.autograd.Function):
         if ctx.param_key != tuple((p.data_ptr(), p._version) for _, p in ctx.module.named_parameters()):
             raise B200Error("the head's parameters changed between forward and backward")
         d = dscores.to(tr.device, torch.float32).contiguous()
+        dx = None
         with torch.cuda.device(tr.device):
-            check(_lib.lib().vmb_mla_train_backward(tr._h, ptr(tr.params), ptr(ctx.x), ptr(d), ctx.x.shape[0],
-                                                    float(tr.dropout_p), ctx.seed, ptr(tr.grads), stream_ptr()),
-                  "vmb_mla_train_backward")
+            if ctx.needs_input_grad[1]:
+                # the embeddings come from a trainable module (VGGish fc1-fc3): norm0's backward pass to its input too
+                dx = torch.empty_like(ctx.x)
+                check(_lib.lib().vmb_mla_train_backward_dx(tr._h, ptr(tr.params), ptr(ctx.x), ptr(d), ctx.x.shape[0],
+                                                           float(tr.dropout_p), ctx.seed, ptr(tr.grads), ptr(dx),
+                                                           stream_ptr()),
+                      "vmb_mla_train_backward_dx")
+            else:
+                check(_lib.lib().vmb_mla_train_backward(tr._h, ptr(tr.params), ptr(ctx.x), ptr(d), ctx.x.shape[0],
+                                                        float(tr.dropout_p), ctx.seed, ptr(tr.grads), stream_ptr()),
+                      "vmb_mla_train_backward")
         grads = []
         for name in st["param_names"]:
             grads.append(None if ".fcf." in name else tr.view(tr.grads, name).clone())
-        return (None, None, *grads)
+        if dx is not None and ctx.x_dtype != dx.dtype:
+            dx = dx.to(ctx.x_dtype)
+        return (None, dx, *grads)
+
+
+def input_grad_supported(emb_in: int, hidden: int, n_classes: int) -> bool:
+    """The head forms d(loss)/d(embeddings) only when the padded input width does not exceed the padded hidden width:
+    the wide first layer (just_bottlenecks, emb_in 12288) runs no dX GEMM."""
+    def pad(v):
+        return (v + 127) // 128 * 128
+    return pad(emb_in) <= max(pad(hidden), pad(n_classes))
 
 
 def head_train_forward(module, x: torch.Tensor) -> torch.Tensor:
-    """Train-mode forward of the reference-named head through the library (autograd-aware)."""
-    if isinstance(x, torch.Tensor) and x.requires_grad and torch.is_grad_enabled():
-        raise NotImplementedError("the head's backward pass produces parameter gradients only: the gradient with respect "
-                                  "to the embeddings is outside this path (the reference freezes the CNN, "
-                                  "model.py:159-160); pass x.detach()")
+    """Train-mode forward of the reference-named head through the library (autograd-aware).  When x requires grad
+    (a trainable module in front of the head, e.g. VGGish's fc1-fc3), backward also returns d(loss)/dx."""
+    if (isinstance(x, torch.Tensor) and x.requires_grad and torch.is_grad_enabled()
+            and not input_grad_supported(module.emb_input_size, module._h, module._k)):
+        raise NotImplementedError("the gradient with respect to the embeddings is formed only when the input width "
+                                  "is not wider than the hidden width; the wide first layer (just_bottlenecks, 12288-d "
+                                  "conv features) has no input gradient, and the VGGish conv stack cannot be trained "
+                                  "on this path (model.py:159-160); pass x.detach()")
     st = module._b200_train_state()
     st["sync_in"]()
     params = [p for _, p in module.named_parameters()]

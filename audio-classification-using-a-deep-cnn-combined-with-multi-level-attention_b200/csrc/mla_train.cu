@@ -1343,7 +1343,7 @@ enum { kPhaseForward = 1, kPhaseBackward = 2 };
 // One implementation for forward, backward and the fused step: the phases share the layout arithmetic.
 int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* running, const float* x,
                  const long long* labels, const float* dscores, long long batch, float dropout_p,
-                 unsigned long long seed, float* grads, float* loss, float* scores, void* stream) {
+                 unsigned long long seed, float* grads, float* loss, float* scores, void* stream, float* dx = nullptr) {
   if (!h) return fail("vmb_mla_train: null handle");
   if (!params || !x) return fail("vmb_mla_train: null pointer");
   if ((phases & kPhaseForward) && !running) return fail("vmb_mla_train: forward needs the running-statistics buffer");
@@ -1806,7 +1806,15 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       // gradient wrt E_{l-1}
       TileOut o{nullptr, nullptr, l > 0 ? h->dEnext : nullptr, Hp, nullptr, l > 0 ? R : 1, l > 0 ? R : 1,
                 (l == 0 && h->wide) ? 0 : F_in, l > 0 ? Hp : 32};
+      float* dx_pad = (da1 == h->dA) ? h->dB : h->dA;   // level 0 with dx: the chain buffer norm0's input does not use
+      if (l == 0 && dx) o = TileOut{nullptr, nullptr, dx_pad, Hp, nullptr, R, R, F_in, inpad};
       TRY(run_tile(f, o, st, "norm0 backward"));
+      if (l == 0 && dx && !rc &&
+          cudaMemcpy2DAsync(dx, size_t(F_in) * 4, dx_pad, size_t(Hp) * 4, size_t(F_in) * 4, size_t(R),
+                            cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+        vmb::set_kernel_error("dx copy failed");
+        rc = 1;
+      }
     }
   }
   before_g_overwrite();   // join: every weight gradient is in `grads` before anything the caller enqueues next
@@ -1947,6 +1955,18 @@ int vmb_mla_train_backward(vmb_mla_trainer_t* h, const float* params, const floa
   if (!dscores) return fail("vmb_mla_train_backward: null d(scores)");
   return train_phases(kPhaseBackward, h, params, nullptr, x, nullptr, dscores, batch, dropout_p, seed, grads, nullptr,
                       nullptr, stream);
+}
+
+int vmb_mla_train_backward_dx(vmb_mla_trainer_t* h, const float* params, const float* x, const float* dscores,
+                              long long batch, float dropout_p, unsigned long long seed, float* grads, float* dx,
+                              void* stream) {
+  if (!dscores) return fail("vmb_mla_train_backward_dx: null d(scores)");
+  if (!dx) return fail("vmb_mla_train_backward_dx: null dx");
+  if (h && h->wide)
+    return fail("vmb_mla_train_backward_dx: the input gradient is formed only when the padded input width does not "
+                "exceed the padded hidden width (the wide first layer runs no dX GEMM)");
+  return train_phases(kPhaseBackward, h, params, nullptr, x, nullptr, dscores, batch, dropout_p, seed, grads, nullptr,
+                      nullptr, stream, dx);
 }
 
 int vmb_adam_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, long long n, float lr,

@@ -5,8 +5,10 @@
 
 #include <cstdio>
 #include <cstring>
+#include <string>
 
 #include "../../include/vggish_mla_b200.h"
+#include "fc_train.cuh"
 #include "igemm_sm100.cuh"
 #include "kernels.cuh"
 
@@ -44,6 +46,11 @@ struct vmb_vggish {
   void* conv_w[6] = {};      // bf16 [C_out][9*C_in] (precision 1: [C_out][2*9*C_in] hi | lo), index 1..5
   void* fc_w[3] = {};        // bf16 [out][in]       (precision 1: [out][2*in] hi | lo)
   float* fc_b[3] = {};
+  // train-mode FC stack (fc_train.cu): three-plane copies of the FC weights, allocated and derived by the first
+  // vmb_vggish_refresh_fc — row-major [out][3 * in] for the forward GEMMs, transposed [in][3 * out] for the dgrad of
+  // fc2 and fc3 (fc1's input gradient is never formed)
+  void* train_w[3] = {};
+  void* train_wt[3] = {};
   HostStage stage;
 };
 
@@ -66,6 +73,50 @@ int fail(const char* fmt, const char* detail = "") {
 }
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// fp32 masters -> the inference copy of FC layer i in the handle's precision (create and refresh share it, so a
+// refreshed handle holds bit for bit what a fresh build would)
+bool fc_inference_copy(vmb_vggish* h, int i, const float* w, const float* b, cudaStream_t st) {
+  if (cudaMemcpyAsync(h->fc_b[i], b, size_t(kFcOut[i]) * 4, cudaMemcpyDeviceToDevice, st) != cudaSuccess) return false;
+  const int fmt = h->precision == 2 ? 1 : 0;
+  return (h->precision == 1 ? vmb::split_f32_to_planes(w, h->fc_w[i], kFcOut[i], kFcIn[i], st)
+                            : vmb::cast_f32_to_bf16(w, h->fc_w[i], static_cast<long long>(kFcOut[i]) * kFcIn[i], st,
+                                                    fmt)) == 0;
+}
+
+// conv1 + the five tensor-core convs into the ping-pong workspace; returns the buffer holding the (h, w, c)-flattened
+// features [n][12288] ([n][hi | lo] in split mode), or null after recording the error
+char* conv_stack(vmb_vggish* h, const float* examples, long long n, void* workspace, cudaStream_t st, const char* who) {
+  const bool split = h->precision == 1;
+  const int fmt = h->precision == 2 ? 1 : 0;
+  int* sat = h->sat;   // null unless fp16
+  const size_t mul = split ? 2 : 1;
+  char* A = static_cast<char*>(workspace);
+  char* B = A + align_up(size_t(n) * kBufA * mul, 1024);
+  {
+    vmb::StageTimer t(VMB_STAGE_CONV1, st);
+    if (vmb::conv1_tc_relu_pool(examples, h->conv1_w, h->conv_b[0], A, n, st, split, fmt, sat)) {
+      fail("%s", (std::string(who) + ": " + vmb::kernels_last_error()).c_str());
+      return nullptr;
+    }
+  }
+  char* src = A;
+  char* dst = B;
+  for (int i = 0; i < 5; ++i) {
+    const ConvGeom& g = kConv[i];
+    vmb::StageTimer t(VMB_STAGE_CONV2 + i, st);
+    const int rc = split ? vmb::igemm_conv3x3_split(src, h->conv_w[i + 1], h->conv_b[i + 1], dst, int(n), g.H, g.W, g.C_in,
+                                                    g.C_out, g.pool, st)
+                         : vmb::igemm_conv3x3(src, h->conv_w[i + 1], h->conv_b[i + 1], dst, int(n), g.H, g.W, g.C_in,
+                                              g.C_out, g.pool, st, fmt, sat ? sat + 1 + i : nullptr);
+    if (rc) {
+      fail("%s", (std::string(who) + ": " + vmb::igemm_last_error()).c_str());
+      return nullptr;
+    }
+    char* sw = src; src = dst; dst = sw;
+  }
+  return src;
+}
 
 }  // namespace
 
@@ -120,10 +171,7 @@ int vmb_vggish_create_ex(vmb_vggish_t** handle, const float* const conv_w[6], co
     dmalloc(&h->fc_w[i], size_t(kFcOut[i]) * kFcIn[i] * 2 * wmul);
     dmalloc(reinterpret_cast<void**>(&h->fc_b[i]), size_t(kFcOut[i]) * 4);
     if (!ok) break;
-    dcopy(h->fc_b[i], fc_b[i], size_t(kFcOut[i]) * 4);
-    ok = ok && (precision == 1 ? vmb::split_f32_to_planes(fc_w[i], h->fc_w[i], kFcOut[i], kFcIn[i], st)
-                               : vmb::cast_f32_to_bf16(fc_w[i], h->fc_w[i], static_cast<long long>(kFcOut[i]) * kFcIn[i], st,
-                                                       fmt)) == 0;
+    ok = ok && fc_inference_copy(h, i, fc_w[i], fc_b[i], st);
   }
   ok = ok && cudaStreamSynchronize(st) == cudaSuccess;
   if (!ok) {
@@ -145,6 +193,8 @@ void vmb_vggish_destroy(vmb_vggish_t* h) {
   for (int i = 0; i < 3; ++i) {
     cudaFree(h->fc_w[i]);
     cudaFree(h->fc_b[i]);
+    cudaFree(h->train_w[i]);
+    cudaFree(h->train_wt[i]);
   }
   if (h->sat) cudaFreeHost(h->sat);
   HostStage& hs = h->stage;
@@ -200,24 +250,9 @@ int vmb_vggish_forward(vmb_vggish_t* h, const float* examples, long long n, floa
   const size_t mul = split ? 2 : 1;
   char* A = static_cast<char*>(workspace);
   char* B = A + align_up(size_t(n) * kBufA * mul, 1024);
-
-  {
-    vmb::StageTimer t(VMB_STAGE_CONV1, st);
-    if (vmb::conv1_tc_relu_pool(examples, h->conv1_w, h->conv_b[0], A, n, st, split, fmt, sat))
-      return fail("vmb_vggish_forward: %s", vmb::kernels_last_error());
-  }
-  char* src = A;
-  char* dst = B;
-  for (int i = 0; i < 5; ++i) {
-    const ConvGeom& g = kConv[i];
-    vmb::StageTimer t(VMB_STAGE_CONV2 + i, st);
-    const int rc = split ? vmb::igemm_conv3x3_split(src, h->conv_w[i + 1], h->conv_b[i + 1], dst, int(n), g.H, g.W, g.C_in,
-                                                    g.C_out, g.pool, st)
-                         : vmb::igemm_conv3x3(src, h->conv_w[i + 1], h->conv_b[i + 1], dst, int(n), g.H, g.W, g.C_in,
-                                              g.C_out, g.pool, st, fmt, sat ? sat + 1 + i : nullptr);
-    if (rc) return fail("vmb_vggish_forward: %s", vmb::igemm_last_error());
-    char* sw = src; src = dst; dst = sw;
-  }
+  char* src = conv_stack(h, examples, n, workspace, st, "vmb_vggish_forward");
+  if (!src) return 1;
+  char* dst = src == A ? B : A;
   // src == B now holds the NHWC [n][6][4][512] features == the (h,w,c)-flattened [n][12288] matrix (vggish.py:26-29);
   // in split mode [n][hi(12288) | lo(12288)]
   if (bottleneck) {
@@ -245,6 +280,99 @@ int vmb_vggish_forward(vmb_vggish_t* h, const float* examples, long long n, floa
   }
   return 0;
 }
+
+// ------------------------------------------------------------------------------------------ train-mode FC stack
+namespace {
+// the conv scratch of the train-mode workspace is sized for the split precision (the largest)
+vmb::FcTrainLayout train_layout(long long n) { return vmb::fc_train_layout(n, vmb_vggish_workspace_bytes(n) * 2); }
+
+int check_train_args(const vmb_vggish_t* h, long long n, const void* ws, size_t ws_bytes, const char* who) {
+  char msg[256];
+  auto bad = [&](const char* why) {
+    snprintf(msg, sizeof msg, "%s: %s", who, why);
+    return fail("%s", msg);
+  };
+  if (!h) return bad("null handle");
+  if (!h->has_fc) return bad("this handle was built without the FC stack (bottleneck features only)");
+  if (!h->train_w[0]) return bad("no training copy of the FC weights: call vmb_vggish_refresh_fc first");
+  if (n < 1) return bad("n must be at least 1");
+  if (n > 1000000) return bad("at most 1 000 000 examples per call");
+  if (!ws) return bad("null workspace");
+  if (reinterpret_cast<uintptr_t>(ws) % 1024) return bad("workspace must be 1024-byte aligned");
+  if (ws_bytes < train_layout(n).total) return bad("workspace too small for n examples");
+  return 0;
+}
+}  // namespace
+
+extern "C" {
+
+size_t vmb_vggish_fc_train_workspace_bytes(long long n) {
+  if (n <= 0) return 0;
+  return train_layout(n).total;
+}
+
+long long vmb_vggish_fc_grad_count(void) { return vmb::kFcGradCount; }
+
+int vmb_vggish_refresh_fc(vmb_vggish_t* h, const float* const fc_w[3], const float* const fc_b[3], void* stream) {
+  if (!h) return fail("vmb_vggish_refresh_fc: null handle");
+  if (!h->has_fc) return fail("vmb_vggish_refresh_fc: this handle was built without the FC stack");
+  if (!fc_w || !fc_b) return fail("vmb_vggish_refresh_fc: null argument");
+  for (int i = 0; i < 3; ++i)
+    if (!fc_w[i] || !fc_b[i]) return fail("vmb_vggish_refresh_fc: null fc tensor");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  bool ok = true;
+  for (int i = 0; i < 3 && ok; ++i) {   // first call: the training copies (the only allocation; later calls reuse them)
+    if (!h->train_w[i])
+      ok = cudaMalloc(&h->train_w[i], size_t(kFcOut[i]) * kFcIn[i] * 2 * 3) == cudaSuccess;
+    if (ok && i > 0 && !h->train_wt[i])
+      ok = cudaMalloc(&h->train_wt[i], size_t(kFcOut[i]) * kFcIn[i] * 2 * 3) == cudaSuccess;
+  }
+  if (!ok) {
+    for (int i = 0; i < 3; ++i) {
+      cudaFree(h->train_w[i]);
+      cudaFree(h->train_wt[i]);
+      h->train_w[i] = h->train_wt[i] = nullptr;
+    }
+    return fail("vmb_vggish_refresh_fc: allocation failed (%s)", cudaGetErrorString(cudaGetLastError()));
+  }
+  for (int i = 0; i < 3; ++i) {
+    if (!fc_inference_copy(h, i, fc_w[i], fc_b[i], st))
+      return fail("vmb_vggish_refresh_fc: %s", vmb::kernels_last_error());
+    if (vmb::fc_weight_planes(fc_w[i], kFcOut[i], kFcIn[i], h->train_w[i], h->train_wt[i], st))
+      return fail("vmb_vggish_refresh_fc: %s", vmb::kernels_last_error());
+  }
+  return 0;
+}
+
+int vmb_vggish_forward_train(vmb_vggish_t* h, const float* examples, long long n, float* emb, void* workspace,
+                             size_t workspace_bytes, void* stream) {
+  if (check_train_args(h, n, workspace, workspace_bytes, "vmb_vggish_forward_train")) return 1;
+  if (!examples || !emb) return fail("vmb_vggish_forward_train: null pointer");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const vmb::FcTrainLayout L = train_layout(n);
+  char* ws = static_cast<char*>(workspace);
+  const char* feat = conv_stack(h, examples, n, ws + L.conv, st, "vmb_vggish_forward_train");
+  if (!feat) return 1;
+  const void* w[3] = {h->train_w[0], h->train_w[1], h->train_w[2]};
+  const float* b[3] = {h->fc_b[0], h->fc_b[1], h->fc_b[2]};
+  if (vmb::fc_train_forward(w, b, feat, h->precision, n, ws, L, emb, st))
+    return fail("vmb_vggish_forward_train: %s", vmb::kernels_last_error());
+  return 0;
+}
+
+int vmb_vggish_fc_backward(vmb_vggish_t* h, void* workspace, size_t workspace_bytes, const float* d_emb, long long n,
+                           float* grads, void* stream) {
+  if (check_train_args(h, n, workspace, workspace_bytes, "vmb_vggish_fc_backward")) return 1;
+  if (!d_emb || !grads) return fail("vmb_vggish_fc_backward: null pointer");
+  if (reinterpret_cast<uintptr_t>(grads) % 32) return fail("vmb_vggish_fc_backward: grads must be 32-byte aligned");
+  const void* wt[3] = {nullptr, h->train_wt[1], h->train_wt[2]};
+  if (vmb::fc_train_backward(wt, n, static_cast<char*>(workspace), train_layout(n), d_emb, grads,
+                             static_cast<cudaStream_t>(stream)))
+    return fail("vmb_vggish_fc_backward: %s", vmb::kernels_last_error());
+  return 0;
+}
+
+}  // extern "C"
 
 // ------------------------------------------------------------------------------------------ whole path
 namespace {

@@ -62,6 +62,46 @@ class B200HandleMixin:
         return tuple((t.data_ptr(), t._version) for t in tensors) + (str(dev),)
 
 
+def handle_action(old_key, new_key, fc_trainable: bool) -> str:
+    """What a change of the VGGish parameters does to the library handle.  A key is (conv part, FC part): the conv
+    part covers the conv tensors and the precision, the FC part the embeddings.* tensors.  "rebuild" (a new handle:
+    vmb_vggish_create_ex re-lays every weight and synchronises), "refresh" (only the FC weights changed and the handle
+    already holds a training copy of them: vmb_vggish_refresh_fc, stream-ordered), or "keep"."""
+    if old_key is None or old_key[0] != new_key[0]:
+        return "rebuild"
+    if old_key[1] != new_key[1]:
+        return "refresh" if fc_trainable else "rebuild"
+    return "keep"
+
+
+class _FcTrainFn(torch.autograd.Function):
+    """Train-mode VGGish with the conv stack frozen and fc1-fc3 trainable: the conv features and the FC stack's
+    activations stay in the handle's train workspace, which holds ONE forward: backward checks it is still this one."""
+
+    @staticmethod
+    def forward(ctx, module, x, *params):
+        h = module._b200_handle(train=True)
+        emb = h.forward_train(x.detach().to(device=h.device, dtype=torch.float32))
+        module._fc_generation = getattr(module, "_fc_generation", 0) + 1
+        ctx.module, ctx.handle, ctx.generation = module, h, module._fc_generation
+        ctx.param_key = tuple((p.data_ptr(), p._version) for p in params)
+        return emb
+
+    @staticmethod
+    def backward(ctx, d_emb):
+        m = ctx.module
+        if ctx.generation != getattr(m, "_fc_generation", 0) or m._handle is not ctx.handle:
+            raise B200Error("backward of a stale VGGish forward: the library keeps the activations of ONE train-mode "
+                            "forward per module, and another train-mode forward ran before this backward; call "
+                            "backward() before the next forward")
+        if ctx.param_key != tuple((p.data_ptr(), p._version) for p in m.embeddings.parameters()):
+            raise B200Error("the VGGish FC parameters changed between forward and backward")
+        views = _engine.fc_grad_views(ctx.handle.fc_backward(d_emb))
+        names = [k for k, _ in m.embeddings.named_parameters()]
+        grads = [views[k] if ctx.needs_input_grad[2 + i] else None for i, k in enumerate(names)]
+        return (None, None, *grads)
+
+
 def _body_tensors(features, embeddings):
     named = [(f"features.{k}", v) for k, v in features.named_parameters()]
     if embeddings is not None:
@@ -95,25 +135,39 @@ class VGG(B200HandleMixin, nn.Module):
         self.b200_precision = precision
         return self
 
-    # -- library handle, rebuilt when a parameter was modified in place, replaced or moved
-    def _b200_handle(self):
+    # -- library handle: rebuilt when a conv parameter was modified in place, replaced or moved; a change of the FC
+    # parameters alone (an optimiser step of FC fine-tuning) refreshes the FC weights of the existing handle
+    def _b200_handle(self, train: bool = False):
         named = _body_tensors(self.features, self.embeddings)
         dev = named[0][1].device
         if dev.type != "cuda":
             raise B200Error("VGGish parameters are on %s: move the module to a CUDA device (.to('cuda')); this build "
                             "has no CPU path" % dev)
-        key = self._tensor_key((v for _, v in named), dev) + (self.b200_precision,)
-        if self._handle is None or key != self._handle_key:
+        fc = [v for _, v in self.embeddings.named_parameters()]
+        key = (self._tensor_key(self.features.parameters(), dev) + (self.b200_precision,), self._tensor_key(fc, dev))
+        action = handle_action(self._handle_key if self._handle is not None else None, key,
+                               self._handle is not None and self._handle.fc_trainable)
+        if action == "rebuild":
             if self._handle is not None:
                 self._handle.close()
             self._handle = _engine.VggishHandle(dict(named), dev, precision=self.b200_precision)
-            self._handle_key = key
+        if action == "refresh" or (train and not self._handle.fc_trainable):
+            self._handle.refresh_fc(fc[0::2], fc[1::2])
+        self._handle_key = key
         return self._handle
 
     def forward(self, x):
-        if any(p.requires_grad for p in self.parameters()) and torch.is_grad_enabled() and self.training:
-            raise NotImplementedError("training the VGGish body is outside the B200 path (the reference freezes it, "
-                                      "model.py:159-160); call set_requires_grad(module, False) or .eval()")
+        if torch.is_grad_enabled() and self.training:
+            if any(p.requires_grad for p in self.features.parameters()):
+                raise NotImplementedError("training the VGGish conv stack is outside the B200 path (the reference "
+                                          "freezes it, model.py:159-160); fine-tuning the FC stack alone "
+                                          "(set_requires_grad(vgg.embeddings, True)) is supported; otherwise call "
+                                          "set_requires_grad(module, False) or .eval()")
+            fc = list(self.embeddings.parameters())
+            if any(p.requires_grad for p in fc):
+                if not isinstance(x, torch.Tensor):
+                    raise TypeError("expected a (N, 1, 96, 64) tensor")
+                return _FcTrainFn.apply(self, x, *fc)
         h = self._b200_handle()
         if not isinstance(x, torch.Tensor):
             raise TypeError("expected a (N, 1, 96, 64) tensor")

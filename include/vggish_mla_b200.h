@@ -184,6 +184,32 @@ size_t vmb_vggish_handle_workspace_bytes(const vmb_vggish_t* handle, long long n
 int vmb_vggish_forward(vmb_vggish_t* handle, const float* examples_dev, long long n, float* emb_dev,
                        void* bottleneck_bf16_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------ VGGish FC fine-tuning
+ * Training embeddings.{0,2,4} (fc1-fc3, vggish.py:13-19,31) with the conv stack frozen: the reference's loop with the
+ * CNN's FC parameters given to its Adam (train.py:133-138, the optimiser of train.py:370).  The conv stack runs exactly
+ * as in vmb_vggish_forward (same kernels, the handle's precision); the FC stack runs on three-plane split-bf16 operands
+ * (hi | mid | lo, fp32-equivalent, the head trainer's GEMMs) from a training copy of the weights that
+ * vmb_vggish_refresh_fc derives.  The input gradient of fc1 is not formed.
+ *
+ * vmb_vggish_refresh_fc: fp32 masters fc_w_dev[i] [out][in], fc_b_dev[i] [out] -> every device copy of the FC weights
+ *   (the inference copy in the handle's precision, bit for bit what vmb_vggish_create_ex would build, and the training
+ *   planes).  Stream-ordered, no synchronisation; the first call allocates the training planes (~0.5 GB).
+ * vmb_vggish_forward_train: examples fp32 [n][96][64] -> emb_dev fp32 [n][128] (post-ReLU embeddings).  The workspace
+ *   (vmb_vggish_fc_train_workspace_bytes(n), 1024-byte aligned) keeps what the backward pass needs; it begins with the
+ *   operand planes of the conv features, bf16 [pad64(n)][3][12288] (hi, mid, lo: their sum is the fp32 feature).
+ * vmb_vggish_fc_backward: d(loss)/d(emb) fp32 [n][128] of the last vmb_vggish_forward_train on this workspace ->
+ *   grads_dev, one flat fp32 buffer of vmb_vggish_fc_grad_count() floats (32-byte aligned) in state_dict order:
+ *   embeddings.0.weight [4096][12288], .0.bias [4096], .2.weight [4096][4096], .2.bias [4096], .4.weight [128][4096],
+ *   .4.bias [128].  Every element is written.                                                                  */
+size_t vmb_vggish_fc_train_workspace_bytes(long long n_examples);
+long long vmb_vggish_fc_grad_count(void);
+int vmb_vggish_refresh_fc(vmb_vggish_t* handle, const float* const fc_w_dev[3], const float* const fc_b_dev[3],
+                          void* stream);
+int vmb_vggish_forward_train(vmb_vggish_t* handle, const float* examples_dev, long long n, float* emb_dev,
+                             void* workspace_dev, size_t workspace_bytes, void* stream);
+int vmb_vggish_fc_backward(vmb_vggish_t* handle, void* workspace_dev, size_t workspace_bytes, const float* d_emb_dev,
+                           long long n, float* grads_dev, void* stream);
+
 /* ------------------------------------------------------------------------------------------ MLA head
  * MultiLevelAttention.forward in eval mode (model.py:258-269; EmbeddedMapping :217-222, AttentionModule
  * :236-242).  `params_dev` is one flat fp32 device buffer holding, in this order (T = time steps):
@@ -263,6 +289,13 @@ int vmb_mla_train_forward(vmb_mla_trainer_t* handle, const float* params_dev, fl
 int vmb_mla_train_backward(vmb_mla_trainer_t* handle, const float* params_dev, const float* emb_dev,
                            const float* dscores_dev, long long batch, float dropout_p, unsigned long long seed,
                            float* grads_dev, void* stream);
+/* vmb_mla_train_backward plus the gradient with respect to the embeddings, dx_dev fp32 [batch][T][emb_in] (the input of
+ * a trainable CNN body in front of the head, train.py:133-138 with the optimiser of train.py:370): norm0's backward
+ * pass to its input, dx = gamma_t rstd_t (g - mean_t g - xhat mean_t(g xhat)).  Only when the padded emb_in does not
+ * exceed the padded hidden width (the wide first layer has no dX GEMM): otherwise it fails.                      */
+int vmb_mla_train_backward_dx(vmb_mla_trainer_t* handle, const float* params_dev, const float* emb_dev,
+                              const float* dscores_dev, long long batch, float dropout_p, unsigned long long seed,
+                              float* grads_dev, float* dx_dev, void* stream);
 /* torch.optim.Adam (amsgrad = False) on flat buffers (train.py:369): step counts from 1; grads are multiplied by
  * grad_scale first (1/world_size after a SUM all-reduce).                                                 */
 int vmb_adam_step(float* params_dev, const float* grads_dev, float* exp_avg_dev, float* exp_avg_sq_dev, long long n,
