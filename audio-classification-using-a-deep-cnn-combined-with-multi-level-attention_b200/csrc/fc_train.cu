@@ -13,9 +13,9 @@
 // Contractions longer than kFwdSlice columns (fc1: 12 288, fc2 / fc3 and the dgrad of fc2: 4 096) are cut into K slices
 // that run on different SMs and add into a zeroed fp32 output: one tcgen05 accumulator over 768 K-steps truncates
 // enough to miss the oracle (the wide head layer, DESIGN §5.5), slices of 768 columns do not.  The weight gradients
-// contract over the B*T rows in slices of at most kDwSlice rows, as the head trainer's do.  Between GEMMs one
-// element-wise pass per layer applies the ReLU (forward) or the ReLU mask (backward), writes the next operand planes and,
-// in the backward pass, the column sums that are the bias gradient.
+// contract over the B*T rows in slices of at most kDwSlice rows (planes_gemm_dw, shared with the head trainer).
+// Between GEMMs one element-wise pass per layer applies the ReLU (forward) or the ReLU mask (backward), writes the next
+// operand planes and, in the backward pass, the column sums that are the bias gradient.
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
@@ -32,20 +32,12 @@ namespace vmb {
 namespace {
 
 constexpr int kPl = 3;
-constexpr int kFwdSlice = 768, kDwSlice = 1024;
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-__device__ __forceinline__ void split3(float v, __nv_bfloat16& hi, __nv_bfloat16& mid, __nv_bfloat16& lo) {
-  hi = __float2bfloat16_rn(v);
-  const float r1 = v - __bfloat162float(hi);      // exact
-  mid = __float2bfloat16_rn(r1);
-  lo = __float2bfloat16_rn(r1 - __bfloat162float(mid));
-}
-
 __device__ __forceinline__ void store3(float v, __nv_bfloat16* dst, long long plane_stride) {
   __nv_bfloat16 h, m, l;
-  split3(v, h, m, l);
+  split_bf16(v, h, m, l);
   dst[0] = h;
   dst[plane_stride] = m;
   dst[2 * plane_stride] = l;
@@ -163,20 +155,10 @@ int gemm(const void* a, const void* w, const float* bias, float* out, long long 
   return 0;
 }
 
-// dW fp32 [M][N] = sum over the K rows of a[r][m] b[r][n]: the head trainer's slicing (gemm_dw_mn, mla_train.cu)
+// dW fp32 [M][N] = sum over the K rows of a[r][m] b[r][n]
 int gemm_dw(const void* a, int a_cols, const void* b, int b_cols, float* out, int M, int N, long long K,
             cudaStream_t st) {
-  const int mn = (M / 128) * (N / 128);
-  int ks = num_sms() / mn;
-  if (ks == 0) ks = int((K + kDwSlice - 1) / kDwSlice);
-  const bool plain = ks == 1 && mn > num_sms();
-  if (ks > K / 32 / 4) ks = int(K / 32 / 4);
-  if (ks < 1) ks = 1;
-  if (!plain && cudaMemsetAsync(out, 0, size_t(M) * N * sizeof(float), st) != cudaSuccess) {
-    set_kernel_error("fc_train: dW clear failed");
-    return 1;
-  }
-  if (planes_gemm_mn(a, a_cols, b, b_cols, out, N, M, N, int(K), kPl, plain ? 0 : ks > 1 ? ks : -1, st)) {
+  if (planes_gemm_dw(a, a_cols, b, b_cols, out, N, M, N, int(K), kPl, st)) {
     set_kernel_error("fc_train: %s", planes_gemm_last_error());
     return 1;
   }

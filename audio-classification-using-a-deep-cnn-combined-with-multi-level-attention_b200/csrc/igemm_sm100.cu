@@ -729,64 +729,6 @@ int igemm_linear_split(const void* a_planes, const void* w_planes, const float* 
                         : launch<128, 1, false, false, kOutF32>(ta, tb, p, stream);
 }
 
-int igemm_linear_split_ksplit(const void* a_planes, const void* w_planes, float* out_zeroed, long long ldo, int M, int N,
-                              int K, cudaStream_t stream, int planes) {
-  if (M <= 0) return 0;
-  if (misaligned32(out_zeroed, "igemm_linear_split_ksplit")) return 1;
-  if (ldo % 4 != 0) {
-    snprintf(g_err, sizeof g_err, "igemm_linear_split_ksplit: ldo must be a multiple of 4 floats (16-byte vector reductions)");
-    return 1;
-  }
-  if (K % kBlockK != 0 || N % 128 != 0 || (planes != 2 && planes != 3)) {
-    snprintf(g_err, sizeof g_err, "igemm_linear_split_ksplit: need K %% 64 == 0, N %% 128 == 0, planes 2|3 (K=%d N=%d)", K, N);
-    return 1;
-  }
-  if (planes_gemm_enabled()) {
-    // one wave of (K slice, tile) work items, each slice at least four 32-column K-blocks long
-    const int mn = ((M + kBlockM - 1) / kBlockM) * (N / 128);
-    int ks = num_sms() / mn;
-    if (ks > K / 32 / 4) ks = K / 32 / 4;
-    if (ks < 1) ks = 1;
-    if (planes_gemm(a_planes, w_planes, nullptr, out_zeroed, ldo, 0, M, N, K, planes, ks > 1 ? ks : -1, stream)) {
-      snprintf(g_err, sizeof g_err, "%s", planes_gemm_last_error());
-      return 1;
-    }
-    return 0;
-  }
-  CUtensorMap ta, tb;
-  {
-    uint64_t dims[2] = {uint64_t(planes) * K, uint64_t(M)};
-    uint64_t str[1] = {uint64_t(planes) * K * 2};
-    uint32_t box[2] = {kBlockK, kBlockM};
-    if (make_tmap_bf16(&ta, a_planes, 2, dims, str, box)) return 1;
-  }
-  {
-    uint64_t dims[2] = {uint64_t(planes) * K, uint64_t(N)};
-    uint64_t str[1] = {uint64_t(planes) * K * 2};
-    uint32_t box[2] = {kBlockK, 128};
-    if (make_tmap_bf16(&tb, w_planes, 2, dims, str, box)) return 1;
-  }
-  IgemmParams p{};
-  p.M = M;
-  p.N = N;
-  p.split_nkb = K / kBlockK;
-  p.split_planes = planes;
-  p.num_kb = (planes == 3 ? 6 : 3) * p.split_nkb;
-  p.num_m_tiles = (M + kBlockM - 1) / kBlockM;
-  p.num_n_tiles = N / 128;
-  // as many K slices as fit in ONE wave of tiles (rounding up would leave a second wave of a few tiles that doubles the
-  // kernel's time: 25 output tiles x 6 slices = 150 tiles on 148 SMs), each slice at least 8 K-blocks long
-  const int mn = p.num_m_tiles * p.num_n_tiles;
-  int ks = num_sms() / mn;
-  if (ks > p.num_kb / 8) ks = p.num_kb / 8;
-  p.ksplit = ks < 1 ? 1 : ks;
-  p.relu = 0;
-  p.ldo = ldo;
-  p.bias = nullptr;
-  p.out = out_zeroed;
-  return launch<128, 1, false, false, kOutF32Atomic>(ta, tb, p, stream);
-}
-
 int igemm_linear_split_out(const void* a_planes, const void* w_planes, const float* bias, void* out_planes, int relu,
                            int M, int N, int K, cudaStream_t stream) {
   if (M <= 0) return 0;

@@ -22,6 +22,7 @@
 // walks K in the same (channel block, dx, dy) order, so their results are bit-identical.
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <cstdint>
 
@@ -67,10 +68,6 @@ int igemm_linear(const void* a_bf16, const void* w_bf16, const float* bias, void
 // must not flip against the fp32 reference).  bias may be null.  K % 64 == 0, N % 128 == 0.
 int igemm_linear_split(const void* a_planes, const void* w_planes, const float* bias, float* out, long long ldo,
                        int relu, int M, int N, int K, cudaStream_t stream, int planes = 2);
-// Split-K variant for tall contractions (the dW GEMMs of head training: K = batch * T rows, only a few output tiles):
-// the K loop is cut into slices that run on different SMs and atomically add into out, which must be zero on entry.
-int igemm_linear_split_ksplit(const void* a_planes, const void* w_planes, float* out_zeroed, long long ldo, int M, int N,
-                              int K, cudaStream_t stream, int planes);
 // Split in, split out (the accuracy mode of the VGGish body): out planes bf16 [M][hi(N) | lo(N)] =
 // split(act(A_hi W_hi^T + A_lo W_hi^T + A_hi W_lo^T + bias)).  K % 64 == 0, N % 256 == 0.
 int igemm_linear_split_out(const void* a_planes, const void* w_planes, const float* bias, void* out_planes, int relu,
@@ -121,9 +118,17 @@ __device__ __forceinline__ float dropout_scale(unsigned long long seed, unsigned
   return u >= p ? 1.f / (1.f - p) : 0.f;
 }
 
+// The three-plane split of the training GEMMs' operands (hi | mid | lo, planes = 3 above): fp32-equivalent operands.
+__device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bfloat16& mid, __nv_bfloat16& lo) {
+  hi = __float2bfloat16_rn(v);
+  const float r1 = v - __bfloat162float(hi);      // exact
+  mid = __float2bfloat16_rn(r1);
+  lo = __float2bfloat16_rn(r1 - __bfloat162float(mid));
+}
+
 // planes_gemm_sm100.cu: the split GEMMs with every operand plane of a K-block loaded once per tile and the hi * hi
-// product in its own TMEM accumulator.  igemm_linear_split / igemm_linear_split_ksplit route to it when
-// planes_gemm_enabled() (default; env VMB_PLANES_GEMM=0 or planes_gemm_set(0) selects the long-K-loop kernel above).
+// product in its own TMEM accumulator.  The training paths call it directly; igemm_linear_split (the eval-mode head)
+// routes to it when planes_gemm_enabled() (default; env VMB_PLANES_GEMM=0 selects the long-K-loop kernel above).
 // ksplit > 1: that many K slices, vector reductions into a zeroed out; ksplit == -1: one slice but still adding into
 // out; ksplit == 0: plain stores (+ bias, optional ReLU).
 int planes_gemm(const void* a_planes, const void* b_planes, const float* bias, float* out, long long ldo, int relu, int M,
@@ -179,8 +184,18 @@ int planes_gemm_stats(const void* a_planes, const void* b_planes, const float* b
 // ksplit > 1 or -1: K slices added into out with vector reductions (out zeroed by the caller); ksplit 0: plain stores.
 int planes_gemm_mn(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M,
                    int N, int K, int planes, int ksplit, cudaStream_t stream);
+// Contraction lengths per tcgen05 accumulator of the three-plane training GEMMs: one accumulator summed over thousands
+// of K steps truncates enough to miss the fp32 reference, so a longer contraction is cut into slices whose fp32 partial
+// sums are added in the output.  Forward GEMMs slice their input columns by kFwdSlice (the caller zeroes the output and
+// passes the slice count as ksplit); planes_gemm_dw slices the rows of a weight gradient by at most kDwSlice.
+constexpr int kFwdSlice = 768, kDwSlice = 1024;
+// Weight gradient of a training Linear, dW = G^T A over the rows: planes_gemm_mn with one wave of (K slice, tile)
+// work items, each slice at least four 32-row K-blocks long.  An output of more tiles than SMs (the 12288-wide first
+// layer of the head) is split only into slices of at most kDwSlice rows, and with one slice stored plainly.  Clears
+// out (M rows of ldo floats) on the stream first whenever the slices add into it.
+int planes_gemm_dw(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M,
+                   int N, int K, int planes, cudaStream_t stream);
 bool planes_gemm_enabled();
-int planes_gemm_set(int on);   // 1 / 0 force the choice, -1 returns to the default; returns the previous setting
 const char* planes_gemm_last_error();
 
 // Shared host helpers (igemm_sm100.cu): bf16 tensor map with 128- or 64-byte swizzle (error text goes to

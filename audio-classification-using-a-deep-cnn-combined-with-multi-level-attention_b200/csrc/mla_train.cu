@@ -5,14 +5,15 @@
 // nn.CrossEntropyLoss applied to the sigmoid outputs (train.py:131,372).  Running statistics are updated like
 // nn.BatchNorm1d does (momentum 0.1, unbiased variance).
 //
-// Every Linear (forward, dX and dW) is a 3-plane split-bf16 tcgen05 GEMM (igemm_linear_split with hi | mid | lo
+// Every Linear (forward, dX and dW) is a 3-plane split-bf16 tcgen05 GEMM (planes_gemm_sm100.cu with hi | mid | lo
 // operands = fp32-equivalent: with 2 planes the 4e-5 error on pre-activations flipped a few ReLU masks per step against
-// the fp32 reference, which moves whole gradient elements); everything between GEMMs
-// is fp32 CUDA-core work in a handful of kernels:
+// the fp32 reference, which moves whole gradient elements).  The dW GEMMs read the same row-major planes as the forward
+// and dX GEMMs, as MN-major operands (planes_gemm_dw).  Everything between GEMMs is fp32 CUDA-core work in a handful of
+// kernels:
 //   bn_time_stats / bn_col_stats   sum and sum-of-squares per time step (or per class), finalised by the last block
-//   tile_split<Functor>            32x32 tiles: evaluate an element-wise functor (BN + ReLU + dropout, BN backward, ...),
-//                                  write hi|lo bf16 planes row-major AND transposed (the dW GEMMs contract over rows),
-//                                  optionally the fp32 values and the column sums (bias gradients)
+//   tile_split<Functor>            64x64 tiles: evaluate an element-wise functor (BN + ReLU + dropout, BN backward),
+//                                  write hi|mid|lo bf16 planes row-major (the weights also transposed: the dX GEMMs'
+//                                  B operand), optionally the fp32 values and the column sums (bias gradients)
 //   att_forward / att_backward     attention pooling over the T time steps of one clip per CTA
 //   out_loss_rows / out_bn_backward  sigmoid + cross-entropy + BatchNorm1d(K) backward
 // Gradients land in one flat fp32 buffer with the layout of the parameters (vmb_mla_train_layout), ready for a single
@@ -41,7 +42,7 @@ namespace {
 constexpr int kMaxLevels = 4, kMaxFc = 4, kMaxBn = kMaxLevels * (1 + kMaxFc) + 2 * kMaxLevels + 1;
 constexpr float kBnEps = 1e-5f;
 constexpr float kBnMomentum = 0.1f;
-constexpr int kPl = 3;   // bf16 planes per GEMM operand: hi | mid | lo (fp32-equivalent, see igemm_linear_split)
+constexpr int kPl = 3;   // bf16 planes per GEMM operand: hi | mid | lo (fp32-equivalent, see vmb::split_bf16)
 
 int fail(const char* fmt, const char* detail = "") {
   char buf[640];
@@ -175,7 +176,6 @@ using vmb::dropout_scale;   // igemm_sm100.cuh: shared with the gradient-statist
 // ------------------------------------------------------------------ 32x32 tile kernel with element functor
 struct TileOut {
   __nv_bfloat16* planes;    // [rows_pad][3 * cols_pad] hi | mid | lo   (may be null)
-  __nv_bfloat16* planes_t;  // [cols_pad][3 * rows_pad] hi | mid | lo   (may be null)
   float* f32;               // [rows][ld_f32]                     (may be null)
   long long ld_f32;
   float* col_sum;           // [cols] += sum over rows (atomic)   (may be null)
@@ -185,14 +185,10 @@ struct TileOut {
   // tile in shared memory and finalised by the last block like bn_time_stats_kernel does: stats_T > 0 switches it on
   StatJob stats = {};
   int stats_T = 0;
+  __nv_bfloat16* planes_t = nullptr;   // [cols_pad][3 * rows_pad] hi | mid | lo: the weights' transposed planes
 };
 
-__device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bfloat16& mid, __nv_bfloat16& lo) {
-  hi = __float2bfloat16_rn(v);
-  const float r1 = v - __bfloat162float(hi);      // exact
-  mid = __float2bfloat16_rn(r1);
-  lo = __float2bfloat16_rn(r1 - __bfloat162float(mid));
-}
+using vmb::split_bf16;
 
 __device__ __forceinline__ uint32_t pack2(__nv_bfloat16 a, __nv_bfloat16 b) {
   return __bfloat16_as_ushort(a) | (uint32_t(__bfloat16_as_ushort(b)) << 16);
@@ -424,8 +420,7 @@ struct FBnBackward {
 //   dbeta_t  = sum_{r in t} G[r,:] . s          dgamma_t = sum_{r in t} G[r,:] . P[r,:]
 //   dW[o][f] = sum_r (gamma_t G[r][o]) xhat[r][f] + c[o],   c[o] = sum_t beta_t sum_{r in t} G[r][o]
 // so no GEMM over the input width runs but the forward one and dW, and nothing divides by gamma.  Both contract in
-// slices of at most kWideSlice (forward: input columns) / kDwSlice (dW: rows) per tcgen05 accumulator.
-constexpr int kWideSlice = 768, kDwSlice = 1024;
+// slices of at most vmb::kFwdSlice (forward: input columns) / vmb::kDwSlice (dW: rows) per tcgen05 accumulator.
 
 // xhat = (x - mean_t) rstd_t (the same expression GradIn::xhat evaluates)
 struct FNormalize {
@@ -574,8 +569,8 @@ struct AttParams {
 };
 
 // y[clip][col0 + k] = sum_t cla * att / sum_t att; row_stats[r] = {max, sum} of the class softmax of row r.
-// With yp != nullptr the same values also go out as the operand planes of the output Linear, yp [rows_pad][3 * yp_cols]
-// (the separate split pass over y is not launched); the grid then covers the padded rows, which are written as zeros.
+// The same values also go out as the operand planes of the output Linear, yp [rows_pad][3 * yp_cols]; the grid covers
+// the padded rows, which are written as zeros.
 __global__ void __launch_bounds__(256)
 att_forward_kernel(AttParams a, float* __restrict__ y, long long ystride, int col0, float* __restrict__ row_stats,
                    __nv_bfloat16* __restrict__ yp, int yp_cols, long long batch) {
@@ -583,7 +578,7 @@ att_forward_kernel(AttParams a, float* __restrict__ y, long long ystride, int co
   vmb::pdl_wait();
   __shared__ float rmax[16], rsum[16], sa_v[16], sb_v[16], sa_f[16], sb_f[16];
   const long long clip = blockIdx.x;
-  if (clip >= batch) {   // padding row of the planes (only reached with yp != nullptr)
+  if (clip >= batch) {   // padding row of the planes
     __nv_bfloat16* row = yp + clip * (static_cast<long long>(kPl) * yp_cols) + col0;
     for (int k = threadIdx.x; k < a.K; k += blockDim.x)
       for (int pl = 0; pl < kPl; ++pl) row[pl * yp_cols + k] = __float2bfloat16_rn(0.f);
@@ -623,14 +618,12 @@ att_forward_kernel(AttParams a, float* __restrict__ y, long long ystride, int co
     }
     const float val = num / den;
     y[clip * ystride + col0 + k] = val;
-    if (yp) {
-      __nv_bfloat16 hi, mid, lo;
-      split_bf16(val, hi, mid, lo);
-      __nv_bfloat16* row = yp + clip * (static_cast<long long>(kPl) * yp_cols) + col0 + k;
-      row[0] = hi;
-      row[yp_cols] = mid;
-      row[2 * yp_cols] = lo;
-    }
+    __nv_bfloat16 hi, mid, lo;
+    split_bf16(val, hi, mid, lo);
+    __nv_bfloat16* row = yp + clip * (static_cast<long long>(kPl) * yp_cols) + col0 + k;
+    row[0] = hi;
+    row[yp_cols] = mid;
+    row[2 * yp_cols] = lo;
   }
 }
 
@@ -947,31 +940,28 @@ struct vmb_mla_trainer {
   // side stream (with their own scratch: G_p2 .. dWtmp2, one dAtt per level) while the last level's chain runs
   cudaStream_t side2 = nullptr;
   cudaEvent_t ev_attb[kMaxLevels] = {};
-  __nv_bfloat16 *G_p2 = nullptr, *G_pt2 = nullptr;
+  __nv_bfloat16* G_p2 = nullptr;
   float *GV2 = nullptr, *GF2 = nullptr, *dWtmp2 = nullptr;
   float* dAtt[kMaxLevels] = {};
   // carved pointers
   double* acc = nullptr; size_t acc_bytes = 0;      // zeroed every step (together with the counters)
   unsigned* counters = nullptr;
   float* stat = nullptr;
-  __nv_bfloat16* xin_p = nullptr;                  // level-0 norm0 output planes [Rp][2 inpad]
-  __nv_bfloat16* xin_pt = nullptr;                 // transposed
+  __nv_bfloat16* xin_p = nullptr;                  // level-0 norm0 output planes [Rp][3 inpad]
   float* U[kMaxLevels][kMaxFc] = {};               // pre-BN Linear outputs [R][Hp]
   __nv_bfloat16* A_p[kMaxLevels][kMaxFc] = {};     // post-activation planes (input of the next Linear / fcv)
-  __nv_bfloat16* A_pt[kMaxLevels][kMaxFc] = {};
   float* E[kMaxLevels] = {};                       // fp32 embeddings of each level (input of the next level's norm0)
   __nv_bfloat16* N_p[kMaxLevels] = {};             // norm0 output planes of levels >= 1
-  __nv_bfloat16* N_pt[kMaxLevels] = {};
   float* Z[kMaxLevels] = {};                       // fcv outputs
   float* row_stats[kMaxLevels] = {};
   float *Y = nullptr, *dY = nullptr;               // [B][ycols]
-  __nv_bfloat16 *Y_p = nullptr, *Y_pt = nullptr;
+  __nv_bfloat16* Y_p = nullptr;
   float *O = nullptr, *dO = nullptr, *lse = nullptr;
-  __nv_bfloat16 *G_p = nullptr, *G_pt = nullptr;   // gradient planes (reused)
+  __nv_bfloat16* G_p = nullptr;                    // gradient planes (reused)
   float *GV = nullptr, *GF = nullptr;              // attention branch gradients / general fp32 scratch [R][Hp]
   float *dA = nullptr, *dB = nullptr, *dEnext = nullptr;  // fp32 gradient buffers [R][Hp]
   float* dWtmp = nullptr;                          // padded dW GEMM output
-  int Hp, Kp, inpad, ycols, ycols_pad;
+  int Hp, inpad, ycols, ycols_pad;
   // wide first layer (inpad > Hp): xin_p holds the planes of xhat, not of the norm0 output (see FNormalize)
   bool wide = false;
   float* P0 = nullptr;                             // xhat W^T of the first Linear [R][Hp]
@@ -1021,36 +1011,28 @@ void carve(vmb_mla_trainer* h, char* base) {
   h->acc_bytes = c.off;
   h->stat = c.take<float>(size_t(h->n_slots) * kSlot * 2);
   h->xin_p = c.take<__nv_bfloat16>(size_t(Rp) * kPl * inpad);
-  if (h->wide) {   // only the MN-major weight-gradient path runs at this width: no transposed planes
+  if (h->wide) {
     h->P0 = c.take<float>(size_t(R) * Hp);
     h->wsum = c.take<float>(size_t(Hp));
     h->gsum_t = c.take<float>(size_t(h->T) * Hp);
-  } else {
-    h->xin_pt = c.take<__nv_bfloat16>(size_t(inpad) * kPl * Rp);
   }
   for (int l = 0; l < h->n_levels; ++l) {
     for (int j = 0; j < h->lvl[l].n_fc; ++j) {
       h->U[l][j] = c.take<float>(size_t(R) * Hp);
       h->A_p[l][j] = c.take<__nv_bfloat16>(size_t(Rp) * kPl * Hp);
-      h->A_pt[l][j] = c.take<__nv_bfloat16>(size_t(Hp) * kPl * Rp);
     }
     h->E[l] = c.take<float>(size_t(R) * Hp);
-    if (l > 0) {
-      h->N_p[l] = c.take<__nv_bfloat16>(size_t(Rp) * kPl * Hp);
-      h->N_pt[l] = c.take<__nv_bfloat16>(size_t(Hp) * kPl * Rp);
-    }
+    if (l > 0) h->N_p[l] = c.take<__nv_bfloat16>(size_t(Rp) * kPl * Hp);
     h->Z[l] = c.take<float>(size_t(R) * Hp);
     h->row_stats[l] = c.take<float>(size_t(R) * 2);
   }
   h->Y = c.take<float>(size_t(B) * h->ycols_pad);
   h->dY = c.take<float>(size_t(B) * h->ycols_pad);
   h->Y_p = c.take<__nv_bfloat16>(size_t(Bp) * kPl * h->ycols_pad);
-  h->Y_pt = c.take<__nv_bfloat16>(size_t(h->ycols_pad) * kPl * Bp);
   h->O = c.take<float>(size_t(B) * Hp);
   h->dO = c.take<float>(size_t(B) * Hp);
   h->lse = c.take<float>(size_t(B));
   h->G_p = c.take<__nv_bfloat16>(size_t(Rp) * kPl * Hp);
-  h->G_pt = c.take<__nv_bfloat16>(size_t(Hp) * kPl * Rp);
   h->GV = c.take<float>(size_t(R) * Hp);
   h->GF = c.take<float>(size_t(R) * Hp);
   h->dA = c.take<float>(size_t(R) * Hp);
@@ -1063,7 +1045,6 @@ void carve(vmb_mla_trainer* h, char* base) {
   h->dWtmp = c.take<float>(size_t(Hp) * widest);
   if (h->n_levels > 1) {
     h->G_p2 = c.take<__nv_bfloat16>(size_t(Rp) * kPl * Hp);
-    h->G_pt2 = c.take<__nv_bfloat16>(size_t(Hp) * kPl * Rp);
     h->GV2 = c.take<float>(size_t(R) * Hp);
     h->GF2 = c.take<float>(size_t(R) * Hp);
     h->dWtmp2 = c.take<float>(size_t(Hp) * Hp);
@@ -1140,50 +1121,11 @@ int run_tile(F f, TileOut o, cudaStream_t st, const char* what) {
   return vmb::check_launch(what);
 }
 
-// dW = A^T B over the rows: tall contraction, few output tiles -> split-K with atomic accumulation into a zeroed buffer
-// The weight-gradient GEMMs read the ROW-major planes (the ones the forward / dX GEMMs consume) as MN-major UMMA operands
-// (planes_gemm_mn): no transposed copy of any activation or gradient is written.  VMB_TRAIN_MN_DW=0, or the planes GEMM
-// switched off, brings back the transposed planes and the K-major kernel (A/B timing).
-bool mn_dw_enabled() {
-  static const bool env_on = [] {
-    const char* e = getenv("VMB_TRAIN_MN_DW");
-    return !(e && e[0] == '0');
-  }();
-  return env_on && vmb::planes_gemm_enabled();
-}
-
-// dW [M][ldo] = sum over rows r of a[r][m] b[r][n]: a_planes [K][kPl * a_cols], b_planes [K][kPl * b_cols]
-int gemm_dw_mn(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M, int N,
-               long long K, cudaStream_t st) {
-  // one wave of (K slice, tile) work items, each slice at least four 32-row K-blocks long.  An output of more tiles
-  // than SMs (the wide first layer's dW) is split only into slices of at most kDwSlice rows, the length the 640-wide
-  // layers' slices have at 512 clips (precision of the tcgen05 accumulator, see gemm_bn); one slice: plain stores.
-  const int mn = (M / 128) * (N / 128);
-  int ks = vmb::num_sms() / mn;
-  if (ks == 0) ks = int((K + kDwSlice - 1) / kDwSlice);
-  const bool plain = ks == 1 && mn > vmb::num_sms();
-  if (ks > K / 32 / 4) ks = int(K / 32 / 4);
-  if (ks < 1) ks = 1;
-  if (!plain && cudaMemsetAsync(out, 0, size_t(M) * ldo * sizeof(float), st) != cudaSuccess) {
-    vmb::set_kernel_error("dW buffer clear failed");
-    return 1;
-  }
-  if (vmb::planes_gemm_mn(a_planes, a_cols, b_planes, b_cols, out, ldo, M, N, int(K), kPl, plain ? 0 : ks > 1 ? ks : -1,
-                          st)) {
+// dW [M][N] = sum over the rows r of g[r][m] b[r][n]: the gradient planes g [rows][kPl * M] against the layer input's
+// planes b [rows][kPl * N], both row-major as the forward / dX GEMMs consume them
+int gemm_dw(const void* g_planes, int M, const void* b_planes, int N, float* out, long long rows, cudaStream_t st) {
+  if (vmb::planes_gemm_dw(g_planes, M, b_planes, N, out, N, M, N, int(rows), kPl, st)) {
     vmb::set_kernel_error("%s", vmb::planes_gemm_last_error());
-    return 1;
-  }
-  return 0;
-}
-
-int gemm_dw(const void* at_planes, const void* bt_planes, float* out, long long ldo, int M, int N, long long K,
-            cudaStream_t st) {
-  if (cudaMemsetAsync(out, 0, size_t(M) * ldo * sizeof(float), st) != cudaSuccess) {
-    vmb::set_kernel_error("dW buffer clear failed");
-    return 1;
-  }
-  if (vmb::igemm_linear_split_ksplit(at_planes, bt_planes, out, ldo, M, N, int(K), st, kPl)) {
-    vmb::set_kernel_error("%s", vmb::igemm_last_error());
     return 1;
   }
   return 0;
@@ -1191,23 +1133,14 @@ int gemm_dw(const void* at_planes, const void* bt_planes, float* out, long long 
 
 int gemm(const void* a_planes, const void* w_planes, const float* bias, float* out, long long ldo, long long M, int N,
          int K, cudaStream_t st) {
-  if (vmb::igemm_linear_split(a_planes, w_planes, bias, out, ldo, 0, int(M), N, K, st, kPl)) {
-    vmb::set_kernel_error("%s", vmb::igemm_last_error());
+  if (vmb::planes_gemm(a_planes, w_planes, bias, out, ldo, 0, int(M), N, K, kPl, 0, st)) {
+    vmb::set_kernel_error("%s", vmb::planes_gemm_last_error());
     return 1;
   }
   return 0;
 }
 
-// Linear + the BatchNorm statistics of its output in one kernel (planes_gemm_stats): replaces gemm() followed by
-// bn_time_stats_kernel.  Falls back to the two-kernel form when the planes GEMM is switched off or T > 16.
-bool stats_in_gemm(int T) {
-  static const bool env_on = [] {
-    const char* e = getenv("VMB_TRAIN_STATS_FUSE");
-    return !(e && e[0] == '0');
-  }();
-  return env_on && vmb::planes_gemm_enabled() && T <= 16;
-}
-
+// Linear + the BatchNorm statistics of its output in one kernel (planes_gemm_stats)
 int gemm_stats(const void* a_planes, const void* w_planes, const float* bias, float* out, long long ldo, long long M, int N,
                int K, const StatJob& j, int cols, cudaStream_t st) {
   vmb::PlanesStats ps{j.acc, j.stat, j.counter, j.run_mean, j.run_var, j.count, j.channels, cols, kBnEps, kBnMomentum};
@@ -1221,12 +1154,7 @@ int gemm_stats(const void* a_planes, const void* w_planes, const float* bias, fl
 // dX GEMM + the BatchNorm-backward reductions of the block that consumes its output (planes_gemm_gradstats): replaces
 // gemm() followed by bn_time_backward_reduce_kernel when the block's only upstream gradient is this GEMM's output.
 bool gradstats_in_gemm(const GradIn& gi) {
-  static const bool env_on = [] {
-    const char* e = getenv("VMB_TRAIN_GRADSTATS_FUSE");
-    return !(e && e[0] == '0');
-  }();
-  return env_on && vmb::planes_gemm_enabled() && gi.T <= 16 && !gi.da2 && gi.ldu % 4 == 0 &&
-         (gi.F + 3) / 4 * 4 <= gi.ldu && (reinterpret_cast<uintptr_t>(gi.u) & 15) == 0;
+  return !gi.da2 && gi.ldu % 4 == 0 && (gi.F + 3) / 4 * 4 <= gi.ldu && (reinterpret_cast<uintptr_t>(gi.u) & 15) == 0;
 }
 
 int gemm_gradstats(const void* a_planes, const void* w_planes, float* out, long long ldo, long long M, int N, int K,
@@ -1284,7 +1212,6 @@ int vmb_mla_trainer_create(vmb_mla_trainer_t** handle, int n_levels, const int* 
   h->max_batch = max_batch;
   h->wide = wide;
   h->Hp = std::max(pad128(hidden), pad128(n_classes));
-  h->Kp = h->Hp;
   h->inpad = pad128(emb_in);
   h->ycols = n_levels * n_classes;
   h->ycols_pad = pad128(h->ycols);
@@ -1382,12 +1309,8 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
   };
   // Side stream (created on first use): work that feeds nothing on the critical chain runs there — in the forward pass
   // the attention branch of every level but the last (fcv GEMM, statistics, pooling: only the concatenation at the end
-  // needs it), in the backward pass the weight-gradient GEMMs.  VMB_TRAIN_FORK=0 keeps everything on the caller's stream.
-  static const bool fork_env = [] {
-    const char* e = getenv("VMB_TRAIN_FORK");
-    return !(e && e[0] == '0');
-  }();
-  if (fork_env && !h->side) {
+  // needs it), in the backward pass the weight-gradient GEMMs.
+  if (!h->side) {
     if (cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->ev_dw, cudaEventDisableTiming) != cudaSuccess ||
@@ -1399,90 +1322,66 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       if (cudaEventCreateWithFlags(&h->ev_attb[i], cudaEventDisableTiming) != cudaSuccess)
         return fail("vmb_mla_train: cannot create the side stream");
   }
-  const bool forked = fork_env;
-  auto time_stats = [&](const float* src, long long ld, int F, const BnRef& bn, bool update_running, cudaStream_t ss) {
-    StatJob j = statjob(bn, double(B) * F);
-    if (!update_running) j.run_mean = j.run_var = nullptr;
-    const unsigned chunks = static_cast<unsigned>(std::min<long long>((B * F + 256 * 8 - 1) / (256 * 8), 64));
-    vmb::launch_pdl(bn_time_stats_kernel, dim3(chunks, T), dim3(256), 0, ss, src, ld, B, F, T, j);
-    vmb::count_launch();
-    return vmb::check_launch("bn_time_stats_kernel");
-  };
-  // weights -> operand planes run on the side stream: the first Linear needs them only after the level-0 norm0
-  // statistics and its activation pass, which do not depend on the weights
-  cudaStream_t ws_stream = forked ? h->side : st;
   WeightJobs wj{};
   auto weights = [&](const FcRef& f) {
     const int j = wj.n++;
-    wj.o[j] = TileOut{f.wp, f.wtp, nullptr, 0, nullptr, f.n_out, f.n_out_pad, f.n_in, f.n_in_pad};
+    wj.o[j] = TileOut{f.wp, nullptr, 0, nullptr, f.n_out, f.n_out_pad, f.n_in, f.n_in_pad};
+    wj.o[j].planes_t = f.wtp;
     wj.f[j] = FIdentity{params + f.w, f.n_in, params + f.b, f.bias_pad, f.n_out};
     const dim3 g = tile_grid(f.n_out_pad, f.n_in_pad);
     wj.tiles_x[j] = int(g.x);
     wj.first_tile[j + 1] = wj.first_tile[j] + int(g.x * g.y);
     return 0;
   };
-  const bool fuse_stats = stats_in_gemm(T);
-  static const bool estats_env = [] {
-    const char* e = getenv("VMB_TRAIN_ESTATS_FUSE");
-    return !(e && e[0] == '0');
-  }();
-  const bool estats_fused = estats_env && T <= 16;   // norm0 statistics of levels >= 1 from the pass that writes the embedding
-  const bool mn_dw = mn_dw_enabled();   // weight-gradient GEMMs read the row-major planes: no transposed planes are written
-  auto tplanes = [&](__nv_bfloat16* pt) { return mn_dw ? static_cast<__nv_bfloat16*>(nullptr) : pt; };
-  if (h->wide && !mn_dw)
-    return fail("vmb_mla_train: emb_in wider than the hidden width needs the planes GEMM and its MN-major weight-gradient "
-                "kernel (VMB_PLANES_GEMM=0 or VMB_TRAIN_MN_DW=0 is set)");
   const LevelRef& L0 = h->lvl[0];
   // Linear (+ bias) into `out` and the BatchNorm statistics of its first `cols` columns
   auto gemm_bn = [&](const void* a, const FcRef& fc, float* out, int k_pad, int cols, const BnRef& bn, cudaStream_t ss) {
     if (h->wide && &fc == &L0.fc[0]) {
-      // P = xhat W^T with the K loop cut into slices of kWideSlice columns (fp32 reductions into a zeroed P): one
+      // P = xhat W^T with the K loop cut into slices of kFwdSlice columns (fp32 reductions into a zeroed P): one
       // tcgen05 accumulator summed over all 12288 columns loses ~1e-4 relative to its per-step truncation, which moved
       // gradients past the fp32 reference's tolerance.  Then U = gamma_t P + beta_t s + b and U's statistics.
       if (cudaMemsetAsync(h->P0, 0, size_t(R) * Hp * sizeof(float), ss) != cudaSuccess) {
         vmb::set_kernel_error("wide-layer output clear failed");
         return 1;
       }
-      if (vmb::planes_gemm(a, fc.wp, nullptr, h->P0, Hp, 0, int(R), Hp, k_pad, kPl, (k_pad + kWideSlice - 1) / kWideSlice,
-                           ss)) {
+      if (vmb::planes_gemm(a, fc.wp, nullptr, h->P0, Hp, 0, int(R), Hp, k_pad, kPl,
+                           (k_pad + vmb::kFwdSlice - 1) / vmb::kFwdSlice, ss)) {
         vmb::set_kernel_error("%s", vmb::planes_gemm_last_error());
         return 1;
       }
       FAffine f{h->P0, Hp, T, params + L0.norm0.g, params + L0.norm0.b, h->wsum, fc.bias_pad};
-      TileOut o{nullptr, nullptr, out, Hp, nullptr, R, R, cols, Hp};
+      TileOut o{nullptr, out, Hp, nullptr, R, R, cols, Hp};
       o.stats = statjob(bn, double(B) * cols);
       o.stats_T = T;
       return run_tile(f, o, ss, "wide-layer affine + statistics");
     }
-    if (fuse_stats) return gemm_stats(a, fc.wp, fc.bias_pad, out, Hp, R, Hp, k_pad, statjob(bn, double(B) * cols), cols, ss);
-    int r = gemm(a, fc.wp, fc.bias_pad, out, Hp, R, Hp, k_pad, ss);
-    return r ? r : time_stats(out, Hp, cols, bn, true, ss);
+    return gemm_stats(a, fc.wp, fc.bias_pad, out, Hp, R, Hp, k_pad, statjob(bn, double(B) * cols), cols, ss);
   };
 
   if (do_fwd) {
-  // ---- weights -> hi|lo planes, row-major and transposed (they changed in the last optimiser step)
-  if (forked) {
-    cudaEventRecord(h->ev_fork, st);                 // after the optimiser step (and everything else) on the caller's stream
-    cudaStreamWaitEvent(h->side, h->ev_fork, 0);
-  }
+  // ---- weights -> hi|mid|lo planes, row-major and transposed (they changed in the last optimiser step), on the side
+  // stream: the first Linear needs them only after the level-0 norm0 statistics and its activation pass, which do not
+  // depend on the weights
+  cudaEventRecord(h->ev_fork, st);   // after the optimiser step (and everything else) on the caller's stream
+  cudaStreamWaitEvent(h->side, h->ev_fork, 0);
   for (int l = 0; l < h->n_levels; ++l) {
     for (int j = 0; j < h->lvl[l].n_fc; ++j) TRY(weights(h->lvl[l].fc[j]));
     TRY(weights(h->lvl[l].fcv));
   }
   TRY(weights(h->fc_out));
   if (!rc) {
-    vmb::launch_pdl(weights_split_kernel, dim3(unsigned(wj.first_tile[wj.n])), dim3(256), 0, ws_stream, wj);
+    vmb::launch_pdl(weights_split_kernel, dim3(unsigned(wj.first_tile[wj.n])), dim3(256), 0, h->side, wj);
     vmb::count_launch();
     TRY(vmb::check_launch("weights_split_kernel"));
   }
   if (!rc && h->wide) {   // s[o] = sum_f W[o][f] of the wide first Linear (its GEMM epilogue and the backward pass)
-    row_sum_kernel<<<static_cast<unsigned>(L0.fc[0].n_out), 256, 0, ws_stream>>>(params + L0.fc[0].w, L0.fc[0].n_in,
-                                                                                h->wsum);
+    row_sum_kernel<<<static_cast<unsigned>(L0.fc[0].n_out), 256, 0, h->side>>>(params + L0.fc[0].w, L0.fc[0].n_in,
+                                                                              h->wsum);
     vmb::count_launch();
     TRY(vmb::check_launch("row_sum_kernel"));
   }
-  if (forked) cudaEventRecord(h->ev_w, h->side);
-  bool weights_pending = forked;
+  cudaEventRecord(h->ev_w, h->side);
+  bool weights_pending = true;
 
   // =============================================================================== forward
   bool att_pending = false;
@@ -1493,14 +1392,19 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     const int F_in = l == 0 ? h->emb_in : H;
     const int in_pad = l == 0 ? inpad : Hp;
     __nv_bfloat16* np = l == 0 ? h->xin_p : h->N_p[l];
-    __nv_bfloat16* npt = tplanes(l == 0 ? h->xin_pt : h->N_pt[l]);
-    if (!(l > 0 && estats_fused)) TRY(time_stats(in, ld_in, F_in, L.norm0, true, st));
+    if (l == 0) {   // the statistics of a later level's input come with the pass that writes it (below)
+      const StatJob j = statjob(L.norm0, double(B) * F_in);
+      const unsigned chunks = static_cast<unsigned>(std::min<long long>((B * F_in + 256 * 8 - 1) / (256 * 8), 64));
+      vmb::launch_pdl(bn_time_stats_kernel, dim3(chunks, T), dim3(256), 0, st, in, ld_in, B, F_in, T, j);
+      vmb::count_launch();
+      TRY(vmb::check_launch("bn_time_stats_kernel"));
+    }
     if (l == 0 && h->wide) {
-      TileOut o{np, nullptr, nullptr, 0, nullptr, R, Rp, F_in, in_pad};
+      TileOut o{np, nullptr, 0, nullptr, R, Rp, F_in, in_pad};
       TRY(run_tile(FNormalize{in, ld_in, T, slotstat(L.norm0.slot)}, o, st, "norm0 forward (xhat)"));
     } else {
       FBnAct f{in, ld_in, T, F_in, slotstat(L.norm0.slot), params + L.norm0.g, params + L.norm0.b, 0, 0.f, h->seed_dev, 0};
-      TileOut o{np, npt, nullptr, 0, nullptr, R, Rp, F_in, in_pad};
+      TileOut o{np, nullptr, 0, nullptr, R, Rp, F_in, in_pad};
       TRY(run_tile(f, o, st, "norm0 forward"));
     }
     const __nv_bfloat16* a = np;
@@ -1514,8 +1418,8 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       const bool last = j == L.n_fc - 1;
       FBnAct f{h->U[l][j], Hp, T, H, slotstat(L.norms[j].slot), params + L.norms[j].g, params + L.norms[j].b, 1,
                dropout_p, h->seed_dev, unsigned(1 + l * kMaxFc + j)};
-      TileOut o{h->A_p[l][j], tplanes(h->A_pt[l][j]), last ? h->E[l] : nullptr, Hp, nullptr, R, Rp, H, Hp};
-      if (last && l + 1 < h->n_levels && estats_fused) {
+      TileOut o{h->A_p[l][j], last ? h->E[l] : nullptr, Hp, nullptr, R, Rp, H, Hp};
+      if (last && l + 1 < h->n_levels) {
         // the embedding this pass writes is the input of the next level's norm0: its batch statistics ride along
         o.stats = statjob(h->lvl[l + 1].norm0, double(B) * H);
         o.stats_T = T;
@@ -1525,7 +1429,7 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     }
     // attention branch of this level: every buffer it writes is per level (Z[l], its statistic slots, columns l*K.. of Y),
     // so with another level still to come it runs on the side stream next to that level's chain
-    const bool side = forked && l + 1 < h->n_levels;
+    const bool side = l + 1 < h->n_levels;
     cudaStream_t as = side ? h->side : st;
     if (side && !rc) {
       cudaEventRecord(h->ev_fork, st);               // the level's last activation planes (a) are complete
@@ -1542,10 +1446,9 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       TRY(vmb::check_launch("bn_running_only_kernel"));
       AttParams ap{h->Z[l], Hp, K, T, slotstat(L.normv.slot), params + L.normv.g, params + L.normv.b,
                    params + L.normf.g, params + L.normf.b};
-      // with row-major planes only (mn_dw) the pooling kernel writes the output Linear's operand planes itself
-      vmb::launch_pdl(att_forward_kernel, dim3(static_cast<unsigned>(mn_dw ? Bp : B)), dim3(256), 0, as, ap, h->Y,
-                      static_cast<long long>(h->ycols_pad), l * K, h->row_stats[l],
-                      mn_dw ? h->Y_p : static_cast<__nv_bfloat16*>(nullptr), h->ycols_pad, B);
+      // the pooling kernel also writes the output Linear's operand planes
+      vmb::launch_pdl(att_forward_kernel, dim3(static_cast<unsigned>(Bp)), dim3(256), 0, as, ap, h->Y,
+                      static_cast<long long>(h->ycols_pad), l * K, h->row_stats[l], h->Y_p, h->ycols_pad, B);
       vmb::count_launch();
       TRY(vmb::check_launch("att_forward_kernel"));
     }
@@ -1556,10 +1459,6 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
   }
   if (att_pending) cudaStreamWaitEvent(st, h->ev_att, 0);   // join: the concatenation below reads every level's pooling
   // output layer
-  if (!mn_dw) {
-    TileOut o{h->Y_p, h->Y_pt, nullptr, 0, nullptr, B, Bp, h->ycols, h->ycols_pad};
-    TRY(run_tile(FIdentity{h->Y, h->ycols_pad}, o, st, "y split"));
-  }
   TRY(gemm(h->Y_p, h->fc_out.wp, h->fc_out.bias_pad, h->O, Hp, B, Hp, h->ycols_pad, st));
   if (!rc) {
     StatJob j = statjob(h->norm_out, double(B));
@@ -1575,45 +1474,32 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
   }  // do_fwd
   if (do_bwd) {
   // =============================================================================== backward
-  // Weight-gradient GEMMs on the side stream: each reads the transposed gradient planes G_pt the tile kernel just wrote
-  // and an activation's transposed planes, and writes only its slice of `grads` — nothing on the dX chain waits for it.
-  // The chain only has to wait (ev_dw) before the NEXT tile kernel overwrites G_pt, one dX GEMM and one reduction later.
+  // Weight-gradient GEMMs on the side stream: each reads the gradient planes G_p the tile kernel just wrote and an
+  // activation's planes, and writes only its slice of `grads` — nothing on the dX chain waits for it.  The chain only
+  // has to wait (ev_dw) before the NEXT tile kernel overwrites G_p, one dX GEMM and one reduction later.
   bool dw_pending = false;
-  // dW (M x N, contraction over the rows) -> dst [rows_out][cols_out] of `grads`
-  // operands of a dW GEMM in both forms: transposed planes (K-major kernel) and the row-major planes with their widths
-  struct DwOps { const void *at, *bt, *a; int a_cols; const void* b; int b_cols; };
-  auto dw_gemm = [&](const DwOps& ops, float* out, long long ldo, int M, int N, long long Kc, cudaStream_t s) {
-    return mn_dw ? gemm_dw_mn(ops.a, ops.a_cols, ops.b, ops.b_cols, out, ldo, M, N, Kc, s)
-                 : gemm_dw(ops.at, ops.bt, out, ldo, M, N, Kc, s);
-  };
-  auto dw_job = [&](const DwOps& ops, long long ldo, int M, int N, long long Kc, float* dst,
-                    size_t dst_pitch, size_t width, size_t height) {
-    cudaStream_t s = forked ? h->side : st;
-    if (forked) {
-      cudaEventRecord(h->ev_fork, st);
-      cudaStreamWaitEvent(h->side, h->ev_fork, 0);
-    }
-    int r = dw_gemm(ops, h->dWtmp, ldo, M, N, Kc, s);
+  // dW [n_out][n_in] of a Linear (G_p against its input's planes b [rows][kPl * b_cols]) -> dst, its block of `grads`
+  auto dw_job = [&](const void* b, int b_cols, long long rows, float* dst, int n_out, int n_in) {
+    cudaEventRecord(h->ev_fork, st);
+    cudaStreamWaitEvent(h->side, h->ev_fork, 0);
+    int r = gemm_dw(h->G_p, Hp, b, b_cols, h->dWtmp, rows, h->side);
     if (!r && dst == grads + L0.fc[0].w && h->wide) {
       // the wide first Linear: dW = the GEMM's sum_r (gamma_t G) xhat + c[o] (see wide_grad_tile_kernel)
-      const int n_in = L0.fc[0].n_in;
-      vmb::launch_pdl(wide_dw_finish_kernel, dim3(unsigned((n_in + 1023) / 1024), unsigned(height)), dim3(256), 0, s,
-                      static_cast<const float*>(h->dWtmp), ldo, dst, n_in, static_cast<const float*>(h->gsum_t), Hp,
-                      params + L0.norm0.b, T);
+      vmb::launch_pdl(wide_dw_finish_kernel, dim3(unsigned((n_in + 1023) / 1024), unsigned(n_out)), dim3(256), 0,
+                      h->side, static_cast<const float*>(h->dWtmp), static_cast<long long>(b_cols), dst, n_in,
+                      static_cast<const float*>(h->gsum_t), Hp, params + L0.norm0.b, T);
       vmb::count_launch();
       r = vmb::check_launch("wide_dw_finish_kernel");
-    } else if (!r && cudaMemcpy2DAsync(dst, dst_pitch, h->dWtmp, size_t(ldo) * 4, width, height, cudaMemcpyDeviceToDevice,
-                                       s) != cudaSuccess) {
+    } else if (!r && cudaMemcpy2DAsync(dst, size_t(n_in) * 4, h->dWtmp, size_t(b_cols) * 4, size_t(n_in) * 4, n_out,
+                                       cudaMemcpyDeviceToDevice, h->side) != cudaSuccess) {
       vmb::set_kernel_error("dW copy failed");
       r = 1;
     }
-    if (forked) {
-      cudaEventRecord(h->ev_dw, h->side);
-      dw_pending = true;
-    }
+    cudaEventRecord(h->ev_dw, h->side);
+    dw_pending = true;
     return r;
   };
-  auto before_g_overwrite = [&]() {   // G_p / G_pt (and dWtmp's reader) are about to be rewritten by the chain
+  auto before_g_overwrite = [&]() {   // G_p (and dWtmp's reader) are about to be rewritten by the chain
     if (dw_pending) {
       cudaStreamWaitEvent(st, h->ev_dw, 0);
       dw_pending = false;
@@ -1628,13 +1514,11 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     TRY(vmb::check_launch("out_bn_backward_kernel"));
   }
   {
-    // dO planes (+ transposed) and d(bias) = column sums
-    TileOut o{h->G_p, tplanes(h->G_pt), nullptr, 0, grads + h->fc_out.b, B, Bp, K, Hp};
+    // dO planes and d(bias) = column sums
+    TileOut o{h->G_p, nullptr, 0, grads + h->fc_out.b, B, Bp, K, Hp};
     TRY(run_tile(FIdentity{h->dO, Hp}, o, st, "dO split"));
-    // dW_fc [K][L*K] = dO^T [K x B] * Y^T [L*K x B]^T
-    TRY(dw_job(DwOps{h->G_pt, h->Y_pt, h->G_p, Hp, h->Y_p, h->ycols_pad}, h->ycols_pad, Hp, h->ycols_pad, Bp,
-               grads + h->fc_out.w, size_t(h->ycols) * 4,
-               size_t(h->ycols) * 4, K));
+    // dW_fc [K][L*K] = dO^T [K x B] * Y [B x L*K]
+    TRY(dw_job(h->Y_p, h->ycols_pad, Bp, grads + h->fc_out.w, K, h->ycols));
     // dY [B][L*K] = dO [B x K] * W_fc [K x L*K]
     TRY(gemm(h->G_p, h->fc_out.wtp, nullptr, h->dY, h->ycols_pad, B, h->ycols_pad, Hp, st));
   }
@@ -1677,9 +1561,8 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
                          int(2 * 16 * 1024 * sizeof(float)));
   auto att_branch = [&](int l, cudaStream_t s, bool own_side, float* out_dA) {
     const LevelRef& L = h->lvl[l];
-    const __nv_bfloat16* e_pt = h->A_pt[l][L.n_fc - 1];
+    const __nv_bfloat16* e_p = h->A_p[l][L.n_fc - 1];
     __nv_bfloat16* gp = own_side ? h->G_p2 : h->G_p;
-    __nv_bfloat16* gpt = own_side ? h->G_pt2 : h->G_pt;
     float* gv = own_side ? h->GV2 : h->GV;
     float* gf = own_side ? h->GF2 : h->GF;
     AttParams ap{h->Z[l], Hp, K, T, slotstat(L.normv.slot), params + L.normv.g, params + L.normv.b,
@@ -1693,19 +1576,18 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     {
       FAttCombine f{ap, gv, gf, Hp, acc_v, acc_f, double(B) * K, grads + L.normv.g, grads + L.normv.b,
                     grads + L.normf.g, grads + L.normf.b};
-      TileOut o{gp, tplanes(gpt), nullptr, 0, grads + L.fcv.b, R, Rp, K, Hp};
+      TileOut o{gp, nullptr, 0, grads + L.fcv.b, R, Rp, K, Hp};
       if (!own_side) before_g_overwrite();
       TRY(run_tile(f, o, s, "attention BN backward"));
     }
-    // dWv [K][H] = dZ^T * E^T ; dE_att [R][H] = dZ * Wv
-    const DwOps att_ops{gpt, e_pt, gp, Hp, h->A_p[l][L.n_fc - 1], Hp};
+    // dWv [K][H] = dZ^T * E ; dE_att [R][H] = dZ * Wv
     if (own_side) {
-      TRY(dw_gemm(att_ops, h->dWtmp2, Hp, Hp, Hp, Rp, s));
+      TRY(gemm_dw(gp, Hp, e_p, Hp, h->dWtmp2, Rp, s));
       if (!rc && cudaMemcpy2DAsync(grads + L.fcv.w, size_t(H) * 4, h->dWtmp2, size_t(Hp) * 4, size_t(H) * 4, K,
                                    cudaMemcpyDeviceToDevice, s) != cudaSuccess)
         rc = 1;
     } else {
-      TRY(dw_job(att_ops, Hp, Hp, Hp, Rp, grads + L.fcv.w, size_t(H) * 4, size_t(H) * 4, K));
+      TRY(dw_job(e_p, Hp, Rp, grads + L.fcv.w, K, H));
     }
     if (own_side) {
       TRY(gemm(gp, L.fcv.wtp, nullptr, out_dA, Hp, R, Hp, Hp, s));     // joins the chain as one of two upstream gradients
@@ -1714,7 +1596,7 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
     }
   };
   // fork: every level below the last starts its attention branch now (dY is complete), on the second side stream
-  const bool att_fork = forked && h->n_levels > 1;
+  const bool att_fork = h->n_levels > 1;
   if (att_fork && !rc) {
     cudaEventRecord(h->ev_fork, st);
     cudaStreamWaitEvent(h->side2, h->ev_fork, 0);
@@ -1772,14 +1654,12 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
           TRY(vmb::check_launch("wide_grad_tile_kernel"));
         }
       } else {
-        TileOut o{h->G_p, tplanes(h->G_pt), nullptr, Hp, grads + fc.b, R, Rp, H, Hp};
+        TileOut o{h->G_p, nullptr, Hp, grads + fc.b, R, Rp, H, Hp};
         TRY(run_tile(f, o, st, "fc BN backward"));
       }
-      // dW [H][n_in] = dU^T * A_prev^T ; dA_prev [R][n_in] = dU * W
-      const __nv_bfloat16* prev_pt = j > 0 ? h->A_pt[l][j - 1] : (l == 0 ? h->xin_pt : h->N_pt[l]);
+      // dW [H][n_in] = dU^T * A_prev ; dA_prev [R][n_in] = dU * W
       const __nv_bfloat16* prev_p = j > 0 ? h->A_p[l][j - 1] : (l == 0 ? h->xin_p : h->N_p[l]);
-      TRY(dw_job(DwOps{h->G_pt, prev_pt, h->G_p, Hp, prev_p, fc.n_in_pad}, fc.n_in_pad, Hp, fc.n_in_pad, Rp, grads + fc.w, size_t(fc.n_in) * 4,
-                 size_t(fc.n_in) * 4, H));
+      TRY(dw_job(prev_p, fc.n_in_pad, Rp, grads + fc.w, H, fc.n_in));
       float* dprev = (da1 == h->dA) ? h->dB : h->dA;
       if (wide0)
         pre_reduced = true;   // no dX GEMM: norm0's two reductions came from wide_grad_tile_kernel
@@ -1804,10 +1684,10 @@ int train_phases(int phases, vmb_mla_trainer* h, const float* params, float* run
       // level 0: only the parameter gradients are needed (written by the prologue); still run one tile row so
       // the prologue executes (with the wide first layer no element is evaluated: there is no dY).  level > 0: fp32
       // gradient wrt E_{l-1}
-      TileOut o{nullptr, nullptr, l > 0 ? h->dEnext : nullptr, Hp, nullptr, l > 0 ? R : 1, l > 0 ? R : 1,
+      TileOut o{nullptr, l > 0 ? h->dEnext : nullptr, Hp, nullptr, l > 0 ? R : 1, l > 0 ? R : 1,
                 (l == 0 && h->wide) ? 0 : F_in, l > 0 ? Hp : 32};
       float* dx_pad = (da1 == h->dA) ? h->dB : h->dA;   // level 0 with dx: the chain buffer norm0's input does not use
-      if (l == 0 && dx) o = TileOut{nullptr, nullptr, dx_pad, Hp, nullptr, R, R, F_in, inpad};
+      if (l == 0 && dx) o = TileOut{nullptr, dx_pad, Hp, nullptr, R, R, F_in, inpad};
       TRY(run_tile(f, o, st, "norm0 backward"));
       if (l == 0 && dx && !rc &&
           cudaMemcpy2DAsync(dx, size_t(F_in) * 4, dx_pad, size_t(Hp) * 4, size_t(F_in) * 4, size_t(R),

@@ -455,25 +455,16 @@ int launch_planes(const CUtensorMap& ta, const CUtensorMap& tb, const PlanesPara
   return 0;
 }
 
-std::atomic<int> g_planes_override{-1};
-
 }  // namespace
 
 const char* planes_gemm_last_error() { return g_perr; }
 
 bool planes_gemm_enabled() {
-  const int o = g_planes_override.load(std::memory_order_relaxed);
-  if (o >= 0) return o != 0;
   static const bool on = [] {
     const char* e = getenv("VMB_PLANES_GEMM");
     return !(e && e[0] == '0');
   }();
   return on;
-}
-
-int planes_gemm_set(int on) {
-  const int prev = g_planes_override.exchange(on < 0 ? -1 : (on ? 1 : 0), std::memory_order_relaxed);
-  return prev;
 }
 
 // Which three-plane variants may take 128 x 64 tiles — bit 0: plain stores, bit 1: statistics epilogue, bit 2:
@@ -617,6 +608,22 @@ int planes_gemm_mn(const void* a_planes, int a_cols, const void* b_planes, int b
                        : launch_planes<2, false, 0, 128, true>(ta, tb, p, stream);
   return planes == 3 ? launch_planes<3, true, 0, 128, true>(ta, tb, p, stream)
                      : launch_planes<2, true, 0, 128, true>(ta, tb, p, stream);
+}
+
+int planes_gemm_dw(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M,
+                   int N, int K, int planes, cudaStream_t stream) {
+  const int mn = (M / 128) * (N / 128);
+  int ks = num_sms() / mn;
+  if (ks == 0) ks = (K + kDwSlice - 1) / kDwSlice;
+  const bool plain = ks == 1 && mn > num_sms();
+  if (ks > K / 32 / 4) ks = K / 32 / 4;
+  if (ks < 1) ks = 1;
+  if (!plain && cudaMemsetAsync(out, 0, size_t(M) * ldo * sizeof(float), stream) != cudaSuccess) {
+    snprintf(g_perr, sizeof g_perr, "planes_gemm_dw: output clear failed");
+    return 1;
+  }
+  return planes_gemm_mn(a_planes, a_cols, b_planes, b_cols, out, ldo, M, N, K, planes, plain ? 0 : ks > 1 ? ks : -1,
+                        stream);
 }
 
 int planes_gemm(const void* a_planes, const void* b_planes, const float* bias, float* out, long long ldo, int relu, int M,

@@ -262,7 +262,7 @@ int vmb_mla_forward_fp32(vmb_mla_t* handle, const float* emb_dev, long long batc
  * vmb_mla_trainer_create: 1..4 levels of 1..4 Linears, hidden and n_classes in 1..1024, T in 1..16, emb_in in
  * 1..16384.  An emb_in wider than the hidden width (padded to 128: the just_bottlenecks head, emb_in = 12288) takes a
  * wide-first-layer path: no gradient with respect to the input is formed (the CNN is frozen), only the forward and the
- * weight-gradient GEMM run over the input width, and it needs the planes GEMM (VMB_PLANES_GEMM, VMB_TRAIN_MN_DW not 0).
+ * weight-gradient GEMM run over the input width.
  * max_batch: 2 <= max_batch and max_batch * T <= 2^31 / 2048; with the wide path also
  * pad64(max_batch * T) * 3 * pad128(emb_in) < 2^31 (the element count of the input's operand planes; 5824 clips at
  * emb_in = 12288, T = 10).  A larger max_batch is rejected before anything is allocated. */
