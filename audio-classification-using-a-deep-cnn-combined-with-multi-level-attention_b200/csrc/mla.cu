@@ -281,14 +281,16 @@ int vmb_mla_create(vmb_mla_t** handle, int n_levels, const int* n_fc, int emb_in
   };
   size_t cur_planes = 0;
   int cur_kpad = 0;
-  auto transpose_w = [&](int n_out, int n_in, size_t& owt, size_t& obias) {
+  // kpad: the contraction length of the weight planes, which is also the row pitch (per plane) of the operand planes
+  // the GEMM reads.  The head lays out every activation of hidden width with a pitch of kPad columns (mla_tc.cu), so a
+  // Linear fed by one takes kpad = kPad; the head's input and the pooled scores come padded to a multiple of 64.
+  auto transpose_w = [&](int n_out, int n_in, int kpad, size_t& owt, size_t& obias) {
     const float* w = take(size_t(n_out) * n_in);
     const float* b = take(n_out);
     const int in_pad = (n_in + 3) & ~3;
     const bool small = n_in <= 4096;   // the transposed fp32 copy feeds the fused fp32 kernel and the output FC
     owt = reserve(small ? size_t(in_pad) * kPad : 4);
     obias = reserve(kPad);
-    const int kpad = (n_in + 63) / 64 * 64;
     cur_planes = planes.size();
     cur_kpad = kpad;
     planes.resize(planes.size() + size_t(kPad) * 2 * kpad, 0);
@@ -311,8 +313,9 @@ int vmb_mla_create(vmb_mla_t** handle, int n_levels, const int* n_fc, int emb_in
     // reference state_dict order inside EmbeddedMapping: norm0, fc.{j}, norms.{j}; the flat layout interleaves
     // (fc j, norm j) as documented in the header
     for (int j = 0; j < n_fc[l]; ++j) {
-      const int in = (l == 0 && j == 0) ? emb_in : H;
-      transpose_w(H, in, lo[l].fc[j].wt, lo[l].fc[j].bias);
+      const bool first = l == 0 && j == 0;
+      const int in = first ? emb_in : H;
+      transpose_w(H, in, first ? (in + 63) / 64 * 64 : kPad, lo[l].fc[j].wt, lo[l].fc[j].bias);
       lo[l].fc[j].wp = cur_planes;
       lo[l].fc[j].kpad = cur_kpad;
       fold_bn(T, lo[l].fc[j].a, lo[l].fc[j].b);
@@ -320,7 +323,7 @@ int vmb_mla_create(vmb_mla_t** handle, int n_levels, const int* n_fc, int emb_in
     }
   }
   for (int l = 0; l < n_levels; ++l) {
-    transpose_w(K, H, lo[l].fcv.wt, lo[l].fcv.bias);
+    transpose_w(K, H, kPad, lo[l].fcv.wt, lo[l].fcv.bias);
     lo[l].fcv.wp = cur_planes;
     lo[l].fcv.kpad = cur_kpad;
     lo[l].fcv.in = (H + 3) & ~3;
@@ -329,7 +332,7 @@ int vmb_mla_create(vmb_mla_t** handle, int n_levels, const int* n_fc, int emb_in
     fold_bn(T, lo[l].af, lo[l].bf);
   }
   size_t fc_wt, fc_bias, out_a, out_b;
-  transpose_w(K, n_levels * K, fc_wt, fc_bias);
+  transpose_w(K, n_levels * K, (n_levels * K + 63) / 64 * 64, fc_wt, fc_bias);
   const size_t fc_wp = cur_planes;
   const int fc_kpad = cur_kpad;
   fold_bn(K, out_a, out_b);

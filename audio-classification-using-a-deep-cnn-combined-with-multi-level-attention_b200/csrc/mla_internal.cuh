@@ -17,7 +17,7 @@ constexpr int kColsPerThread = kPad / kColThreads;  // 10
 
 struct FcDev {
   const void* wp;     // bf16 [kPad][2 * kpad]: hi | lo planes of W (rows = outputs, zero padded)   (tensor-core path)
-  int kpad;           // inputs padded to a multiple of 64
+  int kpad;           // contraction length: kPad for inputs of hidden width, else the inputs padded to 64
   const float* wt;    // [in][kPad]
   const float* bias;  // [kPad]
   const float* a;     // [T] folded BN scale

@@ -424,7 +424,11 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
   // workspace: x planes | three rotating activation plane buffers | normed-input planes | one fp32 z buffer per level |
   // y planes.  Three buffers, not two: a forked fcv GEMM still reads the level's embedding planes while the next level's
   // chain runs, and with two buffers the second GEMM of that chain would have to wait for it before it may start.
-  const size_t total = sz_x + 4 * sz_p + d.n_levels * sz_u + sz_yp;
+  // Two normed-input buffers alternating by level when there are more than two levels: the only Linear of a middle
+  // level reads its input from one while its epilogue writes the next level's input, and the GEMM's tiles are not
+  // ordered, so a tile writing in place could overwrite columns that a sibling tile has still to read.
+  const int n_pn = d.n_levels > 2 ? 2 : 1;
+  const size_t total = sz_x + (3 + n_pn) * sz_p + d.n_levels * sz_u + sz_yp;
   char* ws = nullptr;
   if (cudaMallocAsync(reinterpret_cast<void**>(&ws), total, st) != cudaSuccess) {
     vmb::set_kernel_error("mla: workspace allocation of %zu bytes failed: %s", total,
@@ -433,9 +437,9 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
   }
   void* X = ws;
   void* P[3] = {ws + sz_x, ws + sz_x + sz_p, ws + sz_x + 2 * sz_p};
-  void* Pn = ws + sz_x + 3 * sz_p;
-  float* U = reinterpret_cast<float*>(ws + sz_x + 4 * sz_p);
-  void* Yp = ws + sz_x + 4 * sz_p + d.n_levels * sz_u;
+  void* Pn[2] = {ws + sz_x + 3 * sz_p, ws + sz_x + (2 + n_pn) * sz_p};   // level l writes level l + 1's input to Pn[l & 1]
+  float* U = reinterpret_cast<float*>(ws + sz_x + (3 + n_pn) * sz_p);
+  void* Yp = ws + sz_x + (3 + n_pn) * sz_p + d.n_levels * sz_u;
   int rc = split_rows(emb, d.emb_in, rows, d.emb_in, in_pad, d.T, d.lvl[0].n0a, d.lvl[0].n0b, 0, nullptr, nullptr, X, st);
   const void* cur = X;
   int pp = 0;
@@ -460,7 +464,7 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
       if (j == L.n_fc - 1 && l + 1 < d.n_levels) {   // the embedding with the next level's norm0 applied, same pass
         e.a2 = d.lvl[l + 1].n0a;
         e.b2 = d.lvl[l + 1].n0b;
-        e.dst2 = Pn;
+        e.dst2 = Pn[l & 1];
       }
       if (vmb::planes_gemm_fused(cur, L.fc[j].wp, L.fc[j].bias, e, int(rows), hpad, L.fc[j].kpad, st)) {
         vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
@@ -495,7 +499,7 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
       rc = vmb::check_launch("attention_pool_smem_kernel");
     }
     if (side) cudaEventRecord(h.join_ev[l], h.side);
-    cur = Pn;
+    cur = Pn[l & 1];
   }
   // join the side branches (also on the error path, so that the workspace is not freed under them)
   for (int l = 0; l + 1 < d.n_levels && fork; ++l) cudaStreamWaitEvent(st, h.join_ev[l], 0);

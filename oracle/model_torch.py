@@ -71,6 +71,16 @@ def _bn_time(sd: dict, prefix: str, x: torch.Tensor, training: bool) -> torch.Te
                         sd[prefix + ".weight"], sd[prefix + ".bias"], training, 0.1, BN_EPS)
 
 
+def attention_module(sd: dict, lvl: int, h: torch.Tensor, training: bool = False) -> torch.Tensor:
+    """AttentionModule.forward of level `lvl` (model.py:235-242): (B, T, H) -> (B, K)."""
+    p = f"attention_modules.{lvl}"
+    z = F.linear(h, sd[p + ".fcv.weight"], sd[p + ".fcv.bias"])
+    att = F.softmax(_bn_time(sd, p + ".normv", z, training), dim=2)
+    cla = torch.sigmoid(_bn_time(sd, p + ".normf", z, training))
+    norm_att = att / torch.sum(att, dim=1)[:, None, :]
+    return torch.sum(cla * norm_att, dim=1)
+
+
 def mla_forward(sd: dict, x: torch.Tensor, model_conf, training: bool = False, dropout_p: float = 0.0,
                 masks: dict | None = None, relu_pre: list | None = None):
     """x (B, T, M) -> (B, K) sigmoid scores.  training=True uses batch statistics (running stats are not
@@ -93,15 +103,7 @@ def mla_forward(sd: dict, x: torch.Tensor, model_conf, training: bool = False, d
             elif training and dropout_p > 0:
                 h = F.dropout(h, dropout_p, True)
         embs.append(h)
-    ys = []
-    for lvl in range(len(model_conf)):
-        p = f"attention_modules.{lvl}"
-        z = F.linear(embs[lvl], sd[p + ".fcv.weight"], sd[p + ".fcv.bias"])
-        att = F.softmax(_bn_time(sd, p + ".normv", z, training), dim=2)
-        cla = torch.sigmoid(_bn_time(sd, p + ".normf", z, training))
-        norm_att = att / torch.sum(att, dim=1)[:, None, :]
-        ys.append(torch.sum(cla * norm_att, dim=1))
-    conc = torch.cat(ys, dim=1)
+    conc = torch.cat([attention_module(sd, lvl, embs[lvl], training) for lvl in range(len(model_conf))], dim=1)
     out = F.linear(conc, sd["fc.weight"], sd["fc.bias"])
     out = F.batch_norm(out, None if training else sd["norm.running_mean"], None if training else sd["norm.running_var"],
                        sd["norm.weight"], sd["norm.bias"], training, 0.1, BN_EPS)

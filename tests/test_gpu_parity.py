@@ -449,18 +449,21 @@ def test_head_vs_golden(golden_head, tag, K, conf, seed):
     h.close()
 
 
-@pytest.mark.parametrize("K,conf,emb_in,seed", [(527, (2, 1), 128, 2), (10, (1, 2, 1), 128, 5), (527, (1,), 128, 6),
-                                                (33, (3,), 12288, 4)])
-def test_head_fused_epilogues_are_bit_identical(K, conf, emb_in, seed):
+@pytest.mark.parametrize("K,conf,emb_in,hidden,seed", [(527, (2, 1), 128, 600, 2), (10, (1, 2, 1), 128, 600, 5),
+                                                       (527, (1,), 128, 600, 6), (33, (3,), 12288, 600, 4),
+                                                       (10, (1, 1, 1), 128, 64, 7), (527, (2, 1, 2), 128, 600, 8)])
+def test_head_fused_epilogues_are_bit_identical(K, conf, emb_in, hidden, seed):
     """The glue of the eval-mode head (model.py:219-221 BatchNorm1d(T) + ReLU, :268 BatchNorm1d(K) + sigmoid) runs in
     the GEMM epilogues by default; with vmb_mla_fuse_enable(0) it runs as separate kernels.  Both evaluate the same
-    expressions in the same order: the scores must be equal bit for bit, at full and ragged tile sizes."""
+    expressions in the same order: the scores must be equal bit for bit, at full and ragged tile sizes, and at 400 clips
+    (4 000 rows: 160 tiles of the 640 output columns, more than one wave), where a middle level of one Linear reads its
+    input while its epilogue writes the next level's."""
     L = _lib.lib()
-    sd = synth.mla_state_dict(conf, emb_in, 600, K, 10, seed=seed)
-    h = engine.MlaHandle(sd, conf, emb_in, 600, K, 10, DEV)
+    sd = synth.mla_state_dict(conf, emb_in, hidden, K, 10, seed=seed)
+    h = engine.MlaHandle(sd, conf, emb_in, hidden, K, 10, DEV)
     g = torch.Generator().manual_seed(seed)
     try:
-        for batch in (1, 13, 256, 300):
+        for batch in (1, 13, 256, 300, 400):
             x = (torch.randn(batch, 10, emb_in, generator=g) * 1.5).to(DEV)
             L.vmb_mla_fuse_enable(1)
             n0 = L.vmb_launch_count()
