@@ -58,6 +58,10 @@ SIGNATURES = {
     "vmb_vggish_refresh_fc": (_int, [_c_p, C.POINTER(_c_p), C.POINTER(_c_p), _c_p]),
     "vmb_vggish_forward_train": (_int, [_c_p, _c_p, _ll, _c_p, _c_p, _sz, _c_p]),
     "vmb_vggish_fc_backward": (_int, [_c_p, _c_p, _sz, _c_p, _ll, _c_p, _c_p]),
+    "vmb_vggish_conv4_2_train_workspace_bytes": (_sz, [_ll]),
+    "vmb_vggish_refresh_conv4_2": (_int, [_c_p, _c_p, _c_p, _c_p, _c_p]),
+    "vmb_vggish_forward_train_conv4_2": (_int, [_c_p, _c_p, _ll, _c_p, _c_p, _sz, _c_p]),
+    "vmb_vggish_conv4_2_backward": (_int, [_c_p, _c_p, _sz, _c_p, _ll, _c_p, _c_p, _c_p]),
     "vmb_mla_create": (_int, [C.POINTER(_c_p), _int, C.POINTER(_int), _int, _int, _int, _int, _c_p, _ll, _c_p]),
     "vmb_mla_destroy": (None, [_c_p]),
     "vmb_mla_num_classes": (_int, [_c_p]),

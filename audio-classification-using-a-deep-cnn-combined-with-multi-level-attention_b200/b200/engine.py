@@ -277,8 +277,9 @@ class VggishHandle:
             self._fc_keep = keep        # the masters' copies must outlive the enqueued kernels that read them
         self._fc_refreshed = True
 
-    def _train_workspace(self, n: int):
-        need = int(_lib.lib().vmb_vggish_fc_train_workspace_bytes(n))
+    def _train_workspace(self, n: int, conv4_2: bool = False):
+        fn = _lib.lib().vmb_vggish_conv4_2_train_workspace_bytes if conv4_2 else _lib.lib().vmb_vggish_fc_train_workspace_bytes
+        need = int(fn(n))
         ws = getattr(self, "_train_ws", None)
         if ws is None or ws.numel() < need + 1024:
             self._train_ws = None
@@ -327,6 +328,94 @@ class VggishHandle:
         planes = self._train_ws[off:off + n * 3 * 12288 * 2].view(torch.bfloat16).view(n, 3, 12288)
         return planes.double().sum(dim=1)
 
+    # -- train-mode conv4_2 (features.13 trainable, conv1 .. conv4_1 frozen): csrc/conv_train.cu
+    @property
+    def conv4_2_trainable(self) -> bool:
+        """True once refresh_conv4_2() has derived the training copy of conv4_2's weights."""
+        return bool(getattr(self, "_conv4_2_refreshed", False))
+
+    def refresh_conv4_2(self, weight, bias, fc1_weight) -> None:
+        """Re-derive conv4_2's inference copy and training planes from fp32 masters (features.13.weight OIHW, .bias);
+        the first call also derives fc1's transposed planes from fc1_weight.  Stream-ordered."""
+        if not self.has_fc:
+            raise B200Error("this handle was built without the FC stack")
+        with torch.cuda.device(self.device):
+            keep = [t.detach().to(device=self.device, dtype=torch.float32).contiguous()
+                    for t in (weight, bias, fc1_weight)]
+            check(_lib.lib().vmb_vggish_refresh_conv4_2(self._h, *[t.data_ptr() for t in keep], stream_ptr()),
+                  "vmb_vggish_refresh_conv4_2")
+            self._conv4_2_keep = keep   # the masters' copies must outlive the enqueued kernels that read them
+        self._conv4_2_refreshed = True
+
+    def forward_train_conv4_2(self, examples: torch.Tensor) -> torch.Tensor:
+        """(n, 96, 64) / (n, 1, 96, 64) fp32 CUDA -> (n, 128) fp32 embeddings with conv4_2 in training precision,
+        keeping what conv4_2_backward() needs."""
+        self.check_saturation(synchronize=False)
+        examples = _need_cuda(examples, "examples")
+        if examples.dim() == 4 and examples.shape[1] == 1:
+            examples = examples[:, 0]
+        if examples.dim() != 3 or tuple(examples.shape[1:]) != (96, 64):
+            raise ValueError(f"examples must be (n, 1, 96, 64) or (n, 96, 64), got {tuple(examples.shape)}")
+        examples = examples.contiguous()
+        n = examples.shape[0]
+        emb = torch.empty((n, 128), device=self.device, dtype=torch.float32)
+        with torch.cuda.device(self.device):
+            base, need = self._train_workspace(n, conv4_2=True)
+            check(_lib.lib().vmb_vggish_forward_train_conv4_2(self._h, ptr(examples), n, ptr(emb), base, need,
+                                                              stream_ptr()), "vmb_vggish_forward_train_conv4_2")
+        self._train_n = n
+        return emb
+
+    def conv4_2_backward(self, d_emb: torch.Tensor, want_fc: bool):
+        """d(loss)/d(emb) (n, 128) of the last forward_train_conv4_2 -> (flat conv4_2 gradient [weight OIHW, bias],
+        flat FC gradient in state_dict order or None)."""
+        n = getattr(self, "_train_n", None)
+        if n is None:
+            raise B200Error("conv4_2_backward without a forward_train_conv4_2")
+        d = d_emb.to(device=self.device, dtype=torch.float32).contiguous()
+        if tuple(d.shape) != (n, 128):
+            raise ValueError(f"d_emb must be ({n}, 128), got {tuple(d.shape)}")
+        conv = torch.empty(CONV4_2_GRAD_COUNT, device=self.device, dtype=torch.float32)
+        fc = (torch.empty(int(_lib.lib().vmb_vggish_fc_grad_count()), device=self.device, dtype=torch.float32)
+              if want_fc else None)
+        with torch.cuda.device(self.device):
+            base, need = self._train_workspace(n, conv4_2=True)
+            check(_lib.lib().vmb_vggish_conv4_2_backward(self._h, base, need, ptr(d), n, ptr(conv),
+                                                         ptr(fc) if fc is not None else None, stream_ptr()),
+                  "vmb_vggish_conv4_2_backward")
+        return conv, fc
+
+    def _conv4_2_region(self, n: int, offset: int, nbytes: int) -> torch.Tensor:
+        base, _ = self._train_workspace(n, conv4_2=True)
+        off = base - self._train_ws.data_ptr() + offset
+        return self._train_ws[off:off + nbytes]
+
+    def train_conv4_1_output(self) -> torch.Tensor:
+        """(n, 12, 8, 512) float64 conv4_1 output of the last forward_train_conv4_2, as conv4_2 saw it (NHWC; split
+        mode: hi + lo)."""
+        n = self._train_n
+        L = _lib.lib()
+        off = int(L.vmb_vggish_fc_train_workspace_bytes(n)) - 2 * int(L.vmb_vggish_workspace_bytes(n))
+        if self.precision == "split":
+            t = self._conv4_2_region(n, off, n * 2 * 96 * 512 * 2).view(torch.bfloat16).view(n, 2, 12, 8, 512)
+            return t.double().sum(dim=1)
+        return self._conv4_2_region(n, off, n * 96 * 512 * 2).view(self.act_dtype).view(n, 12, 8, 512).double()
+
+    def train_conv4_2_z(self) -> torch.Tensor:
+        """(n, 12, 8, 512) fp32 pre-activation of conv4_2 from the last forward_train_conv4_2 (NHWC)."""
+        n = self._train_n
+        off = int(_lib.lib().vmb_vggish_fc_train_workspace_bytes(n))
+        return self._conv4_2_region(n, off, n * 96 * 512 * 4).view(torch.float32).view(n, 12, 8, 512)
+
+
+CONV4_2_GRAD_LAYOUT = (("weight", (512, 512, 3, 3)), ("bias", (512,)))
+CONV4_2_GRAD_COUNT = 512 * 512 * 9 + 512
+
+
+def conv4_2_grad_views(flat: torch.Tensor) -> dict:
+    """The flat conv4_2 gradient buffer as {features.13 key suffix: tensor view} in state_dict order."""
+    return _grad_views(flat, CONV4_2_GRAD_LAYOUT)
+
 
 FC_GRAD_LAYOUT = (("0.weight", (4096, 12288)), ("0.bias", (4096,)), ("2.weight", (4096, 4096)), ("2.bias", (4096,)),
                   ("4.weight", (128, 4096)), ("4.bias", (128,)))
@@ -334,8 +423,12 @@ FC_GRAD_LAYOUT = (("0.weight", (4096, 12288)), ("0.bias", (4096,)), ("2.weight",
 
 def fc_grad_views(flat: torch.Tensor) -> dict:
     """The flat FC gradient buffer as {embeddings key suffix: tensor view} in state_dict order."""
+    return _grad_views(flat, FC_GRAD_LAYOUT)
+
+
+def _grad_views(flat: torch.Tensor, layout) -> dict:
     out, off = {}, 0
-    for key, shape in FC_GRAD_LAYOUT:
+    for key, shape in layout:
         n = 1
         for s in shape:
             n *= s

@@ -56,7 +56,7 @@ fc_weight_planes_kernel(const float* __restrict__ w, int rows, int cols, __nv_bf
     const int r = r0 + ty + 8 * i, c = c0 + tx;
     const float v = __ldg(w + static_cast<long long>(r) * cols + c);
     tile[ty + 8 * i][tx] = v;
-    store3(v, planes + static_cast<long long>(r) * (kPl * cols) + c, cols);
+    if (planes) store3(v, planes + static_cast<long long>(r) * (kPl * cols) + c, cols);
   }
   if (!planes_t) return;
   __syncthreads();
@@ -202,7 +202,7 @@ int fc_train_forward(const void* const w_planes[3], const float* const bias[3], 
                      long long n, char* ws, const FcTrainLayout& L, float* emb, cudaStream_t st) {
   const long long np = L.n_pad;
   void* x = ws + L.x;
-  {
+  if (features) {
     const long long total = np * kFcTrainIn;
     const unsigned grid = static_cast<unsigned>(std::min<long long>((total + 255) / 256, 148LL * 16));
     fc_feature_planes_kernel<<<grid, 256, 0, st>>>(features, precision, n, np, static_cast<__nv_bfloat16*>(x));
@@ -222,7 +222,7 @@ int fc_train_forward(const void* const w_planes[3], const float* const bias[3], 
 }
 
 int fc_train_backward(const void* const wt_planes[3], long long n, char* ws, const FcTrainLayout& L,
-                      const float* d_emb, float* grads, cudaStream_t st) {
+                      const float* d_emb, float* grads, float* dx, cudaStream_t st) {
   const long long np = L.n_pad;
   const float* z1 = reinterpret_cast<const float*>(ws + L.z1);
   const float* z2 = reinterpret_cast<const float*>(ws + L.z2);
@@ -230,25 +230,30 @@ int fc_train_backward(const void* const wt_planes[3], long long n, char* ws, con
   float* da = reinterpret_cast<float*>(ws + L.da);
   void* g = ws + L.g;
   double* colsum = reinterpret_cast<double*>(ws + L.colsum);
+  const bool wgrad = grads != nullptr;
   float* dw[3] = {grads + kFcGradW1, grads + kFcGradW2, grads + kFcGradW3};
   float* db[3] = {grads + kFcGradB1, grads + kFcGradB2, grads + kFcGradB3};
-  double* cs[3] = {colsum, colsum + 4096, colsum + 8192};
-  if (cudaMemsetAsync(colsum, 0, size_t(4096 + 4096 + 128) * 8, st) != cudaSuccess) {
-    set_kernel_error("fc_train: column-sum clear failed");
-    return 1;
+  double* cs[3] = {nullptr, nullptr, nullptr};
+  if (wgrad) {
+    cs[0] = colsum, cs[1] = colsum + 4096, cs[2] = colsum + 8192;
+    if (cudaMemsetAsync(colsum, 0, size_t(4096 + 4096 + 128) * 8, st) != cudaSuccess) {
+      set_kernel_error("fc_train: column-sum clear failed");
+      return 1;
+    }
   }
   // fc3
   if (act(d_emb, z3, n, np, 128, g, nullptr, cs[2], st)) return 1;
-  if (gemm_dw(g, 128, ws + L.a2, 4096, dw[2], 128, 4096, np, st)) return 1;
+  if (wgrad && gemm_dw(g, 128, ws + L.a2, 4096, dw[2], 128, 4096, np, st)) return 1;
   if (gemm(g, wt_planes[2], nullptr, da, n, 4096, 128, st)) return 1;
   // fc2
   if (act(da, z2, n, np, 4096, g, nullptr, cs[1], st)) return 1;
-  if (gemm_dw(g, 4096, ws + L.a1, 4096, dw[1], 4096, 4096, np, st)) return 1;
+  if (wgrad && gemm_dw(g, 4096, ws + L.a1, 4096, dw[1], 4096, 4096, np, st)) return 1;
   if (gemm(g, wt_planes[1], nullptr, da, n, 4096, 4096, st)) return 1;
-  // fc1: weight and bias gradients only
+  // fc1: weight and bias gradients, and with dx the input gradient (K = 4096, sliced like fc2's dgrad)
   if (act(da, z1, n, np, 4096, g, nullptr, cs[0], st)) return 1;
-  if (gemm_dw(g, 4096, ws + L.x, kFcTrainIn, dw[0], 4096, kFcTrainIn, np, st)) return 1;
-  for (int i = 0; i < 3; ++i) {
+  if (wgrad && gemm_dw(g, 4096, ws + L.x, kFcTrainIn, dw[0], 4096, kFcTrainIn, np, st)) return 1;
+  if (dx && gemm(g, wt_planes[0], nullptr, dx, n, kFcTrainIn, 4096, st)) return 1;
+  for (int i = 0; i < 3 && wgrad; ++i) {
     const int nb = i == 2 ? 128 : 4096;
     fc_colsum_store_kernel<<<(nb + 255) / 256, 256, 0, st>>>(cs[i], db[i], nb);
     count_launch();

@@ -48,9 +48,12 @@ struct vmb_vggish {
   float* fc_b[3] = {};
   // train-mode FC stack (fc_train.cu): three-plane copies of the FC weights, allocated and derived by the first
   // vmb_vggish_refresh_fc — row-major [out][3 * in] for the forward GEMMs, transposed [in][3 * out] for the dgrad of
-  // fc2 and fc3 (fc1's input gradient is never formed)
+  // fc2 and fc3, and of fc1 once vmb_vggish_refresh_conv4_2 has allocated train_wt[0] (conv4_2 trained)
   void* train_w[3] = {};
   void* train_wt[3] = {};
+  // train-mode conv4_2 (conv_train.cu): three-plane copy of its weights [512][3 * 4608] in (kh, kw, c) order, allocated
+  // and derived by the first vmb_vggish_refresh_conv4_2, which also allocates fc1's transposed planes train_wt[0]
+  void* conv_train_w = nullptr;
   HostStage stage;
 };
 
@@ -85,8 +88,10 @@ bool fc_inference_copy(vmb_vggish* h, int i, const float* w, const float* b, cud
 }
 
 // conv1 + the five tensor-core convs into the ping-pong workspace; returns the buffer holding the (h, w, c)-flattened
-// features [n][12288] ([n][hi | lo] in split mode), or null after recording the error
-char* conv_stack(vmb_vggish* h, const float* examples, long long n, void* workspace, cudaStream_t st, const char* who) {
+// features [n][12288] ([n][hi | lo] in split mode), or null after recording the error.  convs = 4 stops after conv4_1:
+// the returned buffer (the workspace's first region) then holds conv4_1's output NHWC [n][12][8][512] ([n][2][...] split)
+char* conv_stack(vmb_vggish* h, const float* examples, long long n, void* workspace, cudaStream_t st, const char* who,
+                 int convs = 5) {
   const bool split = h->precision == 1;
   const int fmt = h->precision == 2 ? 1 : 0;
   int* sat = h->sat;   // null unless fp16
@@ -102,7 +107,7 @@ char* conv_stack(vmb_vggish* h, const float* examples, long long n, void* worksp
   }
   char* src = A;
   char* dst = B;
-  for (int i = 0; i < 5; ++i) {
+  for (int i = 0; i < convs; ++i) {
     const ConvGeom& g = kConv[i];
     vmb::StageTimer t(VMB_STAGE_CONV2 + i, st);
     const int rc = split ? vmb::igemm_conv3x3_split(src, h->conv_w[i + 1], h->conv_b[i + 1], dst, int(n), g.H, g.W, g.C_in,
@@ -196,6 +201,7 @@ void vmb_vggish_destroy(vmb_vggish_t* h) {
     cudaFree(h->train_w[i]);
     cudaFree(h->train_wt[i]);
   }
+  cudaFree(h->conv_train_w);
   if (h->sat) cudaFreeHost(h->sat);
   HostStage& hs = h->stage;
   for (int i = 0; i < 2; ++i) {
@@ -285,8 +291,10 @@ int vmb_vggish_forward(vmb_vggish_t* h, const float* examples, long long n, floa
 namespace {
 // the conv scratch of the train-mode workspace is sized for the split precision (the largest)
 vmb::FcTrainLayout train_layout(long long n) { return vmb::fc_train_layout(n, vmb_vggish_workspace_bytes(n) * 2); }
+vmb::Conv42Layout conv4_2_layout(long long n) { return vmb::conv4_2_layout(n, vmb_vggish_workspace_bytes(n) * 2); }
 
-int check_train_args(const vmb_vggish_t* h, long long n, const void* ws, size_t ws_bytes, const char* who) {
+int check_train_args(const vmb_vggish_t* h, long long n, const void* ws, size_t ws_bytes, const char* who,
+                     bool conv4_2 = false) {
   char msg[256];
   auto bad = [&](const char* why) {
     snprintf(msg, sizeof msg, "%s: %s", who, why);
@@ -299,7 +307,10 @@ int check_train_args(const vmb_vggish_t* h, long long n, const void* ws, size_t 
   if (n > 1000000) return bad("at most 1 000 000 examples per call");
   if (!ws) return bad("null workspace");
   if (reinterpret_cast<uintptr_t>(ws) % 1024) return bad("workspace must be 1024-byte aligned");
-  if (ws_bytes < train_layout(n).total) return bad("workspace too small for n examples");
+  if (conv4_2 && !h->conv_train_w)
+    return bad("no training copy of conv4_2's weights: call vmb_vggish_refresh_conv4_2 first");
+  if (ws_bytes < (conv4_2 ? conv4_2_layout(n).total : train_layout(n).total))
+    return bad("workspace too small for n examples");
   return 0;
 }
 }  // namespace
@@ -366,9 +377,79 @@ int vmb_vggish_fc_backward(vmb_vggish_t* h, void* workspace, size_t workspace_by
   if (!d_emb || !grads) return fail("vmb_vggish_fc_backward: null pointer");
   if (reinterpret_cast<uintptr_t>(grads) % 32) return fail("vmb_vggish_fc_backward: grads must be 32-byte aligned");
   const void* wt[3] = {nullptr, h->train_wt[1], h->train_wt[2]};
-  if (vmb::fc_train_backward(wt, n, static_cast<char*>(workspace), train_layout(n), d_emb, grads,
+  if (vmb::fc_train_backward(wt, n, static_cast<char*>(workspace), train_layout(n), d_emb, grads, nullptr,
                              static_cast<cudaStream_t>(stream)))
     return fail("vmb_vggish_fc_backward: %s", vmb::kernels_last_error());
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------ train-mode conv4_2
+size_t vmb_vggish_conv4_2_train_workspace_bytes(long long n) {
+  if (n <= 0) return 0;
+  return conv4_2_layout(n).total;
+}
+
+int vmb_vggish_refresh_conv4_2(vmb_vggish_t* h, const float* w, const float* b, const float* fc1_w, void* stream) {
+  if (!h) return fail("vmb_vggish_refresh_conv4_2: null handle");
+  if (!h->has_fc) return fail("vmb_vggish_refresh_conv4_2: this handle was built without the FC stack");
+  if (!w || !b || !fc1_w) return fail("vmb_vggish_refresh_conv4_2: null argument");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bool first = !h->conv_train_w;
+  if (first) {   // the only allocations; later calls reuse them
+    bool ok = cudaMalloc(&h->conv_train_w, size_t(512) * vmb::kConv42K * 2 * 3) == cudaSuccess;
+    if (ok && !h->train_wt[0]) ok = cudaMalloc(&h->train_wt[0], size_t(kFcOut[0]) * kFcIn[0] * 2 * 3) == cudaSuccess;
+    if (!ok) {
+      cudaFree(h->conv_train_w);
+      h->conv_train_w = nullptr;
+      return fail("vmb_vggish_refresh_conv4_2: allocation failed (%s)", cudaGetErrorString(cudaGetLastError()));
+    }
+  }
+  // the inference copy, with the create path's own kernels: bit for bit what vmb_vggish_create_ex would build
+  const ConvGeom& g = kConv[4];
+  if (cudaMemcpyAsync(h->conv_b[5], b, size_t(g.C_out) * 4, cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+    return fail("vmb_vggish_refresh_conv4_2: bias copy failed");
+  if ((h->precision == 1 ? vmb::relayout_conv_weight_split(w, h->conv_w[5], g.C_out, g.C_in, st)
+                         : vmb::relayout_conv_weight(w, h->conv_w[5], g.C_out, g.C_in, st, h->precision == 2 ? 1 : 0)))
+    return fail("vmb_vggish_refresh_conv4_2: %s", vmb::kernels_last_error());
+  if (vmb::conv4_2_weight_planes(w, h->conv_train_w, st))
+    return fail("vmb_vggish_refresh_conv4_2: %s", vmb::kernels_last_error());
+  // fc1's transposed planes (the dgrad of fc1); vmb_vggish_refresh_fc keeps them current from then on
+  if (first && vmb::fc_weight_planes(fc1_w, kFcOut[0], kFcIn[0], nullptr, h->train_wt[0], st))
+    return fail("vmb_vggish_refresh_conv4_2: %s", vmb::kernels_last_error());
+  return 0;
+}
+
+int vmb_vggish_forward_train_conv4_2(vmb_vggish_t* h, const float* examples, long long n, float* emb, void* workspace,
+                                     size_t workspace_bytes, void* stream) {
+  const char* who = "vmb_vggish_forward_train_conv4_2";
+  if (check_train_args(h, n, workspace, workspace_bytes, who, true)) return 1;
+  if (!examples || !emb) return fail("vmb_vggish_forward_train_conv4_2: null pointer");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const vmb::Conv42Layout L = conv4_2_layout(n);
+  char* ws = static_cast<char*>(workspace);
+  const char* act = conv_stack(h, examples, n, ws + L.fc.conv, st, who, 4);
+  if (!act) return 1;
+  if (vmb::conv4_2_train_forward(h->conv_train_w, h->conv_b[5], act, h->precision, n, ws, L, st))
+    return fail("vmb_vggish_forward_train_conv4_2: %s", vmb::kernels_last_error());
+  const void* w[3] = {h->train_w[0], h->train_w[1], h->train_w[2]};
+  const float* b[3] = {h->fc_b[0], h->fc_b[1], h->fc_b[2]};
+  if (vmb::fc_train_forward(w, b, nullptr, h->precision, n, ws, L.fc, emb, st))
+    return fail("vmb_vggish_forward_train_conv4_2: %s", vmb::kernels_last_error());
+  return 0;
+}
+
+int vmb_vggish_conv4_2_backward(vmb_vggish_t* h, void* workspace, size_t workspace_bytes, const float* d_emb,
+                                long long n, float* conv_grads, float* fc_grads, void* stream) {
+  if (check_train_args(h, n, workspace, workspace_bytes, "vmb_vggish_conv4_2_backward", true)) return 1;
+  if (!d_emb || !conv_grads) return fail("vmb_vggish_conv4_2_backward: null pointer");
+  if (reinterpret_cast<uintptr_t>(fc_grads) % 32) return fail("vmb_vggish_conv4_2_backward: fc_grads must be 32-byte aligned");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const vmb::Conv42Layout L = conv4_2_layout(n);
+  char* ws = static_cast<char*>(workspace);
+  const void* wt[3] = {h->train_wt[0], h->train_wt[1], h->train_wt[2]};
+  if (vmb::fc_train_backward(wt, n, ws, L.fc, d_emb, fc_grads, reinterpret_cast<float*>(ws + L.dx1), st) ||
+      vmb::conv4_2_train_backward(ws + L.fc.conv, h->precision, n, ws, L, conv_grads, st))
+    return fail("vmb_vggish_conv4_2_backward: %s", vmb::kernels_last_error());
   return 0;
 }
 

@@ -62,16 +62,19 @@ class B200HandleMixin:
         return tuple((t.data_ptr(), t._version) for t in tensors) + (str(dev),)
 
 
-def handle_action(old_key, new_key, fc_trainable: bool) -> str:
-    """What a change of the VGGish parameters does to the library handle.  A key is (conv part, FC part): the conv
-    part covers the conv tensors and the precision, the FC part the embeddings.* tensors.  "rebuild" (a new handle:
-    vmb_vggish_create_ex re-lays every weight and synchronises), "refresh" (only the FC weights changed and the handle
-    already holds a training copy of them: vmb_vggish_refresh_fc, stream-ordered), or "keep"."""
+def handle_action(old_key, new_key, fc_trainable: bool, conv4_2_trainable: bool = False) -> str:
+    """What a change of the VGGish parameters does to the library handle.  A key is (frozen convs, conv4_2, FCs) or
+    (convs, FCs): the first part covers the conv tensors it names and the precision, the conv4_2 part features.13.*,
+    the last part the embeddings.* tensors.  "rebuild" (a new handle: vmb_vggish_create_ex re-lays every weight and
+    synchronises), "refresh" (only parts the handle holds a training copy of changed: vmb_vggish_refresh_conv4_2 /
+    vmb_vggish_refresh_fc for each changed part, stream-ordered), or "keep"."""
     if old_key is None or old_key[0] != new_key[0]:
         return "rebuild"
-    if old_key[1] != new_key[1]:
-        return "refresh" if fc_trainable else "rebuild"
-    return "keep"
+    conv_changed = len(new_key) == 3 and old_key[1] != new_key[1]
+    fc_changed = old_key[-1] != new_key[-1]
+    if (conv_changed and not conv4_2_trainable) or (fc_changed and not fc_trainable):
+        return "rebuild"
+    return "refresh" if conv_changed or fc_changed else "keep"
 
 
 class _FcTrainFn(torch.autograd.Function):
@@ -100,6 +103,44 @@ class _FcTrainFn(torch.autograd.Function):
         names = [k for k, _ in m.embeddings.named_parameters()]
         grads = [views[k] if ctx.needs_input_grad[2 + i] else None for i, k in enumerate(names)]
         return (None, None, *grads)
+
+
+class _Conv42TrainFn(torch.autograd.Function):
+    """Train-mode VGGish with conv4_2 (features.13) trainable, conv1 .. conv4_1 frozen, fc1-fc3 trainable or frozen:
+    conv4_1's output, conv4_2's pre-activation and the FC stack's activations stay in the handle's train workspace,
+    which holds ONE forward: backward checks it is still this one."""
+
+    @staticmethod
+    def forward(ctx, module, x, n_conv, *params):
+        h = module._b200_handle(train=True, conv4_2=True)
+        emb = h.forward_train_conv4_2(x.detach().to(device=h.device, dtype=torch.float32))
+        module._fc_generation = getattr(module, "_fc_generation", 0) + 1
+        ctx.module, ctx.handle, ctx.generation, ctx.n_conv = module, h, module._fc_generation, n_conv
+        ctx.param_key = tuple((p.data_ptr(), p._version) for p in params)
+        return emb
+
+    @staticmethod
+    def backward(ctx, d_emb):
+        m = ctx.module
+        if ctx.generation != getattr(m, "_fc_generation", 0) or m._handle is not ctx.handle:
+            raise B200Error("backward of a stale VGGish forward: the library keeps the activations of ONE train-mode "
+                            "forward per module, and another train-mode forward ran before this backward; call "
+                            "backward() before the next forward")
+        if ctx.param_key != tuple((p.data_ptr(), p._version) for p in _conv4_2_params(m) + list(m.embeddings.parameters())):
+            raise B200Error("the VGGish conv4_2 or FC parameters changed between forward and backward")
+        need = ctx.needs_input_grad[3:]
+        conv, fc = ctx.handle.conv4_2_backward(d_emb, want_fc=any(need[ctx.n_conv:]))
+        names = [k for k, _ in m.features[13].named_parameters()]
+        views = _engine.conv4_2_grad_views(conv)
+        grads = [views[k] if need[i] else None for i, k in enumerate(names)]
+        names = [k for k, _ in m.embeddings.named_parameters()]
+        views = _engine.fc_grad_views(fc) if fc is not None else {}
+        grads += [views[k] if need[ctx.n_conv + i] else None for i, k in enumerate(names)]
+        return (None, None, None, *grads)
+
+
+def _conv4_2_params(vgg):
+    return list(vgg.features[13].parameters())
 
 
 def _body_tensors(features, embeddings):
@@ -135,35 +176,50 @@ class VGG(B200HandleMixin, nn.Module):
         self.b200_precision = precision
         return self
 
-    # -- library handle: rebuilt when a conv parameter was modified in place, replaced or moved; a change of the FC
-    # parameters alone (an optimiser step of FC fine-tuning) refreshes the FC weights of the existing handle
-    def _b200_handle(self, train: bool = False):
+    # -- library handle: rebuilt when a frozen conv parameter was modified in place, replaced or moved; a change of the
+    # FC parameters or of conv4_2's alone (an optimiser step of fine-tuning) refreshes those weights of the existing
+    # handle when it holds a training copy of them
+    def _b200_handle(self, train: bool = False, conv4_2: bool = False):
         named = _body_tensors(self.features, self.embeddings)
         dev = named[0][1].device
         if dev.type != "cuda":
             raise B200Error("VGGish parameters are on %s: move the module to a CUDA device (.to('cuda')); this build "
                             "has no CPU path" % dev)
         fc = [v for _, v in self.embeddings.named_parameters()]
-        key = (self._tensor_key(self.features.parameters(), dev) + (self.b200_precision,), self._tensor_key(fc, dev))
-        action = handle_action(self._handle_key if self._handle is not None else None, key,
-                               self._handle is not None and self._handle.fc_trainable)
+        c42 = _conv4_2_params(self)
+        frozen = [v for k, v in self.features.named_parameters() if not k.startswith("13.")]
+        key = (self._tensor_key(frozen, dev) + (self.b200_precision,), self._tensor_key(c42, dev),
+               self._tensor_key(fc, dev))
+        old = self._handle_key if self._handle is not None else None
+        action = handle_action(old, key, self._handle is not None and self._handle.fc_trainable,
+                               self._handle is not None and self._handle.conv4_2_trainable)
         if action == "rebuild":
             if self._handle is not None:
                 self._handle.close()
             self._handle = _engine.VggishHandle(dict(named), dev, precision=self.b200_precision)
-        if action == "refresh" or (train and not self._handle.fc_trainable):
-            self._handle.refresh_fc(fc[0::2], fc[1::2])
+        h = self._handle
+        if (action == "refresh" and old[2] != key[2]) or (train and not h.fc_trainable):
+            h.refresh_fc(fc[0::2], fc[1::2])
+        if (action == "refresh" and old[1] != key[1]) or (conv4_2 and not h.conv4_2_trainable):
+            h.refresh_conv4_2(c42[0], c42[1], fc[0])
         self._handle_key = key
-        return self._handle
+        return h
 
     def forward(self, x):
         if torch.is_grad_enabled() and self.training:
-            if any(p.requires_grad for p in self.features.parameters()):
-                raise NotImplementedError("training the VGGish conv stack is outside the B200 path (the reference "
-                                          "freezes it, model.py:159-160); fine-tuning the FC stack alone "
+            conv = [k for k, p in self.features.named_parameters() if p.requires_grad]
+            if any(not k.startswith("13.") for k in conv):
+                raise NotImplementedError("training the VGGish conv stack below conv4_2 is outside the B200 path (the "
+                                          "reference freezes it, model.py:159-160); fine-tuning conv4_2 "
+                                          "(set_requires_grad(vgg.features[13], True)) and / or the FC stack "
                                           "(set_requires_grad(vgg.embeddings, True)) is supported; otherwise call "
                                           "set_requires_grad(module, False) or .eval()")
             fc = list(self.embeddings.parameters())
+            if conv:
+                if not isinstance(x, torch.Tensor):
+                    raise TypeError("expected a (N, 1, 96, 64) tensor")
+                c42 = _conv4_2_params(self)
+                return _Conv42TrainFn.apply(self, x, len(c42), *c42, *fc)
             if any(p.requires_grad for p in fc):
                 if not isinstance(x, torch.Tensor):
                     raise TypeError("expected a (N, 1, 96, 64) tensor")
@@ -207,6 +263,10 @@ class VGGishFeatures(B200HandleMixin, nn.Sequential):
         return self._handle
 
     def forward(self, x):
+        if torch.is_grad_enabled() and self.training and any(p.requires_grad for p in self[0].parameters()):
+            raise NotImplementedError("training the VGGish conv stack behind the wide head (just_bottlenecks) is "
+                                      "outside the B200 path: the head forms no gradient with respect to the 12288-d "
+                                      "features; call set_requires_grad(module, False) or .eval()")
         h = self._b200_handle()
         x = x.detach().to(device=h.device, dtype=torch.float32)
         return h.forward(x, want_bottleneck=True, want_embeddings=False)[1].float()

@@ -210,6 +210,40 @@ int vmb_vggish_forward_train(vmb_vggish_t* handle, const float* examples_dev, lo
 int vmb_vggish_fc_backward(vmb_vggish_t* handle, void* workspace_dev, size_t workspace_bytes, const float* d_emb_dev,
                            long long n, float* grads_dev, void* stream);
 
+/* ------------------------------------------------------------------------------------------ VGGish conv4_2 fine-tuning
+ * Training features.13 (conv4_2, the last Conv2d(512, 512, 3, padding=1) of vggish.py:108-118) with conv1 .. conv4_1
+ * frozen, optionally together with fc1-fc3: the reference's loop with those parameters unfrozen (model.py:159-160) and
+ * given to its Adam (train.py:130-138).  conv1 .. conv4_1 run exactly as in vmb_vggish_forward (same kernels, the
+ * handle's precision).  conv4_2 runs in fp32-equivalent arithmetic: three-plane split-bf16 operands from an im2col of
+ * conv4_1's output and a training copy of the weights, its 4 608-column contraction cut into slices of 768 columns
+ * (DESIGN §5.5c).  Then ReLU, the 2x2 max-pool, the (h, w, c) flatten, and the FC stack as in vmb_vggish_forward_train.
+ * The gradient stops at conv4_2's weights: no input gradient of conv4_2 is formed.
+ *
+ * vmb_vggish_refresh_conv4_2: fp32 masters w_dev OIHW [512][512][3][3], b_dev [512] -> conv4_2's inference copy in the
+ *   handle's precision (bit for bit what vmb_vggish_create_ex would build) and its training planes.  The first call
+ *   allocates the training planes (14 MB) and fc1's transposed planes (302 MB), which it derives from fc1_w_dev
+ *   [4096][12288]; vmb_vggish_refresh_fc keeps them current afterwards.  Stream-ordered, no synchronisation.
+ * vmb_vggish_forward_train_conv4_2: examples fp32 [n][96][64] -> emb_dev fp32 [n][128].  Needs vmb_vggish_refresh_fc
+ *   and vmb_vggish_refresh_conv4_2 first.  The workspace (vmb_vggish_conv4_2_train_workspace_bytes(n), 1024-byte
+ *   aligned) begins with the layout of vmb_vggish_fc_train_workspace_bytes(n) (F bytes), so it too starts with fc1's
+ *   input planes bf16 [pad64(n)][3][12288].  Regions the caller may read (byte offsets, each rounded up to 1024):
+ *     conv4_1's output at F - 2 * vmb_vggish_workspace_bytes(n): NHWC [n][12][8][512] in the handle's precision
+ *       (bf16 / fp16; split: [n][2][12][8][512], hi plane then lo plane per example);
+ *     z at F: conv4_2's fp32 pre-activation [n * 96][512], row = example * 96 + h * 8 + w;
+ *   followed by dz planes bf16 [n * 96][3 * 512], fc1's input gradient fp32 [n][12288], the weight gradient fp32
+ *   [512][4608], bias sums double [512], and the im2col planes of one chunk, bf16 [min(n, 256) * 96][3 * 4608].
+ * vmb_vggish_conv4_2_backward: d(loss)/d(emb) fp32 [n][128] of the last vmb_vggish_forward_train_conv4_2 on this
+ *   workspace -> conv_grads_dev fp32 [512 * 512 * 9 + 512]: features.13.weight [512][512][3][3], then .bias [512]; and,
+ *   when fc_grads_dev is not null (32-byte aligned), the flat FC gradient of vmb_vggish_fc_backward.             */
+size_t vmb_vggish_conv4_2_train_workspace_bytes(long long n_examples);
+int vmb_vggish_refresh_conv4_2(vmb_vggish_t* handle, const float* w_dev, const float* b_dev, const float* fc1_w_dev,
+                               void* stream);
+int vmb_vggish_forward_train_conv4_2(vmb_vggish_t* handle, const float* examples_dev, long long n, float* emb_dev,
+                                     void* workspace_dev, size_t workspace_bytes, void* stream);
+int vmb_vggish_conv4_2_backward(vmb_vggish_t* handle, void* workspace_dev, size_t workspace_bytes,
+                                const float* d_emb_dev, long long n, float* conv_grads_dev, float* fc_grads_dev,
+                                void* stream);
+
 /* ------------------------------------------------------------------------------------------ MLA head
  * MultiLevelAttention.forward in eval mode (model.py:258-269; EmbeddedMapping :217-222, AttentionModule
  * :236-242).  `params_dev` is one flat fp32 device buffer holding, in this order (T = time steps):
