@@ -3,7 +3,6 @@
 
 #include <atomic>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -193,14 +192,12 @@ igemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
             }
             if (++tap == 9) { tap = 0; ++cb; }
           } else {
-            // split mode (p.split_nkb > 0): A and B are stored as column blocks of 2 (hi | lo) or 3 (hi | mid | lo)
-            // bf16 planes and the K loop runs over the products with plane index sum <= planes - 1, smallest first
-            // (see igemm_linear_split)
+            // split mode (p.split_nkb > 0): A and B are stored as column blocks of hi | lo bf16 planes and the K loop
+            // runs over the products hi * hi, lo * hi, hi * lo (see igemm_linear_split_out)
             int a_kb = kb;
             if (p.split_nkb) {
               const int q = kb / p.split_nkb;
-              const int pa = p.split_planes == 3 ? ((0x210100 >> (4 * (5 - q))) & 0xF) : (q == 1 ? 1 : 0);
-              a_kb = pa * p.split_nkb + (kb - q * p.split_nkb);
+              a_kb = (q == 1 ? 1 : 0) * p.split_nkb + (kb - q * p.split_nkb);
             }
 #pragma unroll
             for (int sub = 0; sub < MT; ++sub)
@@ -208,10 +205,9 @@ igemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_const
                           (m_tile * MT + sub) * kBlockM);
           }
           int b_kb = CONV ? b_conv_kb : kb;
-          if (p.split_nkb) {
+          if (!CONV && p.split_nkb) {
             const int q = kb / p.split_nkb;
-            const int pb = p.split_planes == 3 ? ((0x012010 >> (4 * (5 - q))) & 0xF) : (q == 2 ? 1 : 0);
-            b_kb = pb * p.split_nkb + (kb - q * p.split_nkb);
+            b_kb = (q == 2 ? 1 : 0) * p.split_nkb + (kb - q * p.split_nkb);
           }
           tma_load_2d(b_dst, &tmap_b, &full_bar[stage], b_kb * kBlockK, n_tile * BLOCK_N);
           if (++stage == C::kStages) { stage = 0; phase ^= 1; }
@@ -547,43 +543,13 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tb, const IgemmParams& p, c
 
 const char* igemm_last_error() { return g_err; }
 
-#ifndef VMB_PAIR_DEFAULT
-#define VMB_PAIR_DEFAULT 1
-#endif
 namespace {
-std::atomic<int> g_pair_override{-1};   // -1: follow the environment / build default
+std::atomic<int> g_use_pair{1}, g_use_halo{1};
 }
-bool igemm_use_pair() {
-  const int o = g_pair_override.load(std::memory_order_relaxed);
-  if (o >= 0) return o != 0;
-  static const bool on = [] {
-    const char* e = getenv("VMB_IGEMM_PAIR");
-    return e ? (e[0] != '0') : (VMB_PAIR_DEFAULT != 0);
-  }();
-  return on;
-}
-namespace {
-std::atomic<int> g_halo_override{-1};
-}
-bool igemm_use_halo() {
-  const int o = g_halo_override.load(std::memory_order_relaxed);
-  if (o >= 0) return o != 0;
-  static const bool on = [] {
-    const char* e = getenv("VMB_IGEMM_HALO");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-int igemm_set_halo(int on) {
-  const int prev = igemm_use_halo() ? 1 : 0;
-  g_halo_override.store(on < 0 ? -1 : (on ? 1 : 0), std::memory_order_relaxed);
-  return prev;
-}
-int igemm_set_pair(int on) {
-  const int prev = igemm_use_pair() ? 1 : 0;
-  g_pair_override.store(on < 0 ? -1 : (on ? 1 : 0), std::memory_order_relaxed);
-  return prev;
-}
+bool igemm_use_pair() { return g_use_pair.load(std::memory_order_relaxed) != 0; }
+bool igemm_use_halo() { return g_use_halo.load(std::memory_order_relaxed) != 0; }
+int igemm_set_pair(int on) { return g_use_pair.exchange(on != 0, std::memory_order_relaxed); }
+int igemm_set_halo(int on) { return g_use_halo.exchange(on != 0, std::memory_order_relaxed); }
 
 namespace {
 int pair_result(int rc) {
@@ -675,60 +641,6 @@ int igemm_linear_rect(const void* a, const void* w, const float* bias, void* out
                        : launch<128, 1, false, false, kOutBf16>(ta, tb, p, stream);
 }
 
-int igemm_linear_split(const void* a_planes, const void* w_planes, const float* bias, float* out, long long ldo,
-                       int relu, int M, int N, int K, cudaStream_t stream, int planes) {
-  if (M <= 0) return 0;
-  if (misaligned32(out, "igemm_linear_split")) return 1;
-  if (ldo % 8 != 0) {
-    snprintf(g_err, sizeof g_err, "igemm_linear_split: ldo must be a multiple of 8 floats (32-byte rows), got %lld", ldo);
-    return 1;
-  }
-  if (planes != 2 && planes != 3) {
-    snprintf(g_err, sizeof g_err, "igemm_linear_split: planes must be 2 or 3");
-    return 1;
-  }
-  if (K % kBlockK != 0 || N % 128 != 0) {
-    snprintf(g_err, sizeof g_err, "igemm_linear_split: need K %% 64 == 0 and N %% 128 == 0 (got K=%d N=%d)", K, N);
-    return 1;
-  }
-  if (planes_gemm_enabled()) {
-    // every plane of a K-block loaded once per tile (planes_gemm_sm100.cu); the kernel below is kept for A/B timing
-    if (planes_gemm(a_planes, w_planes, bias, out, ldo, relu, M, N, K, planes, 0, stream)) {
-      snprintf(g_err, sizeof g_err, "%s", planes_gemm_last_error());
-      return 1;
-    }
-    return 0;
-  }
-  const int block_n = (N % 256 == 0) ? 256 : 128;
-  CUtensorMap ta, tb;
-  {
-    uint64_t dims[2] = {uint64_t(planes) * K, uint64_t(M)};
-    uint64_t str[1] = {uint64_t(planes) * K * 2};
-    uint32_t box[2] = {kBlockK, kBlockM};
-    if (make_tmap_bf16(&ta, a_planes, 2, dims, str, box)) return 1;
-  }
-  {
-    uint64_t dims[2] = {uint64_t(planes) * K, uint64_t(N)};
-    uint64_t str[1] = {uint64_t(planes) * K * 2};
-    uint32_t box[2] = {kBlockK, uint32_t(block_n)};
-    if (make_tmap_bf16(&tb, w_planes, 2, dims, str, box)) return 1;
-  }
-  IgemmParams p{};
-  p.M = M;
-  p.N = N;
-  p.split_nkb = K / kBlockK;
-  p.split_planes = planes;
-  p.num_kb = (planes == 3 ? 6 : 3) * p.split_nkb;
-  p.num_m_tiles = (M + kBlockM - 1) / kBlockM;
-  p.num_n_tiles = N / block_n;
-  p.relu = relu;
-  p.ldo = ldo;
-  p.bias = bias;
-  p.out = out;
-  return block_n == 256 ? launch<256, 1, false, false, kOutF32>(ta, tb, p, stream)
-                        : launch<128, 1, false, false, kOutF32>(ta, tb, p, stream);
-}
-
 int igemm_linear_split_out(const void* a_planes, const void* w_planes, const float* bias, void* out_planes, int relu,
                            int M, int N, int K, cudaStream_t stream) {
   if (M <= 0) return 0;
@@ -754,7 +666,6 @@ int igemm_linear_split_out(const void* a_planes, const void* w_planes, const flo
   p.M = M;
   p.N = N;
   p.split_nkb = K / kBlockK;
-  p.split_planes = 2;
   p.num_kb = 3 * p.split_nkb;
   p.num_m_tiles = (M + kBlockM - 1) / kBlockM;
   p.num_n_tiles = N / 256;

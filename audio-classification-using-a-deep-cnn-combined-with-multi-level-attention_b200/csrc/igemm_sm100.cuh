@@ -42,8 +42,7 @@ struct IgemmParams {
   int num_m_tiles;
   int num_n_tiles;
   int relu;
-  int split_nkb;     // PLAIN split mode: K / 64 of one plane (0 = ordinary GEMM)
-  int split_planes;  // 2 (hi | lo: 3 products) or 3 (hi | mid | lo: 6 products)
+  int split_nkb;     // PLAIN split mode (hi | lo planes, 3 products): K / 64 of one plane (0 = ordinary GEMM)
   int ksplit;        // PLAIN + atomic fp32 output: number of K slices (<= 1: none)
   int tile_count;    // pair kernel: process only the first tile_count tiles (0 = all); see igemm_pair_linear
   int conv_split;    // CONV: activations are [n][2][H][W][C] hi | lo planes, weights [C_out][2 * 9 C_in]
@@ -61,15 +60,9 @@ struct IgemmParams {
 // fmt: kFmtBf16 (0) or kFmtF16 (1) — the element format of a, w and of a 16-bit out; sat_flag: see IgemmParams.
 int igemm_linear(const void* a_bf16, const void* w_bf16, const float* bias, void* out, int out_f32, int relu,
                  int M, int N, int K, cudaStream_t stream, int fmt = 0, int* sat_flag = nullptr);
-// PLAIN, split-bf16.  planes = 2: A = [A_hi | A_lo] as bf16 [M][2K], W likewise [N][2K];
-// out fp32 [M][ldo] = act(A_hi W_hi^T + A_lo W_hi^T + A_hi W_lo^T + bias): ~16 mantissa bits per operand (the
-// eval-mode attention head, where plain bf16 would move the ranking metric).  planes = 3: [hi | mid | lo] as
-// [M][3K], the six products with plane-index sum <= 2: fp32-equivalent operands (head training, where ReLU masks
-// must not flip against the fp32 reference).  bias may be null.  K % 64 == 0, N % 128 == 0.
-int igemm_linear_split(const void* a_planes, const void* w_planes, const float* bias, float* out, long long ldo,
-                       int relu, int M, int N, int K, cudaStream_t stream, int planes = 2);
-// Split in, split out (the accuracy mode of the VGGish body): out planes bf16 [M][hi(N) | lo(N)] =
-// split(act(A_hi W_hi^T + A_lo W_hi^T + A_hi W_lo^T + bias)).  K % 64 == 0, N % 256 == 0.
+// PLAIN, split-bf16 in and out (the accuracy mode of the VGGish body): A = [A_hi | A_lo] as bf16 [M][2K], W likewise
+// [N][2K]; out planes bf16 [M][hi(N) | lo(N)] = split(act(A_hi W_hi^T + A_lo W_hi^T + A_hi W_lo^T + bias)).
+// K % 64 == 0, N % 256 == 0.
 int igemm_linear_split_out(const void* a_planes, const void* w_planes, const float* bias, void* out_planes, int relu,
                            int M, int N, int K, cudaStream_t stream);
 // CONV 3x3 with hi | lo activations [n][2][H][W][C_in], hi | lo weights [C_out][2 * 9 C_in] and hi | lo output
@@ -82,7 +75,7 @@ int igemm_conv3x3(const void* act_bf16, const void* w_bf16, const float* bias, v
                   int W, int C_in, int C_out, int pool, cudaStream_t stream, int fmt = 0, int* sat_flag = nullptr);
 
 // CTA-pair (cta_group::2) kernels for the bf16 layers with C_out / N a multiple of 256 (igemm_pair_sm100.cu);
-// igemm_conv3x3 / igemm_linear route to them when igemm_use_pair() (env VMB_IGEMM_PAIR=0/1 overrides the default).
+// igemm_conv3x3 / igemm_linear route to them when igemm_use_pair().
 int igemm_pair_linear(const void* a_bf16, const void* w_bf16, const float* bias, void* out_bf16, int relu, int M, int N,
                       int K, cudaStream_t stream, int fmt = 0, int* sat_flag = nullptr);
 int igemm_pair_conv3x3(const void* act_bf16, const void* w_bf16, const float* bias, void* out_bf16, int n_img, int H,
@@ -92,11 +85,13 @@ const char* igemm_pair_last_error();
 // act(A[M][K] W[N][K]^T + bias); used by igemm_pair_linear for the tiles of an incomplete last round.
 int igemm_linear_rect(const void* a_bf16, const void* w_bf16, const float* bias, void* out_bf16, long long ldo, int relu,
                          int M, int N, int K, cudaStream_t stream, int fmt = 0, int* sat_flag = nullptr);
+// On by default; igemm_set_pair(0) selects the single-CTA kernels (the reference of the bit-identity tests), 1 or -1
+// turns the pair kernels back on.  Returns the previous setting (0 / 1).
 bool igemm_use_pair();
 int igemm_set_pair(int on);
-// Haloed activation boxes for the C_out = 128 conv (conv2): same contract as igemm_set_pair.
+// Haloed activation boxes for the C_out = 128 conv (conv2): same contract as igemm_set_pair, 0 selects one box per tap.
 bool igemm_use_halo();
-int igemm_set_halo(int on);   // 1 / 0 force the choice, -1 returns to the default; returns the previous setting
+int igemm_set_halo(int on);
 
 const char* igemm_last_error();
 
@@ -118,7 +113,8 @@ __device__ __forceinline__ float dropout_scale(unsigned long long seed, unsigned
   return u >= p ? 1.f / (1.f - p) : 0.f;
 }
 
-// The three-plane split of the training GEMMs' operands (hi | mid | lo, planes = 3 above): fp32-equivalent operands.
+// The three-plane split of the training GEMMs' operands (hi | mid | lo, planes = 3 in planes_gemm below):
+// fp32-equivalent operands.
 __device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bfloat16& mid, __nv_bfloat16& lo) {
   hi = __float2bfloat16_rn(v);
   const float r1 = v - __bfloat162float(hi);      // exact
@@ -127,10 +123,13 @@ __device__ __forceinline__ void split_bf16(float v, __nv_bfloat16& hi, __nv_bflo
 }
 
 // planes_gemm_sm100.cu: the split GEMMs with every operand plane of a K-block loaded once per tile and the hi * hi
-// product in its own TMEM accumulator.  The training paths call it directly; igemm_linear_split (the eval-mode head)
-// routes to it when planes_gemm_enabled() (default; env VMB_PLANES_GEMM=0 selects the long-K-loop kernel above).
+// product in its own TMEM accumulator.  a_planes bf16 [M][planes * K], b_planes bf16 [N][planes * K], out fp32 [M][ldo].
+// planes = 2 (hi | lo, the products hi*hi + lo*hi + hi*lo): ~16 mantissa bits per operand — the eval-mode attention head
+// and fc3 in split precision, where plain bf16 would move the ranking metric.  planes = 3 (hi | mid | lo, the six
+// products with plane-index sum <= 2): fp32-equivalent operands — training, where ReLU masks must not flip against the
+// fp32 reference.  bias may be null.  K % 32 == 0, N % 128 == 0.
 // ksplit > 1: that many K slices, vector reductions into a zeroed out; ksplit == -1: one slice but still adding into
-// out; ksplit == 0: plain stores (+ bias, optional ReLU).
+// out; ksplit == 0: plain stores (+ bias, optional ReLU) of 32-byte rows, so out must be 32-byte aligned and ldo % 8 == 0.
 int planes_gemm(const void* a_planes, const void* b_planes, const float* bias, float* out, long long ldo, int relu, int M,
                 int N, int K, int planes, int ksplit, cudaStream_t stream);
 // Fused epilogue of the eval-mode head (two planes, no K split): the accumulator row u of (clip, time step
@@ -195,7 +194,6 @@ constexpr int kFwdSlice = 768, kDwSlice = 1024;
 // out (M rows of ldo floats) on the stream first whenever the slices add into it.
 int planes_gemm_dw(const void* a_planes, int a_cols, const void* b_planes, int b_cols, float* out, long long ldo, int M,
                    int N, int K, int planes, cudaStream_t stream);
-bool planes_gemm_enabled();
 const char* planes_gemm_last_error();
 
 // Shared host helpers (igemm_sm100.cu): bf16 tensor map with 128- or 64-byte swizzle (error text goes to

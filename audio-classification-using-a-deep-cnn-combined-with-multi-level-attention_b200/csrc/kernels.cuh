@@ -15,7 +15,6 @@ int check_launch(const char* what);
 
 // Launch `kern` so that it may overlap the tail of the previous kernel in the stream (programmatic dependent launch).
 // Only for kernels that call pdl_wait() (sm100_ptx.cuh) before their first access to global memory.
-bool pdl_enabled();   // environment VMB_PDL=0 turns the overlap off (A/B timing); profile.cu
 template <typename... KArgs, typename... Args>
 cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -27,7 +26,7 @@ cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t sme
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

@@ -9,7 +9,7 @@
 //    products.  Its header comment has the algebra and the data flow.
 //  * split_wave_kernel + logmel_tc_kernel (first half, the first tensor-core version): the waveform is split into three
 //    bf16 planes in HBM, A tiles are TMA boxes of an overlapping-rows view of those planes, straight K = 400 DFT, six
-//    products.  Serves inputs that are not 16-byte aligned; VMB_LOGMEL_PLANES=1 selects it for A/B runs.
+//    products.  Serves inputs that are not 16-byte aligned.
 //
 //   S[f][c] = sum_n x[160 f + n] * W[n][c],   W[n][2j] = hann[n] cos(2 pi k_j n / 512), W[n][2j+1] = hann[n] sin(..)
 //   |X_j| = sqrt(S[f][2j]^2 + S[f][2j+1]^2);  mel[f][m] = sum_j |X_j| M[k_j][m];  out = log(mel + 0.01)
@@ -37,7 +37,6 @@
 #include <cuda_runtime.h>
 
 #include <cmath>
-#include <cstdlib>
 #include <mutex>
 #include <vector>
 
@@ -1261,16 +1260,6 @@ int get_tables(TcTables** out) {
 // plane; a multiple of 160 keeps every stride a multiple of the 320-byte frame stride
 long long logmel_tc_pitch(long long samples_per_clip) { return (samples_per_clip + 16 + kHop - 1) / kHop * kHop; }
 
-// VMB_LOGMEL_PLANES=1 selects the first tensor-core version (split_wave_kernel + logmel_tc_kernel: K = 400 straight DFT
-// over TMA-framed sample planes), kept for A/B timing and as an on-device cross-check of the centred kernel.
-bool logmel_use_planes() {
-  static const bool on = [] {
-    const char* e = std::getenv("VMB_LOGMEL_PLANES");
-    return e && e[0] == '1';
-  }();
-  return on;
-}
-
 // The raw sample tiles are TMA boxes, so the clip base and the clip stride must be 16-byte aligned; other inputs
 // take the plane kernel, which accepts any alignment.
 template <class IN>
@@ -1345,7 +1334,7 @@ int logmel_tc_forward_impl(const IN* wave, long long n_clips, long long samples_
     set_kernel_error("logmel: too many clips / frames for one launch");
     return 1;
   }
-  if (!logmel_use_planes() && logmel_eo_accepts(wave, n_clips, clip_stride))
+  if (logmel_eo_accepts(wave, n_clips, clip_stride))
     return logmel_eo_forward<IN>(t, wave, n_clips, clip_stride, frames_out, logmel, stream);
   constexpr int a_planes = sizeof(IN) == 2 ? 2 : 3;
   const long long pitch = logmel_tc_pitch(samples_per_clip);

@@ -57,7 +57,7 @@ struct Handle {
 
 // Tensor-core forward (mla_tc.cu).  Returns 0 / 1 (message via vmb::kernels_last_error()).
 int tc_forward(Handle& h, const float* emb, long long batch, float* scores, cudaStream_t st);
-// 1 / 0 force the fused-epilogue forward on / off, -1 returns to the default; returns the previous override (-1/0/1)
+// 0 selects the unfused forward, 1 or -1 the fused-epilogue forward (the default); returns the previous setting (0 / 1)
 int mla_fuse_set(int on);
 // One level's EmbeddedMapping / AttentionModule on its own (model.py:217-222, :235-242), from the same kernels.
 int tc_embedded_mapping(const Handle& h, int level, const float* x, long long batch, float* out, cudaStream_t st);

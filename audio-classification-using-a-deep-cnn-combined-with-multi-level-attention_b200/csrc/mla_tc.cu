@@ -1,6 +1,6 @@
 // Multi-level attention head, eval mode, on the tensor cores (reference model.py:199-269).
 //
-// Every Linear of the head is a split-bf16 tcgen05 GEMM (igemm_linear_split: operands carried as hi + lo bf16
+// Every Linear of the head is a split-bf16 tcgen05 GEMM (planes_gemm with two planes: operands carried as hi + lo bf16
 // planes, three products, fp32 accumulation — ~16 mantissa bits, so the head adds nothing visible to the ranking
 // metric); the glue between GEMMs is three small kernels:
 //   rows_affine_split   v = [a2_t * ] relu?(a1_t * u + b1_t) [+ b2_t]  -> hi | lo planes   (BatchNorm1d(T) in eval mode
@@ -13,7 +13,6 @@
 
 #include <algorithm>
 #include <atomic>
-#include <cstdlib>
 
 #include "igemm_sm100.cuh"
 #include "kernels.cuh"
@@ -242,28 +241,25 @@ size_t up(size_t v) { return (v + 1023) / 1024 * 1024; }
 
 }  // namespace
 
-// VMB_MLA_FORK=0 keeps every kernel of the head on the caller's stream (A/B timing; results are identical either way)
-static bool mla_fork_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("VMB_MLA_FORK");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
+// Fused GEMM epilogues (planes_gemm_fused), on by default; mla_fuse_set(0) keeps the stand-alone affine / split / sigmoid
+// passes, the reference of the bit-identity tests.
+static std::atomic<int> g_fuse{1};
+int mla_fuse_set(int on) { return g_fuse.exchange(on != 0, std::memory_order_relaxed); }
 
-// Fused GEMM epilogues (planes_gemm_fused): default on whenever the planes GEMM kernel is; VMB_MLA_FUSE=0 or
-// mla_fuse_set(0) keep the stand-alone affine / split / sigmoid passes (A/B timing and the bit-identity test).
-static std::atomic<int> g_fuse_override{-1};
-int mla_fuse_set(int on) { return g_fuse_override.exchange(on < 0 ? -1 : (on ? 1 : 0), std::memory_order_relaxed); }
-static bool mla_fuse_enabled() {
-  if (!vmb::planes_gemm_enabled()) return false;
-  const int o = g_fuse_override.load(std::memory_order_relaxed);
-  if (o >= 0) return o != 0;
-  static const bool on = [] {
-    const char* e = getenv("VMB_MLA_FUSE");
-    return !(e && e[0] == '0');
-  }();
-  return on;
+// With more than one level, each level's attention branch but the last runs on the handle's side stream: created on
+// first use together with the events that fork and join it.
+static int ensure_side_stream(Handle& h) {
+  if (h.side) return 0;
+  bool ok = cudaStreamCreateWithFlags(&h.side, cudaStreamNonBlocking) == cudaSuccess;
+  for (int i = 0; i < kMaxLevels && ok; ++i)
+    ok = cudaEventCreateWithFlags(&h.fork_ev[i], cudaEventDisableTiming) == cudaSuccess &&
+         cudaEventCreateWithFlags(&h.gemm_ev[i], cudaEventDisableTiming) == cudaSuccess &&
+         cudaEventCreateWithFlags(&h.join_ev[i], cudaEventDisableTiming) == cudaSuccess;
+  if (!ok) {
+    vmb::set_kernel_error("mla: cannot create the side stream: %s", cudaGetErrorString(cudaGetLastError()));
+    return 1;
+  }
+  return 0;
 }
 
 static int tc_forward_fused(Handle& h, const float* emb, long long batch, float* scores, cudaStream_t st);
@@ -271,7 +267,7 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
 int tc_forward(Handle& h, const float* emb, long long batch, float* scores, cudaStream_t st) {
   const HeadDev& d = h.dev;
   const size_t pool_smem = size_t(2) * d.T * ((d.K + 31) & ~31) * sizeof(float);
-  if (mla_fuse_enabled() && pool_smem <= 48 * 1024) return tc_forward_fused(h, emb, batch, scores, st);
+  if (g_fuse.load(std::memory_order_relaxed) && pool_smem <= 48 * 1024) return tc_forward_fused(h, emb, batch, scores, st);
   const long long rows = batch * d.T;
   if (rows > 0x7fffffffLL) {
     vmb::set_kernel_error("mla: too many rows for one call");
@@ -287,19 +283,8 @@ int tc_forward(Handle& h, const float* emb, long long batch, float* scores, cuda
   // The attention branch of a level (z = fcv(emb_l), pooling) does not feed the next level: with more than one level it
   // runs on the handle's side stream, concurrently with the next level's Linear chain (these kernels are 4-22 us each
   // on a fraction of the SMs, so two of them share the GPU).  Needs its own fp32 GEMM output per forked level.
-  bool fork = d.n_levels > 1 && mla_fork_enabled();
-  if (fork && !h.side) {
-    bool ok = cudaStreamCreateWithFlags(&h.side, cudaStreamNonBlocking) == cudaSuccess;
-    for (int i = 0; i < kMaxLevels && ok; ++i)
-      ok = cudaEventCreateWithFlags(&h.fork_ev[i], cudaEventDisableTiming) == cudaSuccess &&
-           cudaEventCreateWithFlags(&h.gemm_ev[i], cudaEventDisableTiming) == cudaSuccess &&
-           cudaEventCreateWithFlags(&h.join_ev[i], cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) {
-      vmb::set_kernel_error("mla: cannot create the side stream: %s", cudaGetErrorString(cudaGetLastError()));
-      return 1;
-    }
-  }
-  const int n_fork = fork ? d.n_levels - 1 : 0;
+  if (d.n_levels > 1 && ensure_side_stream(h)) return 1;
+  const int n_fork = d.n_levels - 1;
   const size_t total = sz_x + 3 * sz_p + (1 + n_fork) * sz_u + sz_y + sz_yp;
   char* ws = nullptr;
   if (cudaMallocAsync(reinterpret_cast<void**>(&ws), total, st) != cudaSuccess) {
@@ -315,8 +300,8 @@ int tc_forward(Handle& h, const float* emb, long long batch, float* scores, cuda
   void* Yp = ws + sz_x + 3 * sz_p + (1 + n_fork) * sz_u + sz_y;
   int rc = 0;
   auto gemm_to = [&](const void* a, const FcDev& fc, float* out, cudaStream_t s) {
-    if (!rc && vmb::igemm_linear_split(a, fc.wp, fc.bias, out, hpad, 0, int(rows), hpad, fc.kpad, s)) {
-      vmb::set_kernel_error("mla: %s", vmb::igemm_last_error());
+    if (!rc && vmb::planes_gemm(a, fc.wp, fc.bias, out, hpad, 0, int(rows), hpad, fc.kpad, 2, 0, s)) {
+      vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
       rc = 1;
     }
   };
@@ -348,7 +333,7 @@ int tc_forward(Handle& h, const float* emb, long long batch, float* scores, cuda
       pp ^= 1;
     }
     // attention branch of this level: on the side stream unless it is the last level (nothing left to overlap with)
-    const bool side = fork && l + 1 < d.n_levels;
+    const bool side = l + 1 < d.n_levels;
     cudaStream_t as = side ? h.side : st;
     float* Uz = side ? U + (1 + l) * (sz_u / sizeof(float)) : U;
     if (side && !rc) {
@@ -376,11 +361,11 @@ int tc_forward(Handle& h, const float* emb, long long batch, float* scores, cuda
   }
   // the concatenated y needs every level's pooling: join the side branches (also on the error path, so that the
   // workspace is not freed under them)
-  for (int l = 0; l + 1 < d.n_levels && fork; ++l) cudaStreamWaitEvent(st, h.join_ev[l], 0);
+  for (int l = 0; l + 1 < d.n_levels; ++l) cudaStreamWaitEvent(st, h.join_ev[l], 0);
   // out = sigmoid(BN_K(fc(concat y))): y -> planes, one more split GEMM into U ([batch][640]), then the sigmoid
   if (!rc) rc = split_rows(Y, ystride, batch, d.n_levels * d.K, d.fc_kpad, 1, nullptr, nullptr, 0, nullptr, nullptr, Yp, st);
-  if (!rc && vmb::igemm_linear_split(Yp, d.fc_wp, d.fc_bias, U, hpad, 0, int(batch), hpad, d.fc_kpad, st)) {
-    vmb::set_kernel_error("mla: %s", vmb::igemm_last_error());
+  if (!rc && vmb::planes_gemm(Yp, d.fc_wp, d.fc_bias, U, hpad, 0, int(batch), hpad, d.fc_kpad, 2, 0, st)) {
+    vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
     rc = 1;
   }
   if (!rc) {
@@ -409,18 +394,7 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
   const int in_pad = d.lvl[0].fc[0].kpad, hpad = kPad;
   const size_t sz_x = up(size_t(rows) * 2 * in_pad * 2), sz_p = up(size_t(rows) * 2 * hpad * 2);
   const size_t sz_u = up(size_t(rows) * hpad * 4), sz_yp = up(size_t(batch) * 2 * d.fc_kpad * 2);
-  bool fork = d.n_levels > 1 && mla_fork_enabled();
-  if (fork && !h.side) {
-    bool ok = cudaStreamCreateWithFlags(&h.side, cudaStreamNonBlocking) == cudaSuccess;
-    for (int i = 0; i < kMaxLevels && ok; ++i)
-      ok = cudaEventCreateWithFlags(&h.fork_ev[i], cudaEventDisableTiming) == cudaSuccess &&
-           cudaEventCreateWithFlags(&h.gemm_ev[i], cudaEventDisableTiming) == cudaSuccess &&
-           cudaEventCreateWithFlags(&h.join_ev[i], cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) {
-      vmb::set_kernel_error("mla: cannot create the side stream: %s", cudaGetErrorString(cudaGetLastError()));
-      return 1;
-    }
-  }
+  if (d.n_levels > 1 && ensure_side_stream(h)) return 1;
   // workspace: x planes | three rotating activation plane buffers | normed-input planes | one fp32 z buffer per level |
   // y planes.  Three buffers, not two: a forked fcv GEMM still reads the level's embedding planes while the next level's
   // chain runs, and with two buffers the second GEMM of that chain would have to wait for it before it may start.
@@ -474,15 +448,15 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
       pp = (pp + 1) % 3;
     }
     if (rc) break;
-    const bool side = fork && l + 1 < d.n_levels;
+    const bool side = l + 1 < d.n_levels;
     cudaStream_t as = side ? h.side : st;
     float* Uz = U + l * (sz_u / sizeof(float));
     if (side) {
       cudaEventRecord(h.fork_ev[l], st);            // emb_l planes (cur) are complete here
       cudaStreamWaitEvent(h.side, h.fork_ev[l], 0);
     }
-    if (vmb::igemm_linear_split(cur, L.fcv.wp, L.fcv.bias, Uz, hpad, 0, int(rows), hpad, L.fcv.kpad, as)) {   // z = fcv(emb_l)
-      vmb::set_kernel_error("mla: %s", vmb::igemm_last_error());
+    if (vmb::planes_gemm(cur, L.fcv.wp, L.fcv.bias, Uz, hpad, 0, int(rows), hpad, L.fcv.kpad, 2, 0, as)) {   // z = fcv(emb_l)
+      vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
       rc = 1;
     }
     if (side) {
@@ -502,13 +476,13 @@ static int tc_forward_fused(Handle& h, const float* emb, long long batch, float*
     cur = Pn[l & 1];
   }
   // join the side branches (also on the error path, so that the workspace is not freed under them)
-  for (int l = 0; l + 1 < d.n_levels && fork; ++l) cudaStreamWaitEvent(st, h.join_ev[l], 0);
+  for (int l = 0; l + 1 < d.n_levels; ++l) cudaStreamWaitEvent(st, h.join_ev[l], 0);
   // The output Linear keeps its separate sigmoid pass: a fused epilogue (planes_gemm mode 2) was measured at 30 us against
   // 12.5 + 3.8 us — ten CTAs each writing 527-float rows with scalar stores lose more than the launch saves.
   if (!rc) {
     float* Uo = U;   // level 0's z buffer is free again: its pooling has been joined
-    if (vmb::igemm_linear_split(Yp, d.fc_wp, d.fc_bias, Uo, hpad, 0, int(batch), hpad, d.fc_kpad, st)) {
-      vmb::set_kernel_error("mla: %s", vmb::igemm_last_error());
+    if (vmb::planes_gemm(Yp, d.fc_wp, d.fc_bias, Uo, hpad, 0, int(batch), hpad, d.fc_kpad, 2, 0, st)) {
+      vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
       rc = 1;
     }
     if (!rc) {
@@ -548,8 +522,8 @@ int tc_embedded_mapping(const Handle& h, int level, const float* x, long long ba
   int rc = split_rows(x, in_dim, rows, in_dim, in_pad, d.T, L.n0a, L.n0b, 0, nullptr, nullptr, X, st);
   const void* cur = X;
   for (int j = 0; j < L.n_fc && !rc; ++j) {
-    if (vmb::igemm_linear_split(cur, L.fc[j].wp, L.fc[j].bias, U, hpad, 0, int(rows), hpad, L.fc[j].kpad, st)) {
-      vmb::set_kernel_error("mla: %s", vmb::igemm_last_error());
+    if (vmb::planes_gemm(cur, L.fc[j].wp, L.fc[j].bias, U, hpad, 0, int(rows), hpad, L.fc[j].kpad, 2, 0, st)) {
+      vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
       rc = 1;
       break;
     }
@@ -587,8 +561,8 @@ int tc_attention(const Handle& h, int level, const float* hemb, long long batch,
   }
   float* U = reinterpret_cast<float*>(ws + sz_p);
   int rc = split_rows(hemb, d.hidden, rows, d.hidden, hpad, d.T, nullptr, nullptr, 0, nullptr, nullptr, ws, st);
-  if (!rc && vmb::igemm_linear_split(ws, L.fcv.wp, L.fcv.bias, U, hpad, 0, int(rows), hpad, L.fcv.kpad, st)) {
-    vmb::set_kernel_error("mla: %s", vmb::igemm_last_error());
+  if (!rc && vmb::planes_gemm(ws, L.fcv.wp, L.fcv.bias, U, hpad, 0, int(rows), hpad, L.fcv.kpad, 2, 0, st)) {
+    vmb::set_kernel_error("mla: %s", vmb::planes_gemm_last_error());
     rc = 1;
   }
   if (!rc) {

@@ -459,26 +459,6 @@ int launch_planes(const CUtensorMap& ta, const CUtensorMap& tb, const PlanesPara
 
 const char* planes_gemm_last_error() { return g_perr; }
 
-bool planes_gemm_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("VMB_PLANES_GEMM");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
-// Which three-plane variants may take 128 x 64 tiles — bit 0: plain stores, bit 1: statistics epilogue, bit 2:
-// gradient-statistics epilogue.  Measured on the training step (A/B on one box, VMB_PLANES_NARROW=<mask>): 0.884 ms with
-// 128-wide tiles everywhere, 0.875 ms with mask 5 (the default), 0.895 ms with mask 7 — the statistics epilogue's
-// per-tile barrier and partial-sum pass cost more per tile than the fuller last wave gives back.
-static int narrow_tiles_mask() {
-  static const int mask = [] {
-    const char* e = getenv("VMB_PLANES_NARROW");
-    return e ? atoi(e) : 5;
-  }();
-  return mask;
-}
-
 // out fp32 [M][ldo] = act(sum of plane products + bias), or with ksplit > 1 / == -1: out += the K slices' partial sums.
 // K % 32 == 0, N % 128 == 0, planes 2 or 3; the operands' rows are planes * K bf16 long.  With epi != nullptr (planes
 // == 2, no K split) the epilogue of PlanesEpi::mode replaces the fp32 store.
@@ -491,6 +471,13 @@ static int planes_gemm_any(const void* a_planes, const void* b_planes, const flo
              planes);
     return 1;
   }
+  // fp32 out without a K split: plain stores of one full 32-byte sector per lane and store
+  const bool reduce = ksplit > 1 || ksplit == -1;
+  if (!epi && !reduce && (ldo % 8 != 0 || (reinterpret_cast<uintptr_t>(out) & 31))) {
+    snprintf(g_perr, sizeof g_perr, "planes_gemm: out must be 32-byte aligned and ldo a multiple of 8 floats (ldo=%lld)",
+             ldo);
+    return 1;
+  }
   if (epi) {
     if (planes != 2 || ksplit != 0 || epi->mode != 1 || epi->cols <= 0 || epi->cols > N || !epi->dst || epi->T <= 0 ||
         epi->cpad < N || epi->cpad % 16 != 0 || (epi->a1 && !epi->b1) || (epi->dst2 && (!epi->a2 || !epi->b2)) ||
@@ -499,12 +486,15 @@ static int planes_gemm_any(const void* a_planes, const void* b_planes, const flo
       return 1;
     }
   }
-  // Tile width: 128, or 64 (three planes, the variants of narrow_tiles_mask()) when that shortens the schedule — whole
-  // waves of 148 tiles at one unit of time each against waves of half-width tiles at ~0.6 units (the narrower MMA
-  // re-reads A twice as often).
+  // Tile width: 128, or 64 (three planes, plain stores or the gradient-statistics epilogue) when that shortens the
+  // schedule — whole waves of 148 tiles at one unit of time each against waves of half-width tiles at ~0.6 units (the
+  // narrower MMA re-reads A twice as often).  The statistics epilogue keeps 128-wide tiles: its per-tile barrier and
+  // partial-sum pass cost more per tile than the fuller last wave gives back.  Measured on the training step: 0.884 ms
+  // with 128-wide tiles everywhere, 0.875 ms with 64-wide tiles allowed for plain stores and gradient statistics (this
+  // policy), 0.895 ms with the statistics epilogue allowed them as well.
   const int m_tiles = (M + kBM - 1) / kBM;
   int bn = 128;
-  if (planes == 3 && !epi && ksplit == 0 && (narrow_tiles_mask() & (gs ? 4 : stats ? 2 : 1))) {
+  if (planes == 3 && !epi && !stats && ksplit == 0) {
     const int sms = num_sms();
     const int t128 = m_tiles * (N / 128);
     const double cost128 = double((t128 + sms - 1) / sms), cost64 = 0.6 * double((2 * t128 + sms - 1) / sms);
@@ -557,10 +547,9 @@ static int planes_gemm_any(const void* a_planes, const void* b_planes, const flo
       return 1;
     }
     p.stats = *stats;
-    if (bn == 64) return launch_planes<3, false, 3, 64>(ta, tb, p, stream);
     return planes == 3 ? launch_planes<3, false, 3>(ta, tb, p, stream) : launch_planes<2, false, 3>(ta, tb, p, stream);
   }
-  if (ksplit > 1 || ksplit == -1)
+  if (reduce)
     return planes == 3 ? launch_planes<3, true>(ta, tb, p, stream) : launch_planes<2, true>(ta, tb, p, stream);
   if (bn == 64) return launch_planes<3, false, 0, 64>(ta, tb, p, stream);
   return planes == 3 ? launch_planes<3, false>(ta, tb, p, stream) : launch_planes<2, false>(ta, tb, p, stream);

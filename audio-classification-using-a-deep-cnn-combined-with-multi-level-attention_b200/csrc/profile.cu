@@ -1,6 +1,5 @@
 // Launch accounting and optional per-stage CUDA-event timing (used by bench.py for the roofline line).
 // Disabled by default: when off, stage marks cost one relaxed atomic load.
-#include <cstdlib>
 #include <atomic>
 #include <mutex>
 #include <vector>
@@ -48,16 +47,6 @@ StageTimer::~StageTimer() {
   g_spans.push_back(Span{a_, b_, stage_});
 }
 
-}  // namespace vmb
-
-namespace vmb {
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("VMB_PDL");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
 }  // namespace vmb
 
 extern "C" {

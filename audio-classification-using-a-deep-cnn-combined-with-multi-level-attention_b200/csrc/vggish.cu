@@ -280,8 +280,10 @@ int vmb_vggish_forward(vmb_vggish_t* h, const float* examples, long long n, floa
                              (sat && i < 2) ? sat + 6 + i : nullptr);
     else if (i < 2)
       rc = vmb::igemm_linear_split_out(fc_in[i], h->fc_w[i], h->fc_b[i], fc_out[i], 1, int(n), kFcOut[i], kFcIn[i], st);
+    else if (vmb::planes_gemm(fc_in[i], h->fc_w[i], h->fc_b[i], emb, kFcOut[i], 1, int(n), kFcOut[i], kFcIn[i], 2, 0, st))
+      return fail("vmb_vggish_forward: %s", vmb::planes_gemm_last_error());
     else
-      rc = vmb::igemm_linear_split(fc_in[i], h->fc_w[i], h->fc_b[i], emb, kFcOut[i], 1, int(n), kFcOut[i], kFcIn[i], st);
+      rc = 0;
     if (rc) return fail("vmb_vggish_forward: %s", vmb::igemm_last_error());
   }
   return 0;

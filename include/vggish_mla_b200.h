@@ -33,20 +33,20 @@ int vmb_device_arch(int device);
  * (no reference counterpart: the reference only wall-clocks whole epochs, train.py:71,164-165)
  * Number of CUDA kernels this library has launched in this process.                                   */
 long long vmb_launch_count(void);
-/* Kernel selection for the bf16 conv3x3 / FC layers with C_out (N) a multiple of 256: 1 = the CTA-pair kernel
- * (tcgen05 cta_group::2, the default), 0 = the single-CTA kernel (kept as the A/B baseline; results are bit-identical),
- * -1 = back to the default (environment VMB_IGEMM_PAIR, else 1).  Returns the previous setting (0/1).  Diagnostics only:
- * the reference has no counterpart (vggish.py:13-19, :108-118 are the layers both kernels implement). */
+/* Kernel selectors for tests and diagnostics.  Each keeps one process-wide setting: 1 or -1 = the default kernel, 0 = the
+ * reference kernel that the bit-identity tests compare it with.  Each returns the previous setting (0 / 1).
+ * The reference has no counterpart for any of them.
+ * vmb_igemm_pair_enable: the bf16 conv3x3 / FC layers with C_out (N) a multiple of 256 (vggish.py:13-19, :108-118) run
+ * on the CTA-pair kernel (tcgen05 cta_group::2, the default) or on the single-CTA kernel; the results are bit-identical. */
 int vmb_igemm_pair_enable(int on);
-/* Same switch for the haloed-box variant of the C_out = 128 conv (conv2, vggish.py:113 with 64 -> 128 channels): one
- * activation box with a one-row halo per (channel block, dx) feeds the three dy taps, instead of one box per tap.
- * 1 (default) / 0 / -1 as above; every bf16 conv kernel adds its partial products in the same order, so the results are
- * bit-identical either way. */
+/* The C_out = 128 conv (conv2, vggish.py:113 with 64 -> 128 channels): one activation box with a one-row halo per
+ * (channel block, dx) feeds the three dy taps (the default), or one box per tap.  Every bf16 conv kernel adds its
+ * partial products in the same order, so the results are bit-identical either way. */
 int vmb_igemm_halo_enable(int on);
-/* Eval-mode head (model.py:258-269): 1 (default) = the glue between the Linear layers of an embedding chain —
- * BatchNorm1d(T) affine + ReLU + operand split (model.py:219-221) — runs in the GEMM epilogues; 0 = as separate
- * kernels (the A/B baseline: every value is computed by the same expressions, so the scores are bit-identical);
- * -1 = back to the default (environment VMB_MLA_FUSE, else 1).  Returns the previous override (-1 / 0 / 1). */
+/* Eval-mode head (model.py:258-269): the glue between the Linear layers of an embedding chain — BatchNorm1d(T) affine +
+ * ReLU + operand split (model.py:219-221) — runs in the GEMM epilogues (the default), or as separate kernels.  Every
+ * value is computed by the same expressions, so the scores are bit-identical.  The separate kernels are also the only
+ * path when the attention pooling of a clip needs more than 48 KB of shared memory. */
 int vmb_mla_fuse_enable(int on);
 /* Per-stage device timing with CUDA events recorded on the caller's stream around each stage of
  * vmb_vggish_forward / vmb_pipeline_forward.  Stage ids: */

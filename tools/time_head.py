@@ -1,5 +1,5 @@
 """Times the eval-mode attention head alone (CUDA events, batch 256 x 10 x 128, K = 527, model_conf [2, 1]).
-Environment switches for A/B runs: VMB_MLA_FUSE, VMB_MLA_FORK, VMB_PLANES_GEMM, VMB_PDL (0 / 1)."""
+VMB_LIB=<path> times another build of the library."""
 import os
 import sys
 

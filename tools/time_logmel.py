@@ -1,5 +1,5 @@
 """Times the log-mel front end alone (CUDA events, 256 clips of 10 s) and compares it with the fp32 CUDA-core kernel.
-VMB_LOGMEL_PLANES=1 in the environment selects the first tensor-core version for an A/B run."""
+Aligned input takes the centred kernel; VMB_LIB=<path> times another build of the library."""
 import os
 import sys
 
@@ -27,4 +27,4 @@ for name, fn, x in (("fp32", engine.logmel, waves), ("pcm16", engine.logmel_pcm1
         fn(x)
     b.record()
     torch.cuda.synchronize()
-    print(f"{name}: {a.elapsed_time(b) / 50:.4f} ms per 256 clips (planes={os.environ.get('VMB_LOGMEL_PLANES', '0')})")
+    print(f"{name}: {a.elapsed_time(b) / 50:.4f} ms per 256 clips")
